@@ -2,6 +2,7 @@
 """Benchmark of the LOB simulation step (BASELINE.json metric: LOB messages/s and env steps/s, whole box).
 
     python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--workload all|replay|rollout|collect|multiticker]
+                    [--dump-outputs DIR]
 
 ONE JSON line.  The headline (`value`, `e2e`, `roofline`, `cpu_baseline`) is BASELINE.json configs[1]: a synthetic
 SPY-shaped day (10 levels, 1e7 messages, seed 0) replayed through 4096 batched books per GPU (weak scaling); one bench
@@ -22,6 +23,11 @@ Timing: CUDA events on the launching stream around the timed calls, inputs resid
 through the host-buffer C-ABI calls (`lobsim_replay_host` / `lobsim_step_host`, pinned host memory, H2D + D2H inside the
 timed region) gives `e2e`.  L2 is flushed (256 MiB write) between timed iterations.  Multi-GPU: one process per GPU
 (torchrun), books sharded by rank; times are the max over ranks.
+
+`--dump-outputs DIR` writes what the timed calls returned in their last step, one DIR/<name>.npy per array (float64, or
+float32 where the call returns float32): the book states after the replays, the books of 16 sampled envs, and the rollout
+tensors of a fixed sample of 1024 envs.  Every input is generated from fixed seeds, so two builds run with the same
+arguments can be compared output for output.
 """
 from __future__ import annotations
 
@@ -48,6 +54,10 @@ S_STATE_L50 = 10816              # ... for L=50, mean queue 12
 CPU_SAMPLE_SECONDS = 10.0        # bounded cpu_baseline sample (the contract asks for about 10-30 s of CPU work)
 PY_REFERENCE_MSGS_PER_CORE = 4.9e4   # BASELINE.md section 2: the CPython reference's Exchange.process_order loop (survey container)
 PY_REFERENCE_ENV_STEPS_PER_CORE = (42, 72)
+HBM_PEAK_GBS = 7700.0            # HBM3e bandwidth of one B200 (NVIDIA HGX B200 data sheet): the roofline's denominator
+HBM_PEAK_SOURCE = "NVIDIA HGX B200 data sheet, one GPU (not measured)"
+DUMP_SAMPLE_ENVS = 1024          # --dump-outputs: envs kept of the large per-env rollout outputs (fixed seeded sample)
+DUMP_MAX_BYTES = 64 << 20
 
 
 def parse_args():
@@ -66,7 +76,18 @@ def parse_args():
     ap.add_argument("--segment-steps", type=int, default=2340)
     ap.add_argument("--sub-steps", type=int, default=4, help="timed steps of each sub-record (warm-up: 3)")
     ap.add_argument("--no-cpu-baseline", action="store_true")
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write what the timed calls returned in their last step as "
+                                                           "DIR/<name>.npy (float64 / float32), to compare two builds")
+    args = ap.parse_args()
+    if args.dump_outputs and args.impl != "ours":
+        ap.error("--dump-outputs needs --impl ours")
+    return args
+
+
+def sub_schedule(args):
+    """(timed steps, warm-up steps) of the rollout / collect / multiticker records: --steps / --warmup when that workload
+    was asked for alone, else --sub-steps after 3 warm-up steps."""
+    return (args.steps, args.warmup) if args.workload != "all" else (args.sub_steps, 3)
 
 
 def ncu_traffic(key: str):
@@ -79,19 +100,10 @@ def ncu_traffic(key: str):
         return None
 
 
-def measured_peaks():
-    p = ROOT / "MEASURED_PEAKS.json"
-    if p.exists():
-        d = json.loads(p.read_text())
-        return float(d["hbm_gbs"]), "measured (MEASURED_PEAKS.json)"
-    return 6650.0, "fallback (B200_PROFILING.md)"
-
-
 def roofline(algo_bytes_per_launch: float, launch_ms: float, kernel: str, traffic_key: str = None, **extra):
-    peak, peak_src = measured_peaks()
     achieved = algo_bytes_per_launch / (launch_ms / 1e3) / 1e9
-    r = {"bound": "hbm", "achieved": achieved, "peak": peak, "unit": "GB/s", "frac": achieved / peak,
-         "traffic": ncu_traffic(traffic_key) if traffic_key else None, "peak_source": peak_src, "kernel": kernel,
+    r = {"bound": "hbm", "achieved": achieved, "peak": HBM_PEAK_GBS, "unit": "GB/s", "frac": achieved / HBM_PEAK_GBS,
+         "traffic": ncu_traffic(traffic_key) if traffic_key else None, "peak_source": HBM_PEAK_SOURCE, "kernel": kernel,
          "algorithmic_bytes_per_launch": algo_bytes_per_launch, "launch_ms": launch_ms}
     r.update(extra)
     return r
@@ -320,6 +332,32 @@ class Ctx:
         self.cur = torch.cuda.current_stream(self.dev)
         self.flush = torch.empty(256 << 20, dtype=torch.uint8, device=self.dev)
         self.launches = 0
+        self.outputs = {} if args.dump_outputs else None
+
+    def keep(self, name: str, arr, envs=None, env_axis: int = 0):
+        """--dump-outputs: hold `arr` (numpy or torch), restricted to `envs` along `env_axis`, as <name>.npy."""
+        if self.outputs is None:
+            return
+        a = arr.detach().cpu().numpy() if hasattr(arr, "detach") else np.asarray(arr)
+        if envs is not None:
+            a = np.take(a, envs, axis=env_axis)
+        self.outputs[name] = a.astype(np.float32 if a.dtype == np.float32 else np.float64)
+
+    def keep_state(self, prefix: str, state):
+        for f in state.dtype.names:
+            self.keep(f"{prefix}_{f}", state[f])
+
+    @staticmethod
+    def env_sample(n_envs: int):
+        return np.sort(np.random.default_rng(0).choice(n_envs, min(n_envs, DUMP_SAMPLE_ENVS), replace=False))
+
+    def write_outputs(self, out_dir: str):
+        total = sum(a.nbytes for a in self.outputs.values())
+        assert total <= DUMP_MAX_BYTES, f"--dump-outputs: {total} bytes"
+        d = Path(out_dir)
+        d.mkdir(parents=True, exist_ok=True)
+        for name, a in self.outputs.items():
+            np.save(d / f"{name}.npy", a)
 
     def barrier(self):
         if self.world > 1:
@@ -366,25 +404,42 @@ def run_replay(ctx: Ctx, stream, line):
     assert sim.kernel_path == "fast"
     sim.load_stream(0, stream)
     total = args.warmup + args.steps
-    assert total * seg <= stream.n_grid_steps, "not enough stream for warmup + steps segments"
+    # bench step i replays segment i mod n_seg of the day; when the day is used up every book starts over from its first
+    # snapshot (untimed), so --steps is not bounded by the length of the stream
+    n_seg = stream.n_grid_steps // seg
+    assert n_seg >= 1, "the stream is shorter than one segment"
+    end = ((total - 1) % n_seg + 1) * seg                       # grid step every book stands at after the last step
+    off = stream.step_off.astype(np.int64)
+    msgs_per_env = int(sum(off[(i % n_seg + 1) * seg] - off[i % n_seg * seg] for i in range(args.warmup, total)))
 
     # ---- device-resident arm -----------------------------------------------------------------------------------------
     sim.reset_book(0, 0)
     sampler = ClockSampler(ctx.local_rank).start()
-    l0 = sim.launch_count
-    ms = ctx.timed(lambda i: sim.replay(seg), args.steps, args.warmup)
-    launches = sim.launch_count - l0 - args.warmup
+    l0, rewind_launches = sim.launch_count, 0
+
+    def rewind(i):
+        nonlocal rewind_launches
+        if i and i % n_seg == 0:
+            c = sim.launch_count
+            sim.reset_book(0, 0)
+            rewind_launches += sim.launch_count - c
+
+    ms = ctx.timed(lambda i: sim.replay(seg), args.steps, args.warmup, before=rewind)
+    launches = sim.launch_count - l0 - args.warmup - rewind_launches
     clocks = sampler.stop()
     t_dev = sum(ms) / 1e3
-    first = args.warmup * seg
-    msgs_per_env = int(stream.step_off[first + args.steps * seg]) - int(stream.step_off[first])
     state = sim.state()
     assert np.all(state["err"] == 0), "error flags raised during the bench: %s" % np.unique(state["err"])
-    assert np.all(state["now_step"] == total * seg)
+    assert np.all(state["now_step"] == end)
     # every book replayed the same stream: they must be identical, and equal to the historical book
     assert len(np.unique(state[["best_buy", "best_sell", "best_buy_volume", "best_sell_volume"]])) == 1
-    snap = stream.snapshots[total * seg // stream.steps_per_second]
+    snap = stream.snapshots[end // stream.steps_per_second]
     assert state["best_buy"][0] == snap[0, 0, 0] and state["best_sell"][0] == snap[1, 0, 0]
+    ctx.keep_state("replay_state", state)
+    if ctx.outputs is not None:     # every entry of both sides of 16 sampled books; rows: env, side, price, volume, ref, level
+        books = [np.column_stack([np.full(len(b), env), np.full(len(b), side)] + [b[f] for f in b.dtype.names])
+                 for env in ctx.env_sample(n_envs)[:16] for side in (0, 1) for b in [sim.dump_book(int(env), side)]]
+        ctx.keep("replay_books", np.concatenate(books))
 
     # ---- end-to-end arm: host buffers through lobsim_replay_host ---------------------------------------------------
     pinned = torch.from_numpy(stream.msgs.view(np.uint8).reshape(-1, 16)).pin_memory()
@@ -395,7 +450,10 @@ def run_replay(ctx: Ctx, stream, line):
     h2d = d2h = 0
     t_e2e = 0.0
     for i in range(total):
-        a, b = int(stream.step_off[i * seg]), int(stream.step_off[(i + 1) * seg])
+        s = i % n_seg
+        a, b = int(stream.step_off[s * seg]), int(stream.step_off[(s + 1) * seg])
+        if i and s == 0:
+            sim.reset_book(0, 0)
         if i == args.warmup:
             ctx.barrier()
         ctx.flush.zero_()
@@ -407,7 +465,7 @@ def run_replay(ctx: Ctx, stream, line):
             t_e2e += dt
             h2d += (b - a) * 16
             d2h += state_out.nbytes
-    assert np.all(state_out["err"] == 0) and np.all(state_out["now_step"] == total * seg)
+    assert np.all(state_out["err"] == 0) and np.all(state_out["now_step"] == end)
 
     t_dev, t_e2e = ctx.max_over_ranks(t_dev, t_e2e)
     world = ctx.world
@@ -513,9 +571,9 @@ def run_rollout(ctx: Ctx, stream):
             if timed:
                 e1.record(ctx.cur)
                 kev.append((e0, e1))
-        box["obs"] = o
+        box.update(obs=o, rew=r, done=d)
 
-    steps, warm = args.sub_steps, 3
+    steps, warm = sub_schedule(args)
     sampler = ClockSampler(ctx.local_rank).start()
     l0 = sim.launch_count
     now0 = None
@@ -533,6 +591,9 @@ def run_rollout(ctx: Ctx, stream):
     off = stream.step_off.astype(np.int64)
     msgs = int((off[st["now_step"]] - off[now0]).sum())
     kernel_ms = float(np.mean([a.elapsed_time(b) for a, b in kev]))
+    envs = ctx.env_sample(n_envs)           # the last env step of the last bench step
+    for k in ("obs", "rew", "done"):
+        ctx.keep(f"rollout_{k}", box[k], envs)
     # end-to-end: host actions in, host obs/reward/done out through lobsim_step_host (pinned buffers)
     a_host = torch.empty((n_envs, 4), dtype=torch.float64).pin_memory()
     o_host = torch.empty((n_envs, obs.shape[1]), dtype=torch.float64).pin_memory()
@@ -601,8 +662,8 @@ def run_collect(ctx: Ctx, stream):
     sim.reset(0, starts)
     agent = abi.Agent(kind=abi.AGENT_TERADACTYL, inventory_index=5, max_inventory=10000.0, default_kappa=10.0, default_omega=0.5,
                       max_kappa=50.0, exponent=1.0)
-    steps, warm = args.sub_steps, 3
-    gev, res = [], {}
+    steps, warm = sub_schedule(args)
+    gev, res, last = [], {}, {}
 
     def step(i):
         obs, act, rew, done = sim.rollout(T, agent)
@@ -612,6 +673,8 @@ def run_collect(ctx: Ctx, stream):
         allstats = parallel.gather_episode_stats(stats)
         e1.record(ctx.cur)
         gev.append((e0, e1))
+        if ctx.outputs is not None:
+            last.update(obs=obs, act=act, rew=rew, done=done, stats=allstats)
         res["mean_return"] = float(allstats[:, 0].mean().item())          # D2H read of the result: the step's sync point
         res["shape"] = list(allstats.shape)
         res["errs"] = int((allstats[:, 7] != 0).sum().item())
@@ -631,6 +694,9 @@ def run_collect(ctx: Ctx, stream):
     st = sim.state()
     assert np.all(st["err"] == 0), np.unique(st["err"])
     assert res["errs"] == 0 and res["shape"] == [n_envs * world, 8], res
+    envs = ctx.env_sample(n_envs)           # [T, N, ...] rollout tensors and the gathered [N, 8] stats of the last bench step
+    for k, v in last.items():
+        ctx.keep(f"collect_{k}", v, envs, env_axis=0 if k == "stats" else 1)
     off = stream.step_off.astype(np.int64)
     msgs = int((off[st["now_step"]] - off[now0]).sum())
     gather_ms = float(np.mean([a.elapsed_time(b) for a, b in gev[warm:]]))
@@ -671,7 +737,7 @@ def run_multiticker(ctx: Ctx):
     world = ctx.world
     n_envs, seg, n_streams = args.multiticker_envs, 1170, 8
     streams = [synthetic.generate(synthetic.heavy_cancel_ticker(seed=k, n_msgs=args.multiticker_msgs)) for k in range(n_streams)]
-    steps, warm = args.sub_steps, 3
+    steps, warm = sub_schedule(args)
     feats = [abi.feature(abi.FEAT_SPREAD, 0, 100000, 0, 5000), abi.feature(abi.FEAT_BOOK_IMBALANCE, 0, 100000, -1, 1),
              abi.feature(abi.FEAT_INVENTORY, 0, 100000, -1e6, 1e6)]
     # capacities: a side of these streams holds at most ~620 orders over the whole day (oracle replay) + ~45 agent orders: 1 024
@@ -702,6 +768,7 @@ def run_multiticker(ctx: Ctx):
     clocks = sampler.stop()
     st = sim.state()
     assert np.all(st["err"] == 0), np.unique(st["err"])
+    ctx.keep_state("multiticker_state", st)
     msgs = count_msgs(starts.astype(np.int64) + warm * seg, starts.astype(np.int64) + (warm + steps) * seg)
     t_dev = ctx.max_over_ranks(sum(ms) / 1e3)
     algo = ALGO_BYTES_PER_MSG * msgs / steps + (ALGO_BYTES_PER_STEP_REPLAY * seg + 2 * S_STATE_L50) * n_envs
@@ -727,12 +794,21 @@ def run_multiticker(ctx: Ctx):
     starts2 = (rng.integers(600, streams[0].n_seconds - (steps + warm) * T // sps - 2, size=n_envs) * sps).astype(np.int32)
     sim.reset(sid, starts2)
     agent = abi.Agent(kind=abi.AGENT_FIXED, fixed_action=(ctypes.c_double * 5)(1, 2, 1, 2, 0))
-    l0 = sim.launch_count
-    ms = ctx.timed(lambda i: sim.rollout(T, agent, want_obs=True), steps, warm)
+    l0, last = sim.launch_count, []
+
+    def roll(i):
+        out = sim.rollout(T, agent, want_obs=True)
+        if ctx.outputs is not None:
+            last[:] = out
+
+    ms = ctx.timed(roll, steps, warm)
     launches = sim.launch_count - l0 - warm
     st = sim.state()
     bad = st["err"] & ~np.uint32(abi.ERR_AGENT_OVERFLOW)
     assert np.all(bad == 0), np.unique(st["err"])
+    envs = ctx.env_sample(n_envs)           # [T, N, ...] obs, act, rew, done of the last bench step
+    for k, v in zip(("obs", "act", "rew", "done"), last):
+        ctx.keep(f"multiticker_env_{k}", v, envs, env_axis=1)
     msgs = count_msgs(starts2.astype(np.int64) + warm * T, starts2.astype(np.int64) + (warm + steps) * T)
     t_env = ctx.max_over_ranks(sum(ms) / 1e3)
     algo = ALGO_BYTES_PER_MSG * msgs / steps + (ALGO_BYTES_PER_STEP_ENV * T + 2 * S_STATE_L50) * n_envs
@@ -785,6 +861,8 @@ def main():
         line.update(rec)
         line.setdefault("vs_baseline", None)
     line["gpu_launches_total"] = int(ctx.launches)
+    if ctx.rank == 0 and ctx.outputs is not None:
+        ctx.write_outputs(args.dump_outputs)
     if ctx.rank == 0:
         print(json.dumps(line))
     if ctx.world > 1:

@@ -1,7 +1,7 @@
 """TEST INFRASTRUCTURE: generate the golden vectors under tests/golden/ by running the UNMODIFIED reference
-(/root/reference, imported through oracle/refshim.py) in this container.
+(a checkout of the original rl4mm project, imported through oracle/refshim.py).
 
-    python -m oracle.gen_golden            # rewrites tests/golden/*.json.gz
+    RL4MM_REFERENCE=<rl4mm checkout> python -m oracle.gen_golden            # rewrites tests/golden/*.json.gz
 
 The reference cannot travel to the GPU box, the vectors can.  tests/test_oracle_golden.py pins the C oracle against
 them (CPU), tests/test_gpu_parity.py pins the CUDA path against them and against the oracle (GPU).
@@ -21,7 +21,7 @@ sys.path.insert(0, str(ROOT))
 from oracle import refshim  # noqa: E402
 
 GOLDEN = ROOT / "tests" / "golden"
-FIXTURE_DIR = Path("/root/reference/test_data")
+FIXTURE_DIR = Path(refshim.REFERENCE_ROOT or "") / "test_data"     # refshim.install() refuses to run without the reference
 MSG_CSV = FIXTURE_DIR / "MSFT_2012-06-21_34200000_37800000_message_50.csv"
 BOOK_CSV = FIXTURE_DIR / "MSFT_2012-06-21_34200000_37800000_orderbook_50.csv"
 DAY = datetime(2012, 6, 21)
@@ -409,8 +409,8 @@ def golden_exchange_fuzz():
 
 
 def golden_packed_fixture():
-    """The MSFT 2012-06-21 fixture (first 1000 LOBSTER rows, 50 levels) packed by rl4mm_b200.packing, so that the GPU
-    box (which has no /root/reference) can replay it."""
+    """The MSFT 2012-06-21 fixture (first 1000 LOBSTER rows, 50 levels) packed by rl4mm_b200.packing, so that the tests
+    can replay it without the reference."""
     from rl4mm_b200.packing import pack_lobster
 
     arrays = {}

@@ -1,9 +1,9 @@
-"""TEST INFRASTRUCTURE ONLY -- import shims that let the *unmodified* reference (``/root/reference``)
-run in this container so that golden vectors can be generated from it (see ``oracle/gen_golden.py``).
+"""TEST INFRASTRUCTURE ONLY -- import shims that let the *unmodified* reference (a checkout of the original rl4mm
+project, located by the environment variable ``RL4MM_REFERENCE``) run so that golden vectors can be generated from it
+(see ``oracle/gen_golden.py``).
 
-Nothing in the product path (``rl4mm_b200/``), ``bench.py`` or the ``-m gpu`` tests imports this module:
-``/root/reference`` does not exist on the GPU box.  The vectors this module helps to produce are committed
-under ``tests/golden/``.
+Nothing in the product path (``rl4mm_b200/``), ``bench.py`` or the ``-m gpu`` tests imports this module: the reference
+is not part of this repository.  The vectors this module helps to produce are committed under ``tests/golden/``.
 
 What is shimmed (SURVEY.md App. B):
   * ``numpy.infty`` (removed in numpy 2; evaluated eagerly at rl4mm/orderbook/Exchange.py:154,
@@ -17,6 +17,7 @@ What is shimmed (SURVEY.md App. B):
 """
 from __future__ import annotations
 
+import os
 import sys
 import types
 from datetime import datetime, timedelta
@@ -25,7 +26,7 @@ from pathlib import Path
 import numpy as np
 import pandas as pd
 
-REFERENCE_ROOT = Path("/root/reference")
+REFERENCE_ROOT = Path(os.environ["RL4MM_REFERENCE"]) if os.environ.get("RL4MM_REFERENCE") else None
 _INSTALLED = False
 
 
@@ -66,8 +67,8 @@ def install() -> None:
     global _INSTALLED
     if _INSTALLED:
         return
-    if not REFERENCE_ROOT.exists():
-        raise RuntimeError("the reference tree is not present in this container (expected on the build box only)")
+    if REFERENCE_ROOT is None or not (REFERENCE_ROOT / "rl4mm").is_dir():
+        raise RuntimeError("set RL4MM_REFERENCE to a checkout of the original rl4mm project")
     if not hasattr(np, "infty"):
         np.infty = np.inf  # noqa: NPY201
 

@@ -272,6 +272,7 @@ def test_fast_lobster_reader_matches_python_packer(tmp_path):
 def test_native_packer_on_the_msft_fixture_and_a_1e6_row_day(tmp_path):
     """SURVEY 8f.1: the native packer == the numpy packer on the reference's own MSFT fixture, and on a 1e6-row synthetic
     LOBSTER file pair (written from a packed synthetic stream), where it also has to be much faster."""
+    import os
     import time
 
     from pathlib import Path
@@ -280,10 +281,11 @@ def test_native_packer_on_the_msft_fixture_and_a_1e6_row_day(tmp_path):
     from rl4mm_b200 import synthetic
     from rl4mm_b200.packing import pack_lobster
 
-    ref_dir = Path("/root/reference/test_data")       # present in the build container only; the packed fixture is committed
+    # the CSV pair ships with the original rl4mm project (RL4MM_REFERENCE), not with this repository; its packed form is committed
+    ref_dir = Path(os.environ.get("RL4MM_REFERENCE", "")) / "test_data"
     m = ref_dir / "MSFT_2012-06-21_34200000_37800000_message_50.csv"
     b = ref_dir / "MSFT_2012-06-21_34200000_37800000_orderbook_50.csv"
-    if m.exists():
+    if os.environ.get("RL4MM_REFERENCE"):
         for tie in ("reference", "file"):
             x, y = pack_lobster(m, b, 50, max_rows=1000, fast=True, tie_order=tie), load_fixture_stream(tie)
             for f_ in ("msgs", "step_off", "snapshots", "snap_valid", "ext_ids"):
