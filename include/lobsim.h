@@ -38,7 +38,14 @@ extern "C" {
 #define LOBSIM_E_NOMEM -3
 #define LOBSIM_E_STATE -4     /* call order violated (e.g. step before reset)         */
 
-/* ---- per-env sticky error bits (replace the reference's Python exceptions) ---------------------------------- */
+/* ---- per-env sticky error bits (replace the reference's Python exceptions) ----------------------------------
+ * Capacity bits: the book of every kernel family flags the capacity that an order (or a snapshot level of a reset or a resync)
+ * would have to exceed, and only that one: LEVEL_OVERFLOW for one price level more than max_levels_per_side on a side,
+ * ORDER_OVERFLOW for one resting order more than max_orders_per_side (snapshot aggregates count as orders), AGENT_OVERFLOW for one
+ * agent order more than max_agent_orders, FILL_LOG_FULL for one fill more than fill_log_capacity in one call.  The order that
+ * does not fit is dropped, so a flagged book no longer follows the reference.  Straight-line and general kernels flag in the
+ * call in which the capacity is first exceeded; the hybrid replay book (csrc/book_hybrid.cuh) may hold a temporary level excess
+ * in its order pool and flags it when it leaves that form, at the latest at the end of the call.                        */
 #define LOBSIM_ERR_EMPTY_BOOK 1u        /* EmptyOrderbookError, rl4mm/orderbook/Exchange.py:32,183-186            */
 #define LOBSIM_ERR_LEVEL_OVERFLOW 2u    /* more price levels on a side than max_levels_per_side                  */
 #define LOBSIM_ERR_ORDER_OVERFLOW 4u    /* more resting orders on a side than max_orders_per_side                */
@@ -318,7 +325,8 @@ int lobsim_forward_step(lobsim_t* h, int32_t n_steps, void* stream);
 int lobsim_reset_book(lobsim_t* h, const int32_t* env_ids_dev, int32_t n, const int32_t* stream_ids_dev,
                       const int32_t* start_steps_dev, void* stream);
 
-/* Exchange.process_order (rl4mm/orderbook/Exchange.py:58-69) for a host list of orders, applied in order.
+/* Exchange.process_order (rl4mm/orderbook/Exchange.py:58-69) for a host list of orders, applied in order.  Like the reference's
+ * exchange it only moves the books: the env's portfolio (inventory, cash) changes in its steps, not here.
  * fills_out_host (capacity max_fills) receives FilledOrders in emission order; refs_out_host[i] is, for a limit order
  * (or its unfilled remainder) that RESTED in the book -- i.e. whenever the reference's OrderIdConvertor hands out a
  * new internal id (OrderIDConvertor.py:12-18) --, the agent order id (agent orders) or 0xffffffff (external orders),

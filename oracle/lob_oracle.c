@@ -40,6 +40,8 @@ typedef struct {
 typedef struct {
   o_level* lv;    /* ascending price (SortedDict) */
   int n, cap;
+  int nord;              /* resting orders on the side (snapshot aggregates included) */
+  int peak_lv, peak_ord; /* high-water marks of n / nord since the last lo_reset_book / lo_set_book */
 } o_side;
 
 typedef struct {
@@ -100,7 +102,7 @@ static void map_del(o_map* m, int64_t k) {
 
 static void side_clear(o_side* s) {
   for (int i = 0; i < s->n; i++) free(s->lv[i].q);
-  s->n = 0;
+  s->n = 0; s->nord = 0;
 }
 static void book_clear(o_book* b) { side_clear(&b->s[0]); side_clear(&b->s[1]); }
 static void book_free(o_book* b) { book_clear(b); free(b->s[0].lv); free(b->s[1].lv); }
@@ -122,21 +124,26 @@ static o_level* side_get_or_insert(o_side* s, int64_t price) {
   memmove(&s->lv[pos + 1], &s->lv[pos], (size_t)(s->n - pos) * sizeof(o_level));
   s->lv[pos].price = price; s->lv[pos].q = NULL; s->lv[pos].n = s->lv[pos].cap = 0;
   s->n++;
+  if (s->n > s->peak_lv) s->peak_lv = s->n;
   return &s->lv[pos];
 }
 static void side_remove_level(o_side* s, int idx) {
+  s->nord -= s->lv[idx].n;
   free(s->lv[idx].q);
   memmove(&s->lv[idx], &s->lv[idx + 1], (size_t)(s->n - idx - 1) * sizeof(o_level));
   s->n--;
 }
-static void level_append(o_level* l, o_order o) {
+static void level_append(o_side* s, o_level* l, o_order o) {
   if (l->n == l->cap) { l->cap = l->cap ? l->cap * 2 : 4; l->q = (o_order*)realloc(l->q, (size_t)l->cap * sizeof(o_order)); }
   l->q[l->n++] = o;
+  if (++s->nord > s->peak_ord) s->peak_ord = s->nord;
 }
-static void level_erase(o_level* l, int pos) {
+static void level_erase(o_side* s, o_level* l, int pos) {
   memmove(&l->q[pos], &l->q[pos + 1], (size_t)(l->n - pos - 1) * sizeof(o_order));
-  l->n--;
+  l->n--; s->nord--;
 }
+/* deque([order]): the level's queue is replaced by one order */
+static void level_replace(o_side* s, o_level* l, o_order o) { s->nord -= l->n; l->n = 0; level_append(s, l, o); }
 
 /* ------------------------------------------------------------------------------------------------------------ */
 /*  feature state                                                                                                 */
@@ -182,6 +189,7 @@ struct lo {
   /* fills of the current step */
   lobsim_fill_t* fills;
   int n_fills, cap_fills;
+  int call_fills, peak_fills; /* fills since the start of the current API call; its high-water mark since lo_reset_book */
   double prev_action[8];
   int has_reset;
 };
@@ -209,6 +217,7 @@ static void add_fill(lo_t* o, int list, int dir, int64_t price, int64_t vol, int
   lobsim_fill_t* f = &o->fills[o->n_fills++];
   f->list = list; f->direction = dir; f->price = (int32_t)price; f->volume = (int32_t)vol; f->is_market = is_market;
   f->ref = ref;
+  if (++o->call_fills > o->peak_fills) o->peak_fills = o->call_fills;
 }
 
 static uint32_t order_ref(const o_order* r) {
@@ -243,7 +252,7 @@ static int reduce_at(lo_t* o, o_book* book, int dir, int64_t price, int pos, int
   l->q[pos].vol -= v;
   if (l->q[pos].vol == 0) {
     if (l->q[pos].is_ext && l->q[pos].ext >= 0) map_del(&o->ext2int, l->q[pos].ext); /* :243-244 */
-    level_erase(l, pos);
+    level_erase(s, l, pos);
   }
   if (l->n == 0) side_remove_level(s, li);
   return 1;
@@ -256,8 +265,8 @@ static void submit_order(lo_t* o, o_msg* m, uint32_t* ref_out) {
   o_order r;
   r.iid = ++o->counter; r.vol = m->vol; r.ext = m->ext; r.is_ext = m->is_ext;
   if (m->is_ext) map_put(&o->ext2int, m->ext, r.iid);
-  level_append(side_get_or_insert(&o->central.s[m->dir], m->price), r);
-  if (!m->is_ext) level_append(side_get_or_insert(&o->internal.s[m->dir], m->price), r);
+  level_append(&o->central.s[m->dir], side_get_or_insert(&o->central.s[m->dir], m->price), r);
+  if (!m->is_ext) level_append(&o->internal.s[m->dir], side_get_or_insert(&o->internal.s[m->dir], m->price), r);
   if (ref_out) *ref_out = m->is_ext ? 0xffffffffu : (uint32_t)r.iid;
 }
 
@@ -386,6 +395,15 @@ static void price_range(const lo_t* o, int64_t* worst_buy, int64_t* worst_sell) 
   *worst_sell = s->n ? s->lv[s->n - 1].price : 0;
 }
 
+/* capacity high-water marks (lo_peaks): restart from the current book */
+static void reset_peaks(lo_t* o) {
+  for (int side = 0; side < 2; side++) {
+    o_side* c = &o->central.s[side]; o_side* a = &o->internal.s[side];
+    c->peak_lv = c->n; c->peak_ord = c->nord; a->peak_lv = a->n; a->peak_ord = a->nord;
+  }
+  o->call_fills = 0; o->peak_fills = 0;
+}
+
 /* OrderbookSimulator.reset_episode -- OrderbookSimulator.py:55-68 (+ get_historical_start_book :90-97,
  * _get_initial_orders_from_snapshot :156-175, Exchange.get_initial_orderbook_from_orders Exchange.py:172-178,
  * _reset_initial_price_ranges :185-188) */
@@ -394,6 +412,7 @@ int lo_reset_book(lo_t* o, int start_step) {
   int64_t t = o->stream.t0_us + (int64_t)start_step * o->cfg.step_us;
   if (t % 1000000) return LOBSIM_E_INVALID; /* "Episodes must be started on the second." :61 */
   book_clear(&o->central); book_clear(&o->internal);
+  reset_peaks(o);
   o->dead = 0; o->err = 0;
   o->now_step = start_step;
   const int32_t* row = snapshot_row(o, (t - o->stream.t0_us) / 1000000);
@@ -404,8 +423,7 @@ int lo_reset_book(lo_t* o, int start_step) {
       int32_t price = row[(side * L + lvl) * 2], vol = row[(side * L + lvl) * 2 + 1];
       if (price == LOBSIM_NO_PRICE) continue;
       o_order r; r.iid = -1; r.ext = -1; r.is_ext = 1; r.vol = vol;
-      o_level* l = side_get_or_insert(&o->central.s[side], price);
-      l->n = 0; level_append(l, r); /* deque([order]) */
+      level_replace(&o->central.s[side], side_get_or_insert(&o->central.s[side], price), r); /* deque([order]) */
     }
   int64_t bb, bs;
   price_range(o, &o->min_buy_price, &o->max_sell_price);
@@ -453,8 +471,7 @@ static void update_outer_levels(lo_t* o) {
         free(canc);
       }
       o_order r; r.iid = -1; r.ext = -1; r.is_ext = 1; r.vol = vol;
-      o_level* l = side_get_or_insert(&o->central.s[side], price);
-      l->n = 0; level_append(l, r); /* central[dir][price] = deque([order]) :130 */
+      level_replace(&o->central.s[side], side_get_or_insert(&o->central.s[side], price), r); /* central[dir][price] = deque([order]) :130 */
     }
   for (int i = 0; i < nrepl; i++) { repl[i].iid = 0; process_order(o, &repl[i], NULL); }
   free(repl);
@@ -466,7 +483,7 @@ static void update_outer_levels(lo_t* o) {
 /* OrderbookSimulator.forward_step -- OrderbookSimulator.py:70-88; messages of the step come from the packed stream
  * (HistoricalOrderGenerator.generate_orders, HistoricalOrderGenerator.py:32-46, get_order_from_external_message
  * :77-90). */
-static void forward_step(lo_t* o, o_msg* internal_orders, int n_internal) {
+static void forward_step_ex(lo_t* o, o_msg* internal_orders, int n_internal, int resync_check) {
   if (o->dead) return;
   if (o->now_step < 0 || o->now_step >= (int64_t)o->stream.n_grid_steps) { o->err |= LOBSIM_ERR_END_OF_STREAM; o->dead = 1; return; }
   for (int i = 0; i < n_internal && !o->dead; i++) process_order(o, &internal_orders[i], NULL);
@@ -479,13 +496,23 @@ static void forward_step(lo_t* o, o_msg* internal_orders, int n_internal) {
   }
   if (o->dead) return;
   o->now_step += 1;
-  if (o->cfg.resync && near_exiting(o) && now_us(o) % 1000000 == 0) update_outer_levels(o);
+  if (resync_check && o->cfg.resync && near_exiting(o) && now_us(o) % 1000000 == 0) update_outer_levels(o);
 }
+static void forward_step(lo_t* o, o_msg* internal_orders, int n_internal) { forward_step_ex(o, internal_orders, n_internal, 1); }
 
 int lo_replay(lo_t* o, int n_steps) {
   if (!o->has_stream) return LOBSIM_E_STATE;
-  o->n_fills = 0;
+  o->n_fills = 0; o->call_fills = 0;
   for (int i = 0; i < n_steps; i++) forward_step(o, NULL, 0);
+  return LOBSIM_OK;
+}
+
+/* ONE OrderbookSimulator.forward_step(until = now + n_steps * step_size) -- OrderbookSimulator.py:70-88: the messages of the
+ * n_steps grid intervals, then the resync condition (:86-87) evaluated once, at `until` */
+int lo_forward_step(lo_t* o, int n_steps) {
+  if (!o->has_stream) return LOBSIM_E_STATE;
+  o->n_fills = 0; o->call_fills = 0;
+  for (int i = 0; i < n_steps; i++) forward_step_ex(o, NULL, 0, i == n_steps - 1);
   return LOBSIM_OK;
 }
 
@@ -903,7 +930,7 @@ int lo_reset(lo_t* o, int episode_start_step, double* obs_out) {
   if (!o->cfg.portfolio_carryover) { o->inventory = o->cfg.initial_inventory; o->cash = o->cfg.initial_cash; }
   memset(o->prev_action, 0, sizeof o->prev_action);
   o->has_reset = 1;
-  o->n_fills = 0;
+  o->n_fills = 0; o->call_fills = 0;
   int64_t bb, bs, bv, sv;
   if (book_tops(o, &bb, &bs, &bv, &sv)) o->price = book_microprice(bb, bs, bv, sv); else o->price = NAN;
   int64_t ep_start_us = o->stream.t0_us + (int64_t)episode_start_step * o->cfg.step_us;
@@ -920,7 +947,12 @@ int lo_reset(lo_t* o, int episode_start_step, double* obs_out) {
 }
 
 /* HistoricalOrderbookEnvironment.step -- HOE.py:163-178 */
+static int step_impl(lo_t* o, const double* action, double* obs, double* reward, uint8_t* done);
 int lo_step(lo_t* o, const double* action, double* obs, double* reward, uint8_t* done) {
+  o->call_fills = 0;
+  return step_impl(o, action, obs, reward, done);
+}
+static int step_impl(lo_t* o, const double* action, double* obs, double* reward, uint8_t* done) {
   if (!o->has_stream || !o->has_reset) return LOBSIM_E_STATE;
   o_msgs orders = {0};
   if (!o->dead) convert_action_to_orders(o, action, &orders);
@@ -1021,6 +1053,7 @@ int lo_rollout_info(lo_t* o, int T, const lobsim_agent_t* ag, double* obs, doubl
   int od = lo_obs_dim(&o->cfg), ad = lo_action_dim(&o->cfg);
   double cur_obs[LOBSIM_MAX_FEATURES + 8], a[8];
   get_observation(o, o->prev_action, cur_obs);
+  o->call_fills = 0;   /* one call: the device's per-call fill log spans all T steps */
   for (int t = 0; t < T; t++) {
     if (ag->kind == LOBSIM_AGENT_NONE) {
       env_forward(o, NULL, 0);
@@ -1032,7 +1065,7 @@ int lo_rollout_info(lo_t* o, int T, const lobsim_agent_t* ag, double* obs, doubl
     else if (ag->kind == LOBSIM_AGENT_RANDOM) lo_random_action(ag, o->env_index, o->now_step, a);
     else lo_agent_action(ag, cur_obs, a);
     double r; uint8_t d;
-    lo_step(o, a, cur_obs, &r, &d);
+    step_impl(o, a, cur_obs, &r, &d);
     memcpy(o->prev_action, a, sizeof(double) * (size_t)ad);
     if (obs) memcpy(obs + (size_t)t * od, cur_obs, sizeof(double) * (size_t)od);
     if (act && ag->kind != LOBSIM_AGENT_EXTERNAL) memcpy(act + (size_t)t * ad, a, sizeof(double) * (size_t)ad);
@@ -1081,8 +1114,77 @@ int lo_process_order(lo_t* o, const lobsim_order_t* ord, uint32_t* ref_out) {
   if (ord->is_external) { m.ext = ord->ref; m.iid = 0; } else { m.ext = -1; m.iid = (int64_t)(ord->ref & 0x7fffffffu); }
   if (ord->type == LOBSIM_MSG_LIMIT || ord->type == LOBSIM_MSG_MARKET) m.iid = 0;
   if (ref_out) *ref_out = 0;
+  const int peak_fills = o->peak_fills;
   process_order(o, &m, ref_out);
+  o->peak_fills = peak_fills;   /* lobsim_process_orders returns its fills to the caller: they never enter the fill log */
   return LOBSIM_OK;
+}
+
+/* Exchange(central_orderbook=..., internal_orderbook=...) -- Exchange.py:40-49, with L3 entries in the lobsim_dump_book format
+ * (per side best level first, FIFO inside a level; ref = LOBSIM_REF_AGENT | id marks the agent's orders, which also form the
+ * internal book).  A new Exchange has a new OrderIdConvertor, so the external-id map is rebuilt from the given book; the id
+ * counter moves above the largest id.  The clock, the portfolio and the price-range trackers stay; the error bits (and the
+ * capacity high-water marks, which explain them) restart, as on the device (lobsim_set_book).
+ * External orders carry no internal id in the dump: each gets the smallest id above its predecessor in the level, so that the
+ * binary search by internal id (Exchange._find_queue_position) stays valid.  Returns LOBSIM_E_INVALID (book unchanged) for
+ * unsorted levels, negative volumes, or agent ids that leave no room for the external orders queued before them. */
+int lo_set_book(lo_t* o, const lobsim_book_entry_t* buy, int n_buy, const lobsim_book_entry_t* sell, int n_sell) {
+  for (int side = 0; side < 2; side++) {   /* validate first: the book is only replaced by a valid one */
+    const lobsim_book_entry_t* e = side ? sell : buy;
+    const int n = side ? n_sell : n_buy;
+    int64_t last = INT64_MIN;
+    for (int i = 0; i < n; i++) {
+      if (e[i].volume < 0) return LOBSIM_E_INVALID;
+      if (i > 0 && e[i].price != e[i - 1].price) {
+        if (side == 0 ? e[i].price >= e[i - 1].price : e[i].price <= e[i - 1].price) return LOBSIM_E_INVALID;
+        last = INT64_MIN;
+      }
+      if (e[i].ref & LOBSIM_REF_AGENT) {
+        const int64_t id = (int64_t)(e[i].ref & 0x7fffffffu);
+        if (id <= last || id < 1) return LOBSIM_E_INVALID;
+        last = id;
+      } else if (e[i].ref == LOBSIM_REF_AGGREGATE) {
+        if (last != INT64_MIN) return LOBSIM_E_INVALID;   /* a snapshot aggregate heads its level */
+        last = -1;
+      } else last = last < 1 ? 1 : last + 1;
+    }
+  }
+  book_clear(&o->central); book_clear(&o->internal);
+  map_free(&o->ext2int); map_init(&o->ext2int, 1024);
+  int64_t max_id = 0;
+  for (int side = 0; side < 2; side++) {
+    const lobsim_book_entry_t* e = side ? sell : buy;
+    const int n = side ? n_sell : n_buy;
+    o_level* l = NULL; o_level* il = NULL;
+    int64_t last = INT64_MIN;
+    for (int i = 0; i < n; i++) {
+      if (i == 0 || e[i].price != e[i - 1].price) { l = side_get_or_insert(&o->central.s[side], e[i].price); il = NULL; last = INT64_MIN; }
+      o_order r; r.vol = e[i].volume;
+      if (e[i].ref & LOBSIM_REF_AGENT) { r.iid = (int64_t)(e[i].ref & 0x7fffffffu); r.ext = -1; r.is_ext = 0; }
+      else if (e[i].ref == LOBSIM_REF_AGGREGATE) { r.iid = -1; r.ext = -1; r.is_ext = 1; }
+      else { r.iid = last < 1 ? 1 : last + 1; r.ext = e[i].ref; r.is_ext = 1; map_put(&o->ext2int, r.ext, r.iid); }
+      last = r.iid;
+      if (r.iid > max_id) max_id = r.iid;
+      level_append(&o->central.s[side], l, r);
+      if (!r.is_ext) {
+        if (!il) il = side_get_or_insert(&o->internal.s[side], e[i].price);
+        level_append(&o->internal.s[side], il, r);
+      }
+    }
+  }
+  if (o->counter < max_id) o->counter = max_id;
+  reset_peaks(o);
+  o->err = 0; o->dead = 0;
+  return LOBSIM_OK;
+}
+
+void lo_peaks(const lo_t* o, int32_t* out) {
+  for (int side = 0; side < 2; side++) {
+    out[side] = o->central.s[side].peak_lv;
+    out[2 + side] = o->central.s[side].peak_ord;
+    out[4 + side] = o->internal.s[side].peak_ord;
+  }
+  out[6] = o->peak_fills;
 }
 
 void lo_clear_fills(lo_t* o) { o->n_fills = 0; }

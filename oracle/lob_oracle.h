@@ -13,6 +13,11 @@ int lo_reset_book(lo_t* o, int start_step);
 int lo_reset(lo_t* o, int episode_start_step, double* obs_out);
 int lo_step(lo_t* o, const double* action, double* obs, double* reward, uint8_t* done);
 int lo_replay(lo_t* o, int n_steps);
+int lo_forward_step(lo_t* o, int n_steps);
+int lo_set_book(lo_t* o, const lobsim_book_entry_t* buy, int n_buy, const lobsim_book_entry_t* sell, int n_sell);
+/* capacity high-water marks since the last lo_reset_book / lo_reset / lo_set_book: out[0..1] price levels per side, [2..3] resting
+ * orders per side (snapshot aggregates included), [4..5] agent orders per side, [6] the most fills recorded in one call */
+void lo_peaks(const lo_t* o, int32_t* out);
 int lo_rollout(lo_t* o, int T, const lobsim_agent_t* agent, double* obs, double* act, double* rew, uint8_t* done);
 int lo_rollout_info(lo_t* o, int T, const lobsim_agent_t* agent, double* obs, double* act, double* rew, uint8_t* done, double* info);
 void lo_agent_action(const lobsim_agent_t* agent, const double* obs, double* action);

@@ -45,6 +45,9 @@ def lib():
         L.lo_reset.argtypes = [C.c_void_p, C.c_int, C.c_void_p]
         L.lo_step.argtypes = [C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p]
         L.lo_replay.argtypes = [C.c_void_p, C.c_int]
+        L.lo_forward_step.argtypes = [C.c_void_p, C.c_int]
+        L.lo_set_book.argtypes = [C.c_void_p, C.c_void_p, C.c_int, C.c_void_p, C.c_int]
+        L.lo_peaks.argtypes = [C.c_void_p, C.c_void_p]
         L.lo_rollout.argtypes = [C.c_void_p, C.c_int, C.POINTER(abi.Agent), C.c_void_p, C.c_void_p, C.c_void_p,
                                  C.c_void_p]
         L.lo_rollout_info.argtypes = [C.c_void_p, C.c_int, C.POINTER(abi.Agent), C.c_void_p, C.c_void_p, C.c_void_p,
@@ -116,6 +119,24 @@ class Oracle:
 
     def replay(self, n_steps: int):
         self._check(lib().lo_replay(self._h, int(n_steps)))
+
+    def forward_step(self, n_steps: int):
+        """One OrderbookSimulator.forward_step over n_steps grid steps: the resync condition is evaluated once, at the end."""
+        self._check(lib().lo_forward_step(self._h, int(n_steps)))
+
+    def set_book(self, buy: np.ndarray, sell: np.ndarray):
+        """Replace the books by L3 entries in the dump_book format (agent entries also form the internal book)."""
+        buy = np.ascontiguousarray(buy, dtype=abi.BOOK_ENTRY_DTYPE)
+        sell = np.ascontiguousarray(sell, dtype=abi.BOOK_ENTRY_DTYPE)
+        self._check(lib().lo_set_book(self._h, _ptr(buy), len(buy), _ptr(sell), len(sell)))
+
+    def peaks(self) -> dict:
+        """Capacity high-water marks since the last reset_book / reset / set_book, counted like the device book: price levels,
+        resting orders (snapshot aggregates included) and agent orders per side [buy, sell], and the most fills of one call."""
+        out = np.zeros(7, np.int32)
+        lib().lo_peaks(self._h, _ptr(out))
+        return dict(levels=(int(out[0]), int(out[1])), orders=(int(out[2]), int(out[3])), agents=(int(out[4]), int(out[5])),
+                    fills=int(out[6]))
 
     def rollout(self, T: int, agent: abi.Agent, actions=None, want_info=False):
         obs = np.zeros((T, self.obs_dim))

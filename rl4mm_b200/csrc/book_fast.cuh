@@ -352,7 +352,7 @@ __device__ __forceinline__ void fast_resync_level(const FastBook<LT>& fb, FastSt
     return;
   }
   if (nord >= LT::NO) { f.err |= LOBSIM_ERR_ORDER_OVERFLOW; return; }                       // same flags as the general routine
-  if (nlv >= LT::NL) { f.err |= LOBSIM_ERR_LEVEL_OVERFLOW | LOBSIM_ERR_ORDER_OVERFLOW; return; }
+  if (nlv >= LT::NL) { f.err |= LOBSIM_ERR_LEVEL_OVERFLOW; return; }
   const int pos = j > 0 ? (int)fb.LE(sb)[j - 1] : 0;         // the new level's (one-entry) segment starts where level j-1 ends
   __syncwarp();
   for (int base = pos + ((nord - pos + 31) / 32 - 1) * 32; base >= pos; base -= 32) {   // entries [pos, nord) move up by one, descending chunks

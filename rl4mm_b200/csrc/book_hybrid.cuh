@@ -238,7 +238,7 @@ static __device__ __noinline__ uint32_t hyb_leave_fn(unsigned char* blob, int la
     int n_new = 0;
 #pragma unroll
     for (int c = 0; c < HYB_NCH; c++) n_new += __popc(nb[c]);
-    if (cc.x + n_new > LT::NL) { err |= LOBSIM_ERR_LEVEL_OVERFLOW | LOBSIM_ERR_ORDER_OVERFLOW; n_new = LT::NL - cc.x; }   // capacity of the sorted form
+    if (cc.x + n_new > LT::NL) { err |= LOBSIM_ERR_LEVEL_OVERFLOW; n_new = LT::NL - cc.x; }   // capacity of the sorted form
     const unsigned le_mask = 0xffffffffu >> (31 - lane);
 #pragma unroll
     for (int c = 0; c < HYB_NCH; c++) {

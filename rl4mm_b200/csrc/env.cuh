@@ -94,9 +94,11 @@ __device__ __forceinline__ void update_outer_levels_impl(const Book& b, WarpStat
         if (end - start > 1) remove_entries(b, w, side, j, start + 1, end - start - 1);
         if (b.lane == 0) b.ord(side)[start] = make_uint2((unsigned)vol, LOBSIM_REF_AGGREGATE);
         __syncwarp();
-      } else if (NORD(w, side) < b.L.NO && insert_level(b, w, side, j, price)) {
+      } else if (NORD(w, side) >= b.L.NO) {
+        w.err |= LOBSIM_ERR_ORDER_OVERFLOW;
+      } else if (insert_level(b, w, side, j, price)) {   // (a full side: insert_level flags LEVEL_OVERFLOW)
         add_order(b, w, side, j, vol, LOBSIM_REF_AGGREGATE);
-      } else w.err |= LOBSIM_ERR_ORDER_OVERFLOW;
+      }
     }
     if (side == 0) nrepl_buy = nrepl;
   }

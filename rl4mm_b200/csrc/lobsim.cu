@@ -76,6 +76,7 @@ __global__ void __launch_bounds__(32) k_process_orders(const __grid_constant__ O
   Book b; b.blob = smem; b.L = p.L; b.lane = lane;
   WarpState w;
   int cur_env = -1, total_fills = 0;
+  long long inventory_in = 0; double cash_in = 0.0;
   auto load_env = [&](int env) {
     if (p.blob_in_global) b.blob = p.blobs + (size_t)env * p.L.blob_bytes;   // deep-book mode: in place
     else {
@@ -85,10 +86,13 @@ __global__ void __launch_bounds__(32) k_process_orders(const __grid_constant__ O
     }
     __syncwarp();
     load_state<true>(b, w);
+    inventory_in = w.inventory; cash_in = w.cash;
     w.fill_log = p.fills ? p.fills + total_fills : nullptr;
     w.fill_cap = p.max_fills - total_fills; w.n_fills = 0;
   };
   auto store_env = [&](int env) {
+    // Exchange.process_order only returns the fills: the portfolio belongs to the env and moves in its step (HOE.py:280-289)
+    w.inventory = inventory_in; w.cash = cash_in;
     store_state<true>(b, w);
     if (!p.blob_in_global) {
       uint4* dst = reinterpret_cast<uint4*>(p.blobs + (size_t)env * p.L.blob_bytes);

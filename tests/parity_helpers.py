@@ -72,6 +72,37 @@ def cfg_from_env_case(case, n_envs: int = 1, **kw) -> abi.Cfg:
     )
 
 
+CAPACITY_BITS = abi.ERR_LEVEL_OVERFLOW | abi.ERR_ORDER_OVERFLOW | abi.ERR_AGENT_OVERFLOW | abi.ERR_FILL_LOG_FULL
+
+
+def exceeded_bits(peaks: dict, cfg: abi.Cfg) -> int:
+    """The capacity error bits that an unbounded book with these high-water marks (oracle.Oracle.peaks) earns on a device book
+    with the capacities of ``cfg``: more levels, orders or agent orders on a side than it holds, more fills in one call than the
+    fill log holds."""
+    bits = 0
+    if max(peaks["levels"]) > cfg.max_levels_per_side:
+        bits |= abi.ERR_LEVEL_OVERFLOW
+    if max(peaks["orders"]) > cfg.max_orders_per_side:
+        bits |= abi.ERR_ORDER_OVERFLOW
+    if max(peaks["agents"]) > cfg.max_agent_orders:
+        bits |= abi.ERR_AGENT_OVERFLOW
+    if cfg.fill_log_capacity > 0 and peaks["fills"] > cfg.fill_log_capacity:
+        bits |= abi.ERR_FILL_LOG_FULL
+    return bits
+
+
+def capacity_excluded(err, oracle, cfg: abi.Cfg, what="") -> bool:
+    """True when the device flagged a capacity bit for this env, so that it leaves the comparison -- after checking that the flag
+    is justified: the oracle (unbounded) went over at least one capacity since the error bits were last cleared.  A kernel that
+    raised a capacity flag by mistake would otherwise drop the env from the test silently."""
+    bits = int(err) & CAPACITY_BITS
+    if not bits:
+        return False
+    peaks = oracle.peaks()
+    assert exceeded_bits(peaks, cfg), (what, f"capacity bits {bits:#x} without a capacity exceeded", peaks)
+    return True
+
+
 def canon_book(entries: np.ndarray, ext_ids: np.ndarray | None = None):
     """lobsim_book_entry_t[] -> [[price, volume, kind, ext_id]] (kind 0 aggregate, 1 external, 2 agent)."""
     out = []

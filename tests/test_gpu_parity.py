@@ -260,7 +260,8 @@ def rollout_features():
 @pytest.mark.parametrize("agent_kind", ["fixed", "teradactyl", "external", "random"])
 def test_synthetic_rollout_vs_oracle(agent_kind, levels_cap, torch_cuda):
     """Full env path (agent orders, fills, portfolio, features, rewards, resync) on a synthetic SPY-shaped stream.  levels_cap 128
-    = the 128/256/64 layout, whose step / rollout launches run on the flat-only HOT kernel + the DEFERRED kernel (kernels.cuh)."""
+    = the 128/256/64 layout, which the flat form may fill with 128 orders per side (book_flat.cuh); its step / rollout launches run
+    on the classic env kernel (the flat-only HOT + DEFERRED kernels of kernels.cuh are compiled out, csrc/layouts.h)."""
     torch = torch_cuda
     from oracle.oracle import Oracle
     from rl4mm_b200 import synthetic

@@ -66,3 +66,28 @@ def test_episode_stats_shapes():
     assert out.shape == (N, len(STAT_FIELDS)) and out.dtype == torch.float32
     assert out[:, 0].tolist() == rew.sum(0).tolist() and out[:, 6].tolist() == [1, 1, 1]
     assert out[:, 4].tolist() == [12.0, 16.0, 36.0]
+
+
+def test_episode_stats_dev_decodes_state_records_like_episode_stats():
+    """episode_stats_dev reads lobsim_env_state_t records by byte offset (the device path of the collect workload): on hand-built
+    records with every field distinct, it must give what episode_stats computes from the named fields."""
+    from rl4mm_b200 import abi
+    from rl4mm_b200.parallel import episode_stats, episode_stats_dev
+
+    T, N = 4, 5
+    rng = np.random.default_rng(0)
+    rew = torch.tensor(rng.normal(size=(T, N)))
+    done = torch.tensor(rng.integers(0, 2, size=(T, N)), dtype=torch.uint8)
+    st = np.zeros(N, abi.ENV_STATE_DTYPE)
+    for i, name in enumerate(abi.ENV_STATE_DTYPE.names):     # a distinct non-zero value in every field, so a wrong offset shows
+        st[name] = (np.arange(N) + 1 + 10 * i).reshape((N,) + (1,) * (st[name].ndim - 1))
+    st["inventory"] = [-7, 0, 3, 120, -40]
+    st["cash"] = [1e6, -2.5e3, 0.0, 7.25, 1e9]
+    st["price"] = [101.5, 99.0, np.nan, 1e4, 0.5]
+    st["err"] = [0, abi.ERR_EMPTY_BOOK, abi.ERR_AGENT_OVERFLOW | abi.ERR_FILL_LOG_FULL, 0, abi.ERR_BAD_ACTION]
+    spread = torch.tensor(rng.uniform(1, 5, size=(T, N)))
+    state_dev = torch.from_numpy(st.view(np.uint8).reshape(N, abi.ENV_STATE_DTYPE.itemsize).copy())
+    want = episode_stats(rew, done, st, spread)
+    got = episode_stats_dev(rew, done, state_dev, spread)
+    assert torch.equal(torch.isnan(want), torch.isnan(got))
+    assert torch.equal(torch.nan_to_num(want), torch.nan_to_num(got)), (want, got)
