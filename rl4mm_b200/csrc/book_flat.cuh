@@ -108,7 +108,12 @@ __device__ __forceinline__ bool flat_order(unsigned char* blob, int lane, FastSt
   uint4* opp = flat_pool<LT>(blob, OPP);
   FastBook<LT> fb; fb.blob = blob; fb.lane = lane;
   if (VCHK && __builtin_expect(vol <= 0, 0)) { f.err |= LOBSIM_ERR_BAD_VOLUME; return false; }   // assert order.volume > 0, Exchange.py:59-60
-  __syncwarp();                                                             // (!VCHK: the caller has checked the volume)
+  // (!VCHK: the caller has checked the volume)
+  // Pool stores: tracked, lane 0 stores and a warp barrier orders its stores against the other lanes' loads.  Untracked (replay),
+  // every lane stores the same value to the same address, so each lane's own later loads see it whatever the other lanes do, and
+  // the paths need no barrier (control flow is warp-uniform: every value it depends on is the same in all lanes).
+  const bool wr = !TR || lane == 0;
+  if (TR) __syncwarp();
   // ---- the order rests at the back of its price's queue (Exchange.py:74-83) --------------------------------------------
   auto rest = [&](int rem) -> bool {
     if (TR && is_agent) {   // OrderIdConvertor.add_internal_id_to_order_and_track + internal book append
@@ -124,7 +129,7 @@ __device__ __forceinline__ bool flat_order(unsigned char* blob, int lane, FastSt
         h->nag[S] = nag + 1; h->next_agent_id = id + 1;
       }
     }
-    if (lane == 0) own[n_own] = make_uint4((unsigned)price, ref, (unsigned)rem, st.seq);
+    if (wr) own[n_own] = make_uint4((unsigned)price, ref, (unsigned)rem, st.seq);
     n_own += 1; st.seq += 1;
     if (S ? price < best_own : price > best_own) best_own = price;
     return false;
@@ -150,15 +155,15 @@ __device__ __forceinline__ bool flat_order(unsigned char* blob, int lane, FastSt
       aggregate = true;
     }
     const int cur = (int)own[i].z;
-    __syncwarp();
+    if (TR) __syncwarp();
     if (vol < cur) {                                                         // partial: reduce in place
-      if (lane == 0) own[i].z = (unsigned)(cur - vol);
+      if (wr) own[i].z = (unsigned)(cur - vol);
       if (TR && is_agent && !aggregate) { __syncwarp(); fast_agent_reduce(fb, S, ref & 0x7fffffffu, vol, false); }
       return false;
     }
     // full removal (over-size requests remove the resting volume, :142-146): the last order of the pool fills the hole
     if (price == best_own) best_own = flat_best_of<S>(k, n_own, lane, i);
-    if (lane == 0) own[i] = own[n_own - 1];
+    if (wr) own[i] = own[n_own - 1];
     n_own -= 1;
     if (TR && is_agent && !aggregate) { __syncwarp(); fast_agent_reduce(fb, S, ref & 0x7fffffffu, cur, true); }
     return false;
@@ -213,8 +218,8 @@ __device__ __forceinline__ bool flat_order(unsigned char* blob, int lane, FastSt
             if (is_agent) fast_record(fb, f, 0, S, bp, v, 1, href);         // the synthetic MarketOrder fill, :111-115
           }
           if (rem < hv) {                                                  // partial fill of the head
-            __syncwarp();
-            if (lane == 0) opp[i].z = (unsigned)(hv - rem);
+            if (TR) __syncwarp();
+            if (wr) opp[i].z = (unsigned)(hv - rem);
             if (TR && hagent) { __syncwarp(); fast_agent_reduce(fb, OPP, href & 0x7fffffffu, rem, false); }
             rem = 0;
             break;
@@ -226,10 +231,10 @@ __device__ __forceinline__ bool flat_order(unsigned char* blob, int lane, FastSt
           flat_keys(opp, n_opp, lane, k);
           best_opp = flat_best_of<OPP>(k, n_opp, lane, i);
         }
-        __syncwarp();
-        if (lane == 0) opp[i] = opp[n_opp - 1];
+        if (TR) __syncwarp();
+        if (wr) opp[i] = opp[n_opp - 1];
         n_opp -= 1;
-        __syncwarp();
+        if (TR) __syncwarp();
         if (TR && hagent) fast_agent_reduce(fb, OPP, href & 0x7fffffffu, 0, true);   // the resting agent order is gone
       }
     }

@@ -792,16 +792,20 @@ __global__ void __launch_bounds__(128, LOBSIM_REPLAY_FLAT_MIN_BLOCKS) k_replay_f
   const int steps_per_sec = ec.steps_per_sec;
   int sub = now_step >= 0 ? now_step % steps_per_sec : 0;
 
+  // One pass per second, or per part of a second where the launch (T) or the stream begins or ends inside one: a replay book holds
+  // no agent orders, so nothing happens at a step boundary that is not a second boundary, and the message segments run across
+  // steps.  now_step advances by the steps a pass covered; where a book dies, it is recovered from the step offsets of that pass.
 #pragma unroll 1
-  for (int t = 0; t < T && !f.dead; t++) {
-    if (now_step >= n_grid) { f.err |= LOBSIM_ERR_END_OF_STREAM; f.dead = 1; break; }
-    const unsigned g_step_end = __ldg(&st_step_off[now_step + 1]);
+  for (int t = 0; t < T && !f.dead;) {
+    const int k = min(min(steps_per_sec - sub, T - t), n_grid - now_step);   // steps of this pass
+    if (k <= 0) { f.err |= LOBSIM_ERR_END_OF_STREAM; f.dead = 1; break; }
+    const unsigned g_pass_end = __ldg(&st_step_off[now_step + k]);
 #pragma unroll 1
-    while (g < g_step_end) {
+    while (g < g_pass_end) {
       const unsigned tile = g / MSG_TILE - tile0;
       if (tile == next_wait) wait_tile();
       const unsigned tile_end = (g / MSG_TILE + 1) * MSG_TILE;
-      const unsigned lim = g_step_end < tile_end ? g_step_end : tile_end;
+      const unsigned lim = g_pass_end < tile_end ? g_pass_end : tile_end;
       const uint4* mp = reinterpret_cast<const uint4*>(msgbuf + (tile & 1) * MSG_TILE_BYTES) + (g % MSG_TILE);
       const unsigned cnt = lim - g;
       unsigned i = 0;
@@ -832,15 +836,18 @@ __global__ void __launch_bounds__(128, LOBSIM_REPLAY_FLAT_MIN_BLOCKS) k_replay_f
           if (f.dead) break;
         }
       }
-      if (f.dead) break;
+      if (f.dead) { g += i; break; }                        // g: the message the book died of
       g = lim;
       if (g == tile_end) { __syncwarp(); issue_tile(); }
     }
-    if (f.dead) break;
-    now_step++;
-    if (++sub == steps_per_sec) {                            // whole second: outer-level resync, OrderbookSimulator.py:86-87
+    if (f.dead) {                                            // now_step: the step that holds message g (a step without messages holds none)
+      while (__ldg(&st_step_off[now_step + 1]) <= g) now_step++;
+      break;
+    }
+    now_step += k; t += k; sub += k;
+    if (sub == steps_per_sec) {                              // whole second: outer-level resync, OrderbookSimulator.py:86-87
       sub = 0;
-      if (c.resync && (!p.resync_last_only || t == T - 1)) {
+      if (c.resync && (!p.resync_last_only || t == T)) {
         const double prop = ec.outer_prop;
         const double bb = f.best0 == INT32_MIN ? 0.0 : (double)f.best0;
         const double bs = f.best1 == INT32_MAX ? (double)INFINITY : (double)f.best1;
