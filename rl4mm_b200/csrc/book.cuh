@@ -81,8 +81,6 @@ struct WarpState {
   int fill_cap, n_fills;
 };
 
-static_assert(sizeof(WarpState) <= 128, "WarpState must fit the 128-byte per-warp shared slot");
-
 struct Book {
   unsigned char* blob; // shared memory
   Layout L;

@@ -17,12 +17,12 @@
 // FLAT_CAP = 32 * NCH orders per side, NCH = 2 or 4 chunks by the handle's capacities (flat_nch<LT>): a flat side may hold
 // FLAT_CAP distinct prices, so the sorted layout must have room for as many levels, and the pool lives in the side's order array.
 //
-// A book is flat or sorted PER BOOK: in shared memory during a launch, and in HBM between launches (header marker, kernels.cuh) --
-// one launch is one env step when a policy runs in between, so converting per launch would cost more than the flat path saves.
+// The flat form is the replay's (k_replay_flat, kernels.cuh).  A book is flat or sorted PER BOOK: in shared memory during a launch,
+// and in HBM between launches (header marker, kernels.cuh), so that consecutive replay launches do not convert every book twice each.
 // Conversions: flat_enter (sorted -> flat: trivial, seq = position in the sorted order array) when a book fits with some slack;
 // flat_leave (flat -> sorted: rank-by-counting sort on (price, seq)) when a pool is full, when update_outer_levels
-// (OrderbookSimulator.py:105-135) really has a level to overwrite (leave -> resync on the sorted form -> enter), and by k_to_sorted
-// before anything outside the straight-line kernels reads a book.
+// (OrderbookSimulator.py:105-135) really has a level to overwrite (leave -> resync on the sorted form -> enter), on load by the env
+// and hybrid replay kernels, and by k_to_sorted before anything else reads a book.
 #pragma once
 #include "book_fast.cuh"
 
@@ -88,48 +88,30 @@ __device__ __forceinline__ int flat_best_scan(unsigned char* blob, int lane, int
   return flat_best_of<S>(k, n, lane, -1);
 }
 
-// One order of side S (0 buy, 1 sell) through the flat book.  Same results as fast_order_full<LT,TR> on the sorted book; TR: fills /
-// flows / the agent's order tables are tracked (env kernels), exactly as in book_fast.cuh.
+// One historical order of side S (0 buy, 1 sell) through the flat book.  Same results as fast_order_full<LT,false> on the sorted book:
+// a replay book holds no agent orders, so nothing is tracked.
 // Sets f.bail = FLAT_BAIL_FULL -- with the book untouched -- when the order may have to rest and the pool of its side is full: the
 // caller converts the book to the sorted form and runs the order there.  Returns true when the caller's message loop has to stop
 // (f.bail or f.dead set) -- a constant per return site, so the compiler threads the rare exits straight out of the loop and the
 // common paths carry no status register.
 #define FLAT_BAIL_FULL 3
-template <class LT, int S, bool TR, bool VCHK = true>
-__device__ __forceinline__ bool flat_order(unsigned char* blob, int lane, FastState& f, FlatState& st, int type, int price, int vol, uint32_t ref, bool is_agent) {
+template <class LT, int S, bool VCHK = true>
+__device__ __forceinline__ bool flat_order(unsigned char* blob, int lane, FastState& f, FlatState& st, int type, int price, int vol, uint32_t ref) {
   constexpr int OPP = S ^ 1;
   constexpr int NCH = flat_nch<LT>();
-  if (!TR) is_agent = false;
   int& n_own = S ? st.n1 : st.n0;
   int& n_opp = S ? st.n0 : st.n1;
   int& best_own = S ? f.best1 : f.best0;
   int& best_opp = S ? f.best0 : f.best1;
   uint4* own = flat_pool<LT>(blob, S);
   uint4* opp = flat_pool<LT>(blob, OPP);
-  FastBook<LT> fb; fb.blob = blob; fb.lane = lane;
   if (VCHK && __builtin_expect(vol <= 0, 0)) { f.err |= LOBSIM_ERR_BAD_VOLUME; return false; }   // assert order.volume > 0, Exchange.py:59-60
   // (!VCHK: the caller has checked the volume)
-  // Pool stores: tracked, lane 0 stores and a warp barrier orders its stores against the other lanes' loads.  Untracked (replay),
-  // every lane stores the same value to the same address, so each lane's own later loads see it whatever the other lanes do, and
-  // the paths need no barrier (control flow is warp-uniform: every value it depends on is the same in all lanes).
-  const bool wr = !TR || lane == 0;
-  if (TR) __syncwarp();
+  // Pool stores: every lane stores the same value to the same address, so each lane's own later loads see it whatever the other
+  // lanes do, and the paths need no barrier (control flow is warp-uniform: every value it depends on is the same in all lanes).
   // ---- the order rests at the back of its price's queue (Exchange.py:74-83) --------------------------------------------
   auto rest = [&](int rem) -> bool {
-    if (TR && is_agent) {   // OrderIdConvertor.add_internal_id_to_order_and_track + internal book append
-      BookHdr* h = reinterpret_cast<BookHdr*>(blob);
-      const int nag = h->nag[S];
-      if (nag >= LT::NA) { f.err |= LOBSIM_ERR_AGENT_OVERFLOW; return false; }
-      const uint32_t id = h->next_agent_id;
-      ref = LOBSIM_REF_AGENT | id;
-      __syncwarp();
-      if (lane == 0) {
-        int32_t* ap = reinterpret_cast<int32_t*>(blob + LT::agent_off + S * LT::NA * 12);
-        ap[nag] = price; ap[LT::NA + nag] = rem; reinterpret_cast<uint32_t*>(ap)[2 * LT::NA + nag] = id;
-        h->nag[S] = nag + 1; h->next_agent_id = id + 1;
-      }
-    }
-    if (wr) own[n_own] = make_uint4((unsigned)price, ref, (unsigned)rem, st.seq);
+    own[n_own] = make_uint4((unsigned)price, ref, (unsigned)rem, st.seq);
     n_own += 1; st.seq += 1;
     if (S ? price < best_own : price > best_own) best_own = price;
     return false;
@@ -143,7 +125,6 @@ __device__ __forceinline__ bool flat_order(unsigned char* blob, int lane, FastSt
 #pragma unroll
     for (int c = 0; c < NCH; c++) if (c * 32 + lane < n_own && (int)k[c].x == price && k[c].y == ref) mine = c * 32 + lane;
     int i = __reduce_max_sync(FULL_MASK, mine);
-    bool aggregate = false;
     if (i < 0) {
       // unknown id: the level's snapshot aggregate (internal_id -1, always the head of its level) takes the hit (:133-137);
       // no such level, or no aggregate left at it: nothing happens (:129-132,138-139)
@@ -152,20 +133,16 @@ __device__ __forceinline__ bool flat_order(unsigned char* blob, int lane, FastSt
       for (int c = NCH - 1; c >= 0; c--) if (c * 32 + lane < n_own && (int)k[c].x == price && k[c].y == LOBSIM_REF_AGGREGATE) mine = c * 32 + lane;
       i = __reduce_min_sync(FULL_MASK, mine);
       if (i == INT32_MAX) return false;
-      aggregate = true;
     }
     const int cur = (int)own[i].z;
-    if (TR) __syncwarp();
     if (vol < cur) {                                                         // partial: reduce in place
-      if (wr) own[i].z = (unsigned)(cur - vol);
-      if (TR && is_agent && !aggregate) { __syncwarp(); fast_agent_reduce(fb, S, ref & 0x7fffffffu, vol, false); }
+      own[i].z = (unsigned)(cur - vol);
       return false;
     }
     // full removal (over-size requests remove the resting volume, :142-146): the last order of the pool fills the hole
     if (price == best_own) best_own = flat_best_of<S>(k, n_own, lane, i);
-    if (wr) own[i] = own[n_own - 1];
+    own[i] = own[n_own - 1];
     n_own -= 1;
-    if (TR && is_agent && !aggregate) { __syncwarp(); fast_agent_reduce(fb, S, ref & 0x7fffffffu, cur, true); }
     return false;
   };
   // dispatch, the common cases first: a limit order that neither crosses nor finds the pool full, then cancellations / deletions.
@@ -205,37 +182,20 @@ __device__ __forceinline__ bool flat_order(unsigned char* blob, int lane, FastSt
           at_best += __popc(__ballot_sync(FULL_MASK, q[c] != 0xffffffffu));
         }
         const int i = __reduce_max_sync(FULL_MASK, head);                                       // the head of the best queue
-        const uint4 he = opp[i];
-        const int hv = (int)he.z;
-        const uint32_t href = he.y;
-        const bool hagent = TR && (href & LOBSIM_REF_AGENT) != 0;
-        const bool self_match = TR && is_agent && hagent;                  // cannot fill our own order => delete it, :91-94
-        if (!self_match) {
-          const int v = rem < hv ? rem : hv;
-          if (TR) {
-            if (hagent) fast_record(fb, f, 0, OPP, bp, v, 0, href);
-            else fast_record(fb, f, 1, OPP, bp, v, 0, href);
-            if (is_agent) fast_record(fb, f, 0, S, bp, v, 1, href);         // the synthetic MarketOrder fill, :111-115
-          }
-          if (rem < hv) {                                                  // partial fill of the head
-            if (TR) __syncwarp();
-            if (wr) opp[i].z = (unsigned)(hv - rem);
-            if (TR && hagent) { __syncwarp(); fast_agent_reduce(fb, OPP, href & 0x7fffffffu, rem, false); }
-            rem = 0;
-            break;
-          }
-          rem -= hv;                                                       // the head is consumed
+        const int hv = (int)opp[i].z;
+        if (rem < hv) {                                                    // partial fill of the head
+          opp[i].z = (unsigned)(hv - rem);
+          rem = 0;
+          break;
         }
+        rem -= hv;                                                         // the head is consumed
         if (at_best == 1) {                                                // the level emptied: next best price
           uint2 k[NCH];
           flat_keys(opp, n_opp, lane, k);
           best_opp = flat_best_of<OPP>(k, n_opp, lane, i);
         }
-        if (TR) __syncwarp();
-        if (wr) opp[i] = opp[n_opp - 1];
+        opp[i] = opp[n_opp - 1];
         n_opp -= 1;
-        if (TR) __syncwarp();
-        if (TR && hagent) fast_agent_reduce(fb, OPP, href & 0x7fffffffu, 0, true);   // the resting agent order is gone
       }
     }
     if (!(rem > 0 && type == LOBSIM_MSG_LIMIT)) return false;
@@ -249,28 +209,8 @@ __device__ __forceinline__ bool flat_order(unsigned char* blob, int lane, FastSt
 template <class LT, bool VCHK = true>
 __device__ __forceinline__ bool flat_message(unsigned char* blob, int lane, FastState& f, FlatState& st, int price, int vol, uint32_t ref, uint32_t meta) {
   const int type = (int)(meta & 7u);
-  if (meta & 8u) return flat_order<LT, 1, false, VCHK>(blob, lane, f, st, type, price, vol, ref, false);
-  return flat_order<LT, 0, false, VCHK>(blob, lane, f, st, type, price, vol, ref, false);
-}
-// the tracked form (env kernels): historical messages and the agent's own orders; false: pool full (see flat_order)
-template <class LT>
-__device__ __forceinline__ bool flat_order_tracked(unsigned char* blob, int lane, FastState& f, FlatState& st, int type, int side, int price, int vol, uint32_t ref, bool is_agent) {
-  if (side) flat_order<LT, 1, true>(blob, lane, f, st, type, price, vol, ref, is_agent);
-  else flat_order<LT, 0, true>(blob, lane, f, st, type, price, vol, ref, is_agent);
-  if (f.bail) { f.bail = 0; return false; }
-  return true;
-}
-
-// volume resting at the best price of side S (Orderbook.best_buy_volume / best_sell_volume, models.py:80-85)
-template <class LT, int S>
-__device__ __forceinline__ int flat_best_volume(unsigned char* blob, int lane, const FastState& f, const FlatState& st) {
-  const int n = S ? st.n1 : st.n0, best = S ? f.best1 : f.best0;
-  const uint4* pool = flat_pool<LT>(blob, S);
-  int v = 0;
-#pragma unroll
-  for (int c = 0; c < flat_nch<LT>(); c++)
-    if (c * 32 + lane < n) { const uint4 e = pool[c * 32 + lane]; if ((int)e.x == best) v += (int)e.z; }
-  return __reduce_add_sync(FULL_MASK, v);
+  if (meta & 8u) return flat_order<LT, 1, VCHK>(blob, lane, f, st, type, price, vol, ref);
+  return flat_order<LT, 0, VCHK>(blob, lane, f, st, type, price, vol, ref);
 }
 
 // ---- sorted -> flat (kernel entry, after a reset / resync, when a book has shrunk) ----------------------------------------------

@@ -26,33 +26,16 @@ static cudaError_t set_attr(const void* k, int dyn) {
   return cudaFuncSetAttribute(k, cudaFuncAttributePreferredSharedMemoryCarveout, cudaSharedmemCarveoutMaxShared);
 }
 
-// layouts whose env launches run on the flat-only HOT kernel + the DEFERRED kernel (kernels.cuh ENV_HOT): the one layout whose books
-// (10-level history + the agent's ladders) practically always fit the 128-order pools
-constexpr bool kEnvHot = LOBSIM_LAYOUT_ENV_HOT(LT::NL, LT::NO, LT::NA);
-
 template <bool RARE>
 static cudaError_t env_attrs(int dyn_env) {
-  cudaError_t e = set_attr((const void*)k_env_fast<LT, true, RARE, ENV_CLASSIC>, dyn_env);
-  if (e == cudaSuccess) e = set_attr((const void*)k_env_fast<LT, false, RARE, ENV_CLASSIC>, dyn_env);
-  if constexpr (kEnvHot) {
-    if (e == cudaSuccess) e = set_attr((const void*)k_env_fast<LT, true, RARE, ENV_HOT>, dyn_env);
-    if (e == cudaSuccess) e = set_attr((const void*)k_env_fast<LT, false, RARE, ENV_HOT>, dyn_env);
-    if (e == cudaSuccess) e = set_attr((const void*)k_env_fast<LT, false, RARE, ENV_DEFERRED>, dyn_env);
-  }
+  cudaError_t e = set_attr((const void*)k_env_fast<LT, true, RARE>, dyn_env);
+  if (e == cudaSuccess) e = set_attr((const void*)k_env_fast<LT, false, RARE>, dyn_env);
   return e;
 }
 template <bool RARE>
-static void env_launch(int mode, bool sync, int grid, int block, size_t dyn, cudaStream_t stream, const AdvParams& p, const EnvConst& ec) {
-  if constexpr (kEnvHot) {
-    if (mode == ENV_HOT) {
-      if (sync) k_env_fast<LT, true, RARE, ENV_HOT><<<grid, block, dyn, stream>>>(p, ec);
-      else k_env_fast<LT, false, RARE, ENV_HOT><<<grid, block, dyn, stream>>>(p, ec);
-      return;
-    }
-    if (mode == ENV_DEFERRED) { k_env_fast<LT, false, RARE, ENV_DEFERRED><<<grid, block, dyn, stream>>>(p, ec); return; }
-  }
-  if (sync) k_env_fast<LT, true, RARE, ENV_CLASSIC><<<grid, block, dyn, stream>>>(p, ec);
-  else k_env_fast<LT, false, RARE, ENV_CLASSIC><<<grid, block, dyn, stream>>>(p, ec);
+static void env_launch(bool sync, int grid, int block, size_t dyn, cudaStream_t stream, const AdvParams& p, const EnvConst& ec) {
+  if (sync) k_env_fast<LT, true, RARE><<<grid, block, dyn, stream>>>(p, ec);
+  else k_env_fast<LT, false, RARE><<<grid, block, dyn, stream>>>(p, ec);
 }
 
 #if LOBSIM_TU_PART == 0
@@ -77,12 +60,12 @@ void FN(_to_sorted)(unsigned char* blobs, int n_envs, cudaStream_t stream) {
   const int wpc = 4 * LT::blob_bytes <= 227 * 1024 ? 4 : 1;
   k_to_sorted<LT><<<(n_envs + wpc - 1) / wpc, wpc * 32, (size_t)wpc * LT::blob_bytes, stream>>>(blobs, n_envs);
 }
-void FN(_env)(int mode, bool sync, int grid, int block, size_t dyn, cudaStream_t stream, const AdvParams& p, const EnvConst& ec) {
-  env_launch<false>(mode, sync, grid, block, dyn, stream, p, ec);
+void FN(_env)(bool sync, int grid, int block, size_t dyn, cudaStream_t stream, const AdvParams& p, const EnvConst& ec) {
+  env_launch<false>(sync, grid, block, dyn, stream, p, ec);
 }
 #else
 cudaError_t FN(_attrs_rare)(int dyn_env) { return env_attrs<true>(dyn_env); }
-void FN(_env_rare)(int mode, bool sync, int grid, int block, size_t dyn, cudaStream_t stream, const AdvParams& p, const EnvConst& ec) {
-  env_launch<true>(mode, sync, grid, block, dyn, stream, p, ec);
+void FN(_env_rare)(bool sync, int grid, int block, size_t dyn, cudaStream_t stream, const AdvParams& p, const EnvConst& ec) {
+  env_launch<true>(sync, grid, block, dyn, stream, p, ec);
 }
 #endif

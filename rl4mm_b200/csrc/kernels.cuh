@@ -65,9 +65,6 @@ __device__ __forceinline__ void tma_store_wait() { asm volatile("cp.async.bulk.w
 // ====================================================================================================================
 //  kernel parameters
 // ====================================================================================================================
-#ifndef LOBSIM_WS_IN_SMEM
-#define LOBSIM_WS_IN_SMEM 0
-#endif
 #ifndef LOBSIM_ENV_MIN_BLOCKS
 #define LOBSIM_ENV_MIN_BLOCKS 3
 #endif
@@ -102,8 +99,6 @@ struct AdvParams {
   int32_t out_final_obs_only;       // reset: write obs once, after the warm-up
   int32_t resync_last_only;         // forward_step over several grid steps: resync check only at the end
   int32_t blob_in_global;           // deep books: the blob does not fit in the shared memory of an SM and is worked on in place in HBM / L2
-  int32_t* defer_count;             // env HOT kernel: number of (env, step) items handed to the deferred kernel
-  int2* defer_list;                 // [n_sel] {selection index, env step to resume at}
   int32_t hybrid;                   // deep layouts: the replay launch runs k_replay_hyb (book_hybrid.cuh); blobs stay sorted in HBM
   int32_t allow_flat;               // fast kernels: books that fit run on -- and are stored in -- the flat order pools (book_flat.cuh)
   const double* actions_in;         // EXTERNAL: [T][n_sel][action_dim]
@@ -192,13 +187,7 @@ __global__ void __launch_bounds__(128, kEnv ? LOBSIM_ENV_MIN_BLOCKS : 4) k_advan
   __syncwarp();
   if (!p.blob_in_global) mbar_wait(&bars[2], 0);
 
-#if LOBSIM_WS_IN_SMEM
-  // the uniform per-warp state lives in shared memory (not registers): every lane stores identical values, so plain
-  // accesses are race-free; it trades a few broadcast LDS for ~35 registers per thread => more resident books per SM
-  WarpState& w = *reinterpret_cast<WarpState*>(reinterpret_cast<unsigned char*>(bars) + 32);
-#else
   WarpState w;
-#endif
   load_state<kTrack>(b, w);
   w.fill_log = p.fill_log ? p.fill_log + (size_t)env * p.fill_cap : nullptr;
   w.fill_cap = p.fill_cap; w.n_fills = 0;
@@ -662,7 +651,8 @@ __global__ void __launch_bounds__(128, 3) k_replay_hyb(const __grid_constant__ A
 
 // ---- the flat form of a blob in HBM (book_flat.cuh): header with cnt[0] = {-1, n0}, cnt[1] = {seq, n1}; per side the order pool
 //      (n x 16 B at the start of the side's order array); the agent tables as always.  Parts: lanes 0-1 the pools, 2-7 the agent tables.
-template <class LT, bool LOAD>
+//      Loads the body of a flat blob whose header is in shared memory; returns the bytes expected on `bar` (0: nothing was issued).
+template <class LT>
 __device__ __forceinline__ uint32_t flat_body_copy(unsigned char* sm, unsigned char* gm, uint64_t* bar, int lane, int n0, int n1) {
   const BookHdr* h = reinterpret_cast<const BookHdr*>(sm);
   uint32_t off = 0, len = 0;
@@ -674,8 +664,9 @@ __device__ __forceinline__ uint32_t flat_body_copy(unsigned char* sm, unsigned c
   }
   const uint32_t total = __reduce_add_sync(FULL_MASK, len);
   if (total == 0) return 0;
-  if (LOAD) { if (lane == 0) mbar_expect_tx(bar, total); __syncwarp(); }
-  if (len) { if (LOAD) tma_load(sm + off, gm + off, len, bar); else tma_store_part(gm + off, sm + off, len); }
+  if (lane == 0) mbar_expect_tx(bar, total);
+  __syncwarp();
+  if (len) tma_load(sm + off, gm + off, len, bar);
   return total;
 }
 // FlatState of a flat blob whose header and pools are in shared memory; the best prices are recomputed from the pools
@@ -939,53 +930,21 @@ constexpr int env_min_blocks() {
   const int fit = (227 * 1024) / (LOBSIM_ENVFAST_WARPS * warp_bytes);
   return fit < 1 ? 1 : (fit < LOBSIM_ENVFAST_MINB ? fit : LOBSIM_ENVFAST_MINB);
 }
-#ifndef LOBSIM_PHASE_SYNC
-#define LOBSIM_PHASE_SYNC 1
-#endif
-// MODE of k_env_fast:
-//   ENV_CLASSIC  -- the sorted level arrays of book_fast.cuh with every rare path in the kernel; flat blobs are converted on load.
-//   ENV_HOT      -- flat order pools ONLY (book_flat.cuh): no sorted order path, no any-depth routines, no flat_leave, no tracked
-//                   resync in the kernel.  A book that does not fit the pools, a pool that fills up, or an update_outer_levels with a
-//                   level to overwrite makes the warp ABORT the env step: nothing of it has reached HBM (the blob is stored only
-//                   at step ends, the feature state is written in phase C), so the env is handed -- {selection index, step} in
-//                   p.defer_list -- to the ENV_DEFERRED launch that follows, which redoes that step and the rest of the launch.
-//   ENV_DEFERRED -- ENV_CLASSIC over the items of p.defer_list (usually none: the launch exits at once).
-// Why: the env kernel is bound by instruction fetch, not issue slots (profiles/r02_env_ab.txt): the flat path next to the sorted path
-// in one kernel is 16 % slower than the sorted path alone, the flat path ALONE is 6 % faster (and 11 % fewer instructions).
-#define ENV_CLASSIC 0
-#define ENV_HOT 1
-#define ENV_DEFERRED 2
-#ifndef LOBSIM_SYNC_B
-#define LOBSIM_SYNC_B 1           // barrier between phase A (ladders) and phase B (orders)
-#endif
-#ifndef LOBSIM_SYNC_C
-#define LOBSIM_SYNC_C 1           // barrier between phase B (orders) and phase C (features, reward)
-#endif
-#if LOBSIM_PHASE_SYNC
-#define PHASE_SYNC() __syncthreads()
-#else
-#define PHASE_SYNC() ((void)0)
-#endif
 // SYNC: the launch consists of full CTAs only, whose warps move through the phases of a step together
 // (launch_env puts the n_sel % warps-per-CTA tail into a second, free-running launch).
 // Per-warp values that are only needed outside the order-processing phase (B) live in the spare shared memory behind the
 // mbarriers instead of in registers: the kernel is register-bound (128 registers at 16 resident warps per SM) and phase B is where it spills.
 struct StepSave { double cash0, p0, price; long long inv0, episode_start_us, st_t0_us; };
+static_assert(sizeof(StepSave) <= 128, "StepSave must fit the 128-byte per-warp slot behind the mbarriers (warp_smem_bytes)");
 // RARE: the configuration uses z-score normalisation or a RollingSharpe reward (their code is compiled out otherwise).
-template <class LT, bool SYNC, bool RARE, int MODE>
+template <class LT, bool SYNC, bool RARE>
 __global__ void __launch_bounds__(32 * LOBSIM_ENVFAST_WARPS, env_min_blocks<LT>()) k_env_fast(const __grid_constant__ AdvParams p, const __grid_constant__ EnvConst ec) {
   extern __shared__ __align__(128) unsigned char smem[];
   const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
-  // The warps of a CTA move through the phases of a step together (PHASE_SYNC = __syncthreads): the instruction
+  // The warps of a CTA move through the phases of a step together (SYNC: a __syncthreads between phases): the instruction
   // working set at any moment is a single phase, which is what keeps the 32 KB L1.5 I-cache warm
   // (profiles/r01_envstep_*: "no instruction" was the top stall with free-running warps).
-  int sel = p.sel_offset + blockIdx.x * (blockDim.x >> 5) + warp, t_start = 0;
-  if (MODE == ENV_DEFERRED) {
-    static_assert(MODE != ENV_DEFERRED || !SYNC, "the deferred launch has no block-level barriers");
-    if (sel >= *p.defer_count) return;
-    const int2 item = p.defer_list[sel];
-    sel = item.x; t_start = item.y;
-  }
+  const int sel = p.sel_offset + blockIdx.x * (blockDim.x >> 5) + warp;
   if (sel >= p.n_sel) return; // only in SYNC == false launches
   const int env = p.env_ids ? p.env_ids[sel] : sel;
   const lobsim_cfg_t& c = ec.cfg;
@@ -1007,18 +966,12 @@ __global__ void __launch_bounds__(32 * LOBSIM_ENVFAST_WARPS, env_min_blocks<LT>(
   FastBook<LT> fb; fb.blob = base; fb.lane = lane;
   Book b; b.blob = base; b.L = p.L; b.lane = lane;
   BookHdr* h = reinterpret_cast<BookHdr*>(base);
-  // flat: the book is in the flat order pools of book_flat.cuh (every book that fits them, when the handle allows it) -- in shared
-  // memory during the launch AND in HBM between launches (one launch = one env step when a policy runs in between, so a
-  // conversion per launch would cost more than the flat order path saves)
-  bool flat = false;
-  bool aborted = false;                                  // ENV_HOT: this env step goes to the deferred launch
-  FlatState fs; fs.n0 = fs.n1 = 0; fs.seq = 0;
-  auto defer = [&](int t) { aborted = true; if (lane == 0) { const int k = atomicAdd(p.defer_count, 1); p.defer_list[k] = make_int2(sel, t); } };
+  // a blob in the flat form of book_flat.cuh (stored by k_replay_flat) is converted to the sorted level arrays on load: this kernel
+  // runs on the sorted form only
   if (!p.reset_mode) {
     if (hdr_is_flat(h)) {
-      if (flat_body_copy<LT, true>(base, gblob, &bars[2], lane, h->cnt[0][1], h->cnt[1][1])) mbar_wait(&bars[2], 1);
-      if (MODE == ENV_HOT) flat = true;
-      else flat_leave_fn<LT>(base, lane, h->cnt[0][1], h->cnt[1][1]);     // the sorted kernels convert a flat blob on load
+      if (flat_body_copy<LT>(base, gblob, &bars[2], lane, h->cnt[0][1], h->cnt[1][1])) mbar_wait(&bars[2], 1);
+      flat_leave_fn<LT>(base, lane, h->cnt[0][1], h->cnt[1][1]);
     } else if (blob_body_copy<LT, true>(base, gblob, &bars[2], lane)) mbar_wait(&bars[2], 1);
   }
   FastState f; f.err = h->err; f.dead = h->dead; f.bail = 0; f.bail_vol = 0;
@@ -1041,14 +994,7 @@ __global__ void __launch_bounds__(32 * LOBSIM_ENVFAST_WARPS, env_min_blocks<LT>(
     }
     __syncwarp();
   }
-  if (MODE == ENV_HOT && flat) flat_adopt<LT>(base, lane, f, fs);
-  else {
-    fast_refresh_best(fb, f);
-    if (MODE == ENV_HOT) {
-      if (flat_fits(fb, 8)) { flat_enter(fb, fs); flat = true; }
-      else defer(0);                                       // too many resting orders for the pools: the sorted kernel takes this env
-    }
-  }
+  fast_refresh_best(fb, f);
   const lobsim_stream_t* stp = &p.streams[stream_id];
   const lobsim_msg_t* __restrict__ st_msgs = stp->msgs;
   const uint32_t* __restrict__ st_step_off = stp->step_off;
@@ -1068,8 +1014,7 @@ __global__ void __launch_bounds__(32 * LOBSIM_ENVFAST_WARPS, env_min_blocks<LT>(
     if (v.have_tops) {
       v.bb = f.best0; v.bs = f.best1;
       __syncwarp();
-      if (MODE == ENV_HOT) { v.bv = flat_best_volume<LT, 0>(base, lane, f, fs); v.sv = flat_best_volume<LT, 1>(base, lane, f, fs); }
-      else { v.bv = best_level_volume(b, 0, h->cnt[0][0]); v.sv = best_level_volume(b, 1, h->cnt[1][0]); }
+      v.bv = best_level_volume(b, 0, h->cnt[0][0]); v.sv = best_level_volume(b, 1, h->cnt[1][0]);
       double imb; v.price = microprice(v.bb, v.bs, v.bv, v.sv, imb);
     } else { v.bb = v.bs = v.bv = v.sv = 0; v.price = NAN; }
   };
@@ -1087,9 +1032,9 @@ __global__ void __launch_bounds__(32 * LOBSIM_ENVFAST_WARPS, env_min_blocks<LT>(
   // ---- message pipeline ----------------------------------------------------------------------------------------------
   const int T = p.T;
   const int n_grid = (int)stp->n_grid_steps;   // steps beyond the end: the existing ones are run, the first one past the end sets END_OF_STREAM
-  if ((now_step < 0 || now_step > n_grid) && !f.dead && T > t_start) { f.err |= LOBSIM_ERR_END_OF_STREAM; f.dead = 1; }
+  if ((now_step < 0 || now_step > n_grid) && !f.dead && T > 0) { f.err |= LOBSIM_ERR_END_OF_STREAM; f.dead = 1; }
   unsigned g = 0, g_end_all = 0;
-  if (!f.dead && !aborted && T > t_start) { g = __ldg(&st_step_off[now_step]); g_end_all = __ldg(&st_step_off[min((long long)now_step + (T - t_start), (long long)n_grid)]); }
+  if (!f.dead && T > 0) { g = __ldg(&st_step_off[now_step]); g_end_all = __ldg(&st_step_off[min((long long)now_step + T, (long long)n_grid)]); }
   const unsigned tile0 = g / MSG_TILE;
   unsigned next_issue = 0, next_wait = 0;
   auto issue_tile = [&]() {
@@ -1107,43 +1052,23 @@ __global__ void __launch_bounds__(32 * LOBSIM_ENVFAST_WARPS, env_min_blocks<LT>(
   auto wait_tile = [&]() { mbar_wait(&bars[next_wait & 1], (next_wait >> 1) & 1); next_wait++; };
   if (g < g_end_all) { issue_tile(); issue_tile(); }
   __syncwarp();
-  if (SYNC) PHASE_SYNC();
+  if (SYNC) __syncthreads();
   const int steps_per_sec = ec.steps_per_sec;
   int sub = now_step >= 0 ? now_step % steps_per_sec : 0;
 
-  // shared memory -> HBM: the header and the occupied part of the arrays (sorted form) or of the pools (flat form); every issuing lane
-  // commits and waits for its own copy.  ENV_HOT stores after EVERY step of a multi-step launch, so that an aborted step finds HBM
-  // consistent (book, feature state, outputs) at the end of the step before.
-  auto store_blob = [&]() {
-    __syncwarp();
-    if (lane == 0) {
-      if (f.fill_log && h->n_fills > f.fill_cap) f.err |= LOBSIM_ERR_FILL_LOG_FULL;
-      h->now_step = now_step; h->price = sv->price; h->err = f.err; h->dead = f.dead;
-      if (p.fill_count) p.fill_count[env] = h->n_fills;
-      if (MODE == ENV_HOT) flat_mark(h, fs);
-    }
-    __syncwarp();
-    fence_proxy_async();
-    __syncwarp();
-    if (lane == 12) tma_store_part(gblob, base, (uint32_t)sizeof(BookHdr));
-    if (MODE == ENV_HOT) flat_body_copy<LT, false>(base, gblob, nullptr, lane, fs.n0, fs.n1);
-    else blob_body_copy<LT, false>(base, gblob, nullptr, lane);
-    if (lane <= 12) { tma_store_commit(); tma_store_wait(); }
-    __syncwarp();
-  };
   AgentGenFast gen; gen.side = 3; gen.stage = 0; gen.need = 0; gen.todo0 = gen.todo1 = gen.wm0 = gen.wm1 = 0; gen.wide_removed = gen.wide_pos = 0;
   gen.pending_id = 0; gen.base0 = gen.base1 = 0; gen.clear_vol = -1; gen.clear_side = 0;
   const int Q = c.max_quote_level - c.min_quote_level;
   int* diff_scratch = reinterpret_cast<int*>(scratch);
   bool agent_phase = false;
 #pragma unroll 1
-  for (int t = t_start; t < T; t++) {
-    if (SYNC) PHASE_SYNC(); // ---- phase A: action -> ladders (fp64) --------------------------------------------------------
+  for (int t = 0; t < T; t++) {
+    if (SYNC) __syncthreads(); // ---- phase A: action -> ladders (fp64) -----------------------------------------------------
     __syncwarp();
     if (lane == 0) { sv->cash0 = h->cash; sv->p0 = sv->price; sv->inv0 = h->inventory; } // deepcopy(self.state), HOE.py:166
     if (lane < 8) h->flow[lane] = 0;
     __syncwarp();
-    if (p.agent_kind != LOBSIM_AGENT_NONE && !(MODE == ENV_HOT && aborted)) {
+    if (p.agent_kind != LOBSIM_AGENT_NONE) {
       double* act_sm = reinterpret_cast<double*>(scratch);
       if (p.agent_kind == LOBSIM_AGENT_EXTERNAL) {
         const double* a = p.actions_in + ((size_t)t * p.n_sel + sel) * ec.action_dim;
@@ -1167,14 +1092,13 @@ __global__ void __launch_bounds__(32 * LOBSIM_ENVFAST_WARPS, env_min_blocks<LT>(
         agent_phase = true;
       }
     }
-    if (SYNC && LOBSIM_SYNC_B) PHASE_SYNC(); // ---- phase B: the step's orders: the agent's first, then the historical messages of (now, now + step]
+    if (SYNC) __syncthreads(); // ---- phase B: the step's orders: the agent's first, then the historical messages of (now, now + step]
     {
       if (!f.dead && now_step >= (int)stp->n_grid_steps) { f.err |= LOBSIM_ERR_END_OF_STREAM; f.dead = 1; } // re-read: keeps a register free
       const unsigned g_step_end = f.dead ? g : __ldg(&st_step_off[now_step + 1]);
 #pragma unroll 1
       for (;;) {
         int type, side, oprice, vol; uint32_t ref; bool is_agent;
-        if (MODE == ENV_HOT && aborted) break;
         if (agent_phase) {
           if (!agent_next_fast(fb, f, gen, diff_scratch, Q, c.tick_size, type, side, oprice, vol, ref)) { agent_phase = false; continue; }
           is_agent = true;
@@ -1188,13 +1112,10 @@ __global__ void __launch_bounds__(32 * LOBSIM_ENVFAST_WARPS, env_min_blocks<LT>(
           g++;
           if (g % MSG_TILE == 0) { __syncwarp(); issue_tile(); }
         }
-        if (!f.dead) {
-          if (MODE == ENV_HOT) { if (!flat_order_tracked<LT>(base, lane, f, fs, type, side, oprice, vol, ref, is_agent)) defer(t); }   // pool full
-          else fast_order_full<LT, true>(fb, f, type, side, oprice, vol, ref, is_agent);
-        }
+        if (!f.dead) fast_order_full<LT, true>(fb, f, type, side, oprice, vol, ref, is_agent);
       }
     }
-    if (!f.dead && !(MODE == ENV_HOT && aborted)) {
+    if (!f.dead) {
       now_step++;
       if (++sub == steps_per_sec) {                          // whole second: outer-level resync, OrderbookSimulator.py:86-87
         sub = 0;
@@ -1206,17 +1127,13 @@ __global__ void __launch_bounds__(32 * LOBSIM_ENVFAST_WARPS, env_min_blocks<LT>(
             const int sec = now_step / steps_per_sec;
             if (sec <= (int)stp->n_seconds && stp->snap_valid[sec]) {
               const int32_t* row = stp->snapshots + (size_t)sec * 2 * c.n_levels * 2;
-              if (MODE == ENV_HOT) {
-                if (flat_resync_needed(h, row, c.n_levels, lane)) defer(t);   // a level to overwrite: the sorted kernel redoes this step
-                else flat_update_trackers<LT>(base, lane, fs);
-              } else fast_resync_tracked(fb, f, row, c.n_levels, scratch);
+              fast_resync_tracked(fb, f, row, c.n_levels, scratch);
             }
           }
         }
       }
     }
-    if (SYNC && LOBSIM_SYNC_C) PHASE_SYNC(); // ---- phase C: update_internal_state + _update_features + reward, HOE.py:163-178,199-204 -------------
-    if (MODE == ENV_HOT && aborted) continue;              // (keeps taking part in the phase barriers of its CTA)
+    if (SYNC) __syncthreads(); // ---- phase C: update_internal_state + _update_features + reward, HOE.py:163-178,199-204 -------------
     StepView v; tops(v);
     if (!v.have_tops) f.err |= LOBSIM_ERR_EMPTY_BOOK;
     const double price = v.price;
@@ -1243,7 +1160,6 @@ __global__ void __launch_bounds__(32 * LOBSIM_ENVFAST_WARPS, env_min_blocks<LT>(
       }
       if (p.info) write_info(p.info + ((size_t)t * p.n_sel + sel) * LOBSIM_INFO_DIM, lane, v, cash1, inv1, f.err);
     }
-    if (MODE == ENV_HOT && t + 1 < T) store_blob();       // checkpoint (see store_blob)
   }
   if (T == 0 && p.obs && p.reset_mode == 2) { // reset with no warm-up: obs straight after _reset_features
     double* o = p.obs + (size_t)sel * ec.obs_dim;
@@ -1251,5 +1167,19 @@ __global__ void __launch_bounds__(32 * LOBSIM_ENVFAST_WARPS, env_min_blocks<LT>(
     if (c.inc_prev_action_in_obs && lane < ec.action_dim) o[F + lane] = 0.0;
   }
   while (next_wait < next_issue) wait_tile();
-  if (!(MODE == ENV_HOT && aborted)) store_blob();        // (an aborted env step leaves HBM as it was at the end of the step before)
+
+  // ---- shared memory -> HBM: the header and the occupied part of the arrays; every issuing lane commits and waits for its own copy
+  __syncwarp();
+  if (lane == 0) {
+    if (f.fill_log && h->n_fills > f.fill_cap) f.err |= LOBSIM_ERR_FILL_LOG_FULL;
+    h->now_step = now_step; h->price = sv->price; h->err = f.err; h->dead = f.dead;
+    if (p.fill_count) p.fill_count[env] = h->n_fills;
+  }
+  __syncwarp();
+  fence_proxy_async();
+  __syncwarp();
+  if (lane == 12) tma_store_part(gblob, base, (uint32_t)sizeof(BookHdr));
+  blob_body_copy<LT, false>(base, gblob, nullptr, lane);
+  if (lane <= 12) { tma_store_commit(); tma_store_wait(); }
+  __syncwarp();
 }

@@ -17,13 +17,3 @@
                           the flat form may hold 128 orders per side (book_flat.cuh)               */
 
 #define LOBSIM_N_FAST_LAYOUTS 6
-
-// env launches of these layouts use the flat-only HOT kernel + the DEFERRED kernel (kernels.cuh, ENV_HOT).  NONE by default: built,
-// verified (847 GPU tests with it on for 128/256/64) and measured -- no faster than the classic kernel for one-step launches
-// (4.65e7 vs 4.66e7 env steps/s: what the smaller hot kernel gains, the extra launch and the abort plumbing take back) and 10 %
-// slower for fused 128-step rollouts (5.80e7 vs 6.48e7: the blob has to be checkpointed to HBM after every step so that an aborted
-// step can be redone), profiles/r02_env_ab.txt.  Enable with -DLOBSIM_ENV_HOT_LAYOUTS=1 for the 128/256/64 layout.
-#ifndef LOBSIM_ENV_HOT_LAYOUTS
-#define LOBSIM_ENV_HOT_LAYOUTS 0
-#endif
-#define LOBSIM_LAYOUT_ENV_HOT(nl, no, na) (LOBSIM_ENV_HOT_LAYOUTS && (nl) == 128 && (no) == 256)

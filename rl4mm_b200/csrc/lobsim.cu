@@ -33,14 +33,13 @@
 // ---- the compiled straight-line layouts (layouts.h; one pair of translation units each, fast_layout.cu) -------------
 struct FastLayoutOps {
   int NL, NO, NA;
-  bool env_hot;
   cudaError_t (*attrs)(int dyn_replay, int dyn_env);
   cudaError_t (*attrs_rare)(int dyn_env);
   void (*replay)(int grid, int block, size_t dyn, cudaStream_t stream, const AdvParams& p, const EnvConst& ec);
   void (*replay_flat)(int grid, int block, size_t dyn, cudaStream_t stream, const AdvParams& p, const EnvConst& ec);
   void (*to_sorted)(unsigned char* blobs, int n_envs, cudaStream_t stream);
-  void (*env)(int mode, bool sync, int grid, int block, size_t dyn, cudaStream_t stream, const AdvParams& p, const EnvConst& ec);
-  void (*env_rare)(int mode, bool sync, int grid, int block, size_t dyn, cudaStream_t stream, const AdvParams& p, const EnvConst& ec);
+  void (*env)(bool sync, int grid, int block, size_t dyn, cudaStream_t stream, const AdvParams& p, const EnvConst& ec);
+  void (*env_rare)(bool sync, int grid, int block, size_t dyn, cudaStream_t stream, const AdvParams& p, const EnvConst& ec);
 };
 #define X(i, nl, no, na)                                                                                                   \
   cudaError_t lobsim_fast##i##_attrs(int, int);                                                                            \
@@ -48,11 +47,11 @@ struct FastLayoutOps {
   void lobsim_fast##i##_replay(int, int, size_t, cudaStream_t, const AdvParams&, const EnvConst&);                         \
   void lobsim_fast##i##_replay_flat(int, int, size_t, cudaStream_t, const AdvParams&, const EnvConst&);                    \
   void lobsim_fast##i##_to_sorted(unsigned char*, int, cudaStream_t);                                                      \
-  void lobsim_fast##i##_env(int, bool, int, int, size_t, cudaStream_t, const AdvParams&, const EnvConst&);                 \
-  void lobsim_fast##i##_env_rare(int, bool, int, int, size_t, cudaStream_t, const AdvParams&, const EnvConst&);
+  void lobsim_fast##i##_env(bool, int, int, size_t, cudaStream_t, const AdvParams&, const EnvConst&);                      \
+  void lobsim_fast##i##_env_rare(bool, int, int, size_t, cudaStream_t, const AdvParams&, const EnvConst&);
 LOBSIM_FAST_LAYOUTS(X)
 #undef X
-#define X(i, nl, no, na) {nl, no, na, LOBSIM_LAYOUT_ENV_HOT(nl, no, na), lobsim_fast##i##_attrs, lobsim_fast##i##_attrs_rare, lobsim_fast##i##_replay, lobsim_fast##i##_replay_flat, lobsim_fast##i##_to_sorted, lobsim_fast##i##_env, lobsim_fast##i##_env_rare},
+#define X(i, nl, no, na) {nl, no, na, lobsim_fast##i##_attrs, lobsim_fast##i##_attrs_rare, lobsim_fast##i##_replay, lobsim_fast##i##_replay_flat, lobsim_fast##i##_to_sorted, lobsim_fast##i##_env, lobsim_fast##i##_env_rare},
 static const FastLayoutOps g_fast_layouts[LOBSIM_N_FAST_LAYOUTS] = {LOBSIM_FAST_LAYOUTS(X)};
 #undef X
 static const FastLayoutOps* find_fast_layout(const Layout& L) {
@@ -215,10 +214,9 @@ struct lobsim {
                                       // -1 (default) when NO >= 1024, LOBSIM_REPLAY_HYBRID=1 on every such layout, =0 never
   bool replay_flat = true;            // LOBSIM_REPLAY_FLAT=0: the replay fast path keeps every book in the sorted level arrays (A/B, testing)
   bool flat_blobs = true;             // LOBSIM_FLAT_BLOBS=0: the fast kernels never keep a book in the flat order pools across launches
-                                      // (env kernels: sorted path only; replay: converts back at the end of every launch)
+                                      // (the flat replay converts back at the end of every launch)
   lobsim_order_t* po_orders = nullptr; uint32_t* po_refs = nullptr; lobsim_fill_t* po_fills = nullptr; int32_t* po_nf = nullptr;   // lobsim_process_orders staging
   int po_cap = 0, po_fill_cap = 0;
-  int32_t* defer_count = nullptr; int2* defer_list = nullptr;   // env HOT kernel -> DEFERRED kernel hand-over (kernels.cuh ENV_HOT)
   bool blob_in_global = false;        // deep-book mode: the blob exceeds the shared memory of an SM and is worked on in place in HBM
   bool maybe_flat = false;            // some blob in HBM may be in the flat form: ensure_sorted() before anything that reads level arrays
   bool agent_orders_possible = false; // an agent order may rest in some book (disables the replay fast path)
@@ -334,15 +332,9 @@ int lobsim_create(const lobsim_cfg_t* cfg, int device, lobsim_t** out) {
   h->warps_per_cta = best_wpc(4, 1.0, h->warp_smem);
   h->replay_warps_per_cta = best_wpc(4, 1.0, h->replay_warp_smem);
   h->env_warps_per_cta = best_wpc(LOBSIM_ENVFAST_WARPS, 0.95, h->warp_smem);   // (deep 128/1024/64 books: 5 warps x 2 CTAs = 10 resident, +11 % over 8 x 1)
-  { const char* e = getenv("LOBSIM_ENV_WPC"); const int w = e ? atoi(e) : 0;   // A/B override (tools/)
-    if (w >= 1 && w <= LOBSIM_ENVFAST_WARPS && (long long)w * h->warp_smem <= max_smem - 1024) h->env_warps_per_cta = w; }
   CUDA_TRY((cudaFuncSetAttribute(k_advance<true, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, h->warps_per_cta * h->warp_smem)));
   CUDA_TRY((cudaFuncSetAttribute(k_advance<false, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, h->warps_per_cta * h->warp_smem)));
   h->fast = h->force_general ? nullptr : find_fast_layout(h->L);
-  if (h->fast && h->fast->env_hot) {   // (allocated here, not at the first launch: that one may be inside a CUDA-graph capture)
-    CUDA_TRY(cudaMalloc(&h->defer_count, sizeof(int32_t)));
-    CUDA_TRY(cudaMalloc(&h->defer_list, (size_t)cfg->n_envs * sizeof(int2)));
-  }
   if (h->fast) {
     CUDA_TRY(h->fast->attrs(h->replay_warps_per_cta * h->replay_warp_smem, h->env_warps_per_cta * h->warp_smem));
     if (h->rare_paths) CUDA_TRY(h->fast->attrs_rare(h->env_warps_per_cta * h->warp_smem));
@@ -434,7 +426,7 @@ int lobsim_destroy(lobsim_t* h) {
   cudaFree(h->blobs); cudaFree(h->fstate); cudaFree(h->nstate); cudaFree(h->beta_tab); cudaFree(h->rings); cudaFree(h->rs_ring); cudaFree(h->rs_state); cudaFree(h->fill_log); cudaFree(h->fill_count); cudaFree(h->agents_dev);
   cudaFree(h->streams_dev); cudaFree(h->st_actions); cudaFree(h->st_obs); cudaFree(h->st_rew); cudaFree(h->st_done);
   cudaFree(h->st_state); cudaFree(h->st_msgs);
-  cudaFree(h->po_orders); cudaFree(h->po_refs); cudaFree(h->po_fills); cudaFree(h->po_nf); cudaFree(h->defer_count); cudaFree(h->defer_list);
+  cudaFree(h->po_orders); cudaFree(h->po_refs); cudaFree(h->po_fills); cudaFree(h->po_nf);
   delete h;
   return LOBSIM_OK;
 }
@@ -527,31 +519,16 @@ static int launch_env(lobsim* h, const AdvParams& p, cudaStream_t stream) {
   const size_t dyn = (size_t)wpc * h->warp_smem;
   const int full = p.n_sel / wpc, tail = p.n_sel % wpc;
   auto launch = h->rare_paths ? h->fast->env_rare : h->fast->env;
-  // Step / rollout launches of an ENV_HOT layout: the flat-only kernel for every env, then the deferred (sorted) kernel for the env
-  // steps it handed over (usually none).  Resets, fill-logged handles and LOBSIM_FLAT_BLOBS=0 take the classic kernel, which reads both
-  // book forms and stores the sorted one.
-  const bool hot = h->fast->env_hot && h->defer_list && p.allow_flat && p.reset_mode == 0 && !h->fill_log && p.T > 0;
-  AdvParams q = p;
-  if (hot) {
-    CUDA_TRY(cudaMemsetAsync(h->defer_count, 0, sizeof(int32_t), stream));
-    q.defer_count = h->defer_count; q.defer_list = h->defer_list;
-    h->maybe_flat = true;
-  }
-  const int mode = hot ? ENV_HOT : ENV_CLASSIC;
+  // (no ensure_sorted: the env kernel converts a flat blob on load and stores the sorted form)
   if (full > 0) { // full CTAs: phase-synchronous
-    launch(mode, true, full, wpc * 32, dyn, stream, q, h->ec);
+    launch(true, full, wpc * 32, dyn, stream, p, h->ec);
     CUDA_TRY(cudaGetLastError());
     h->launches++;
   }
   if (tail > 0) { // the remaining n_sel % wpc envs: one partially filled CTA without block-level barriers
-    AdvParams pt = q;
+    AdvParams pt = p;
     pt.sel_offset = full * wpc;
-    launch(mode, false, 1, wpc * 32, dyn, stream, pt, h->ec);
-    CUDA_TRY(cudaGetLastError());
-    h->launches++;
-  }
-  if (hot) {
-    launch(ENV_DEFERRED, false, (p.n_sel + wpc - 1) / wpc, wpc * 32, dyn, stream, q, h->ec);
+    launch(false, 1, wpc * 32, dyn, stream, pt, h->ec);
     CUDA_TRY(cudaGetLastError());
     h->launches++;
   }
