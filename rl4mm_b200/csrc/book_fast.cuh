@@ -1,4 +1,4 @@
-// book_fast.cuh -- the straight-line order path (k_replay_fast, k_env_fast): same semantics as process_order in
+// book_fast.cuh -- the straight-line order path (the sorted books of the replay kernels, k_env_fast): same semantics as process_order in
 // book.cuh, specialised for the overwhelmingly common shapes -- the touched level is among the 32 best, at most 32
 // (64 for removals) queue entries have to move, no capacity is exhausted -- as straight-line warp-wide code without
 // search / shift loops.  Anything else goes, BEFORE the book is mutated, to the any-depth routines at the end of this file

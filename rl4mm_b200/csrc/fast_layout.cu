@@ -1,6 +1,7 @@
-// fast_layout.cu -- ONE compiled StaticLayout of the straight-line kernels (k_replay_fast / k_env_fast, kernels.cuh).
+// fast_layout.cu -- ONE compiled StaticLayout of the straight-line kernels (k_replay_flat / k_replay_fast / k_replay_hyb /
+// k_env_fast, kernels.cuh).
 // Compiled once per entry of layouts.h and per part (-DLOBSIM_LAYOUT_INDEX=i -DLOBSIM_TU_PART=p, build.py), in parallel:
-//   part 0: the replay kernel + the env kernels without the z-score / RollingSharpe code
+//   part 0: the replay kernels + the env kernels without the z-score / RollingSharpe code
 //   part 1: the env kernels with that code (RARE)
 // lobsim.cu calls the launchers below through the FastLayoutOps table.
 #include "kernels.cuh"
@@ -47,14 +48,12 @@ cudaError_t FN(_attrs)(int dyn_replay, int dyn_env) {
   if (e == cudaSuccess) e = env_attrs<false>(dyn_env);
   return e;
 }
-void FN(_replay)(int grid, int block, size_t dyn, cudaStream_t stream, const AdvParams& p, const EnvConst& ec) {
-  k_replay_fast<LT><<<grid, block, dyn, stream>>>(p, ec);
-}
-void FN(_replay_flat)(int grid, int block, size_t dyn, cudaStream_t stream, const AdvParams& p, const EnvConst& ec) {
+void FN(_replay)(ReplayKind kind, int grid, int block, size_t dyn, cudaStream_t stream, const AdvParams& p, const EnvConst& ec) {
   if constexpr (hyb_layout<LT>()) {
-    if (p.hybrid) { k_replay_hyb<LT><<<grid, block, dyn, stream>>>(p, ec); return; }
+    if (kind == REPLAY_HYBRID) { k_replay_hyb<LT><<<grid, block, dyn, stream>>>(p, ec); return; }
   }
-  k_replay_flat<LT><<<grid, block, dyn, stream>>>(p, ec);
+  if (kind == REPLAY_SORTED) k_replay_fast<LT><<<grid, block, dyn, stream>>>(p, ec);
+  else k_replay_flat<LT><<<grid, block, dyn, stream>>>(p, ec);
 }
 void FN(_to_sorted)(unsigned char* blobs, int n_envs, cudaStream_t stream) {
   const int wpc = 4 * LT::blob_bytes <= 227 * 1024 ? 4 : 1;

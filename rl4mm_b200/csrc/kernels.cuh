@@ -74,6 +74,10 @@ __device__ __forceinline__ void tma_store_wait() { asm volatile("cp.async.bulk.w
 // int[64] for the agent's resting volume per ladder level (agent_prepare) and the 5 action doubles
 __host__ __device__ constexpr int scratch_bytes(int NA) { return 2 * NA * 8 > 256 ? 2 * NA * 8 : 256; }
 
+// the replay kernel of a handle with compiled straight-line kernels, fixed by lobsim_create: k_replay_fast (sorted level arrays
+// only), k_replay_flat (flat order pools, book_flat.cuh) or k_replay_hyb (hybrid book of deep layouts, book_hybrid.cuh)
+enum ReplayKind { REPLAY_SORTED, REPLAY_FLAT, REPLAY_HYBRID };
+
 struct AdvParams {
   unsigned char* blobs;             // [n_envs][blob_bytes]
   FeatState* fstate;                // [n_envs][LOBSIM_MAX_FEATURES]
@@ -99,7 +103,6 @@ struct AdvParams {
   int32_t out_final_obs_only;       // reset: write obs once, after the warm-up
   int32_t resync_last_only;         // forward_step over several grid steps: resync check only at the end
   int32_t blob_in_global;           // deep books: the blob does not fit in the shared memory of an SM and is worked on in place in HBM / L2
-  int32_t hybrid;                   // deep layouts: the replay launch runs k_replay_hyb (book_hybrid.cuh); blobs stay sorted in HBM
   int32_t allow_flat;               // fast kernels: books that fit run on -- and are stored in -- the flat order pools (book_flat.cuh)
   const double* actions_in;         // EXTERNAL: [T][n_sel][action_dim]
   double* obs; double* act; double* rew; uint8_t* done; // [T][n_sel][...] (any may be null)
@@ -149,6 +152,51 @@ __device__ __forceinline__ int us_in_minute(int t0_mod_min, int now_step, const 
 }
 
 __device__ __forceinline__ unsigned char* warp_smem_base(unsigned char* smem, int warp, int warp_smem) { return smem + (size_t)warp * warp_smem; }
+
+// The messages [g, g_end_all) of the T grid steps from now_step.  Steps beyond the end of the grid: the steps that exist are run,
+// the first one past the end sets END_OF_STREAM (here: a launch that starts outside the grid).  `err` / `dead` of the caller's state.
+__device__ __forceinline__ void stream_window(const uint32_t* __restrict__ step_off, int n_grid, int now_step, int T, uint32_t& err, int& dead,
+                                              unsigned& g, unsigned& g_end_all) {
+  if ((now_step < 0 || now_step > n_grid) && !dead && T > 0) { err |= LOBSIM_ERR_END_OF_STREAM; dead = 1; }
+  g = 0; g_end_all = 0;
+  if (!dead && T > 0) { g = __ldg(&step_off[now_step]); g_end_all = __ldg(&step_off[min((long long)now_step + T, (long long)n_grid)]); }
+}
+
+// The message tiles of one warp: TMA bulk loads of MSG_TILE records into a double buffer, one tile ahead of the reader.  Tiles are
+// MSG_TILE-aligned in the global message index space; relative tile r (rel(g)) lives in buffer r & 1 and completes phase
+// (r >> 1) & 1 of that buffer's mbarrier.  Tiles are issued and consumed strictly in order.  All members are warp-uniform.
+struct MsgTiles {
+  const lobsim_stream_t* stp;
+  const lobsim_msg_t* msgs;
+  unsigned char* buf;     // 2 x MSG_TILE_BYTES
+  uint64_t* bars;         // bars[0], bars[1]: one per buffer
+  int lane;
+  unsigned tile0, g_end, next_issue, next_wait;
+  // (constructed where the stream is known, started where the range is: the kernels' register allocation depends on that order)
+  __device__ __forceinline__ explicit MsgTiles(const lobsim_stream_t* s) : stp(s), msgs(s->msgs) {}
+  // the first two tiles of [g, g_end_all)
+  __device__ __forceinline__ void start(unsigned char* msgbuf, uint64_t* b, int ln, unsigned g, unsigned g_end_all) {
+    buf = msgbuf; bars = b; lane = ln;
+    tile0 = g / MSG_TILE; g_end = g_end_all; next_issue = next_wait = 0;
+    if (g < g_end_all) { issue(); issue(); }
+    __syncwarp();
+  }
+  __device__ __forceinline__ void issue() { // lane 0 talks to the TMA unit
+    const unsigned first = (tile0 + next_issue) * MSG_TILE;
+    if (first >= g_end) return;
+    if (lane == 0) {
+      const unsigned n_total = (unsigned)stp->n_msgs;   // (read here, not cached: a cached copy costs the replay kernels spills)
+      const unsigned cnt = n_total - first < MSG_TILE ? n_total - first : MSG_TILE;
+      uint64_t* bar = &bars[next_issue & 1];
+      mbar_expect_tx(bar, cnt * 16);
+      tma_load(buf + (next_issue & 1) * MSG_TILE_BYTES, msgs + first, cnt * 16, bar);
+    }
+    next_issue++;
+  }
+  __device__ __forceinline__ void wait() { mbar_wait(&bars[next_wait & 1], (next_wait >> 1) & 1); next_wait++; }
+  __device__ __forceinline__ unsigned rel(unsigned g) const { return g / MSG_TILE - tile0; }
+  __device__ __forceinline__ void drain() { while (next_wait < next_issue) wait(); }   // TMA loads still in flight (aborted episode)
+};
 
 // ====================================================================================================================
 //  the advance kernel: [reset] + T x ([agent orders] + messages of the step + [resync] + [features, reward])
@@ -211,7 +259,7 @@ __global__ void __launch_bounds__(128, kEnv ? LOBSIM_ENV_MIN_BLOCKS : 4) k_advan
     w.inventory = h->inventory; w.cash = h->cash;
   }
   const lobsim_stream_t* stp = &p.streams[stream_id];
-  const lobsim_msg_t* __restrict__ st_msgs = stp->msgs;
+  MsgTiles mt(stp);
   const uint32_t* __restrict__ st_step_off = stp->step_off;
   const long long st_t0_us = kEnv ? stp->t0_us : 0;
   int now_step = h->now_step;
@@ -246,33 +294,10 @@ __global__ void __launch_bounds__(128, kEnv ? LOBSIM_ENV_MIN_BLOCKS : 4) k_advan
 
   // ---- message pipeline ----------------------------------------------------------------------------------------------
   const int T = p.T;
-  // steps beyond the end of the grid: the steps that exist are run, the first one past the end sets END_OF_STREAM
   const int n_grid = (int)stp->n_grid_steps;
-  if ((now_step < 0 || now_step > n_grid) && !w.dead && T > 0) { w.err |= LOBSIM_ERR_END_OF_STREAM; w.dead = 1; }
-  unsigned g = 0, g_end_all = 0;
-  if (!w.dead && T > 0) { g = __ldg(&st_step_off[now_step]); g_end_all = __ldg(&st_step_off[min((long long)now_step + T, (long long)n_grid)]); }
-  // tiles are MSG_TILE-aligned in the global message index space; `rel` tile r lives in buffer r & 1 and completes
-  // phase (r >> 1) & 1 of that buffer's mbarrier.  Tiles are issued and consumed strictly in order.
-  const unsigned tile0 = g / MSG_TILE;
-  unsigned next_issue = 0, next_wait = 0;
-  auto issue_tile = [&]() { // uniform; lane 0 talks to the TMA unit
-    const unsigned first = (tile0 + next_issue) * MSG_TILE;
-    if (first >= g_end_all) return;
-    if (lane == 0) {
-      const unsigned n_total = (unsigned)stp->n_msgs;
-      unsigned cnt = n_total - first < MSG_TILE ? n_total - first : MSG_TILE;
-      uint64_t* bar = &bars[next_issue & 1];
-      mbar_expect_tx(bar, cnt * 16);
-      tma_load(msgbuf + (next_issue & 1) * MSG_TILE_BYTES, st_msgs + first, cnt * 16, bar);
-    }
-    next_issue++;
-  };
-  auto wait_tile = [&]() { // wait for relative tile `next_wait`
-    mbar_wait(&bars[next_wait & 1], (next_wait >> 1) & 1);
-    next_wait++;
-  };
-  if (g < g_end_all) { issue_tile(); issue_tile(); }
-  __syncwarp();
+  unsigned g, g_end_all;
+  stream_window(st_step_off, n_grid, now_step, T, w.err, w.dead, g, g_end_all);
+  mt.start(msgbuf, bars, lane, g, g_end_all);
 
   AgentGen gen; gen.side = 3;
   bool agent_phase = false;
@@ -316,13 +341,13 @@ __global__ void __launch_bounds__(128, kEnv ? LOBSIM_ENV_MIN_BLOCKS : 4) k_advan
           is_agent = true;
         } else {
           if (w.dead || g >= g_step_end) break;
-          const unsigned tile = g / MSG_TILE - tile0;
-          if (tile == next_wait) wait_tile();
+          const unsigned tile = mt.rel(g);
+          if (tile == mt.next_wait) mt.wait();
           const uint4 m = *reinterpret_cast<const uint4*>(msgbuf + (tile & 1) * MSG_TILE_BYTES + (g % MSG_TILE) * 16);
           price = (int)m.x; vol = (int)m.y; ref = m.z; type = (int)LOBSIM_META_TYPE(m.w); side = (int)LOBSIM_META_DIR(m.w);
           is_agent = false;
           g++;
-          if (g % MSG_TILE == 0) { __syncwarp(); issue_tile(); } // tile consumed: refill its buffer
+          if (g % MSG_TILE == 0) { __syncwarp(); mt.issue(); } // tile consumed: refill its buffer
         }
         process_order<kTrack>(b, w, type, side, price, vol, ref, is_agent);
       }
@@ -373,7 +398,7 @@ __global__ void __launch_bounds__(128, kEnv ? LOBSIM_ENV_MIN_BLOCKS : 4) k_advan
     if (c.inc_prev_action_in_obs && lane < ec.action_dim) o[F + lane] = 0.0;
   }
 
-  while (next_wait < next_issue) wait_tile(); // drain TMA loads still in flight (only after an aborted episode)
+  mt.drain();
 
   // ---- write back ----------------------------------------------------------------------------------------------------
   // OrderbookSimulator.forward_step only returns the fills: the portfolio belongs to the env (HOE.py:280-289)
@@ -391,23 +416,12 @@ __global__ void __launch_bounds__(128, kEnv ? LOBSIM_ENV_MIN_BLOCKS : 4) k_advan
 }
 
 // ====================================================================================================================
-//  the replay fast kernel: T x (messages of the step + [resync]) with the straight-line message path of book_fast.cuh.
-//  Used by lobsim_replay when no fill log is requested, no agent order can be resting and the book capacities match
-//  one of the compiled StaticLayouts.  72 registers => 7 CTAs x 4 warps = 28 books resident per SM.
+//  the frame of the straight-line replay kernels: a replay book holds no agent orders, so the agent tables at the end of the
+//  blob stay in HBM (deep books are shared-memory bound: 128/1536/64 capacities = 8 instead of 7 resident books per SM)
 // ====================================================================================================================
+// the blob up to the agent tables, HBM -> shared memory on bars[2] (bars[0..1]: the message tiles)
 template <class LT>
-__global__ void __launch_bounds__(128, 7) k_replay_fast(const __grid_constant__ AdvParams p, const __grid_constant__ EnvConst ec) {
-  extern __shared__ __align__(128) unsigned char smem[];
-  const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
-  const int env = blockIdx.x * (blockDim.x >> 5) + warp;
-  if (env >= p.n_sel) return;
-  const lobsim_cfg_t& c = ec.cfg;
-  // a replay book holds no agent orders: the agent tables at the end of the blob stay in HBM (deep books are shared-memory bound:
-  // 128/1536/64 capacities = 8 instead of 7 resident books per SM)
-  unsigned char* base = warp_smem_base(smem, warp, p.warp_smem);
-  unsigned char* msgbuf = base + LT::agent_off;
-  uint64_t* bars = reinterpret_cast<uint64_t*>(msgbuf + 2 * MSG_TILE_BYTES);
-  unsigned char* gblob = p.blobs + (size_t)env * LT::blob_bytes;
+__device__ __forceinline__ void replay_blob_load(unsigned char* base, const unsigned char* gblob, uint64_t* bars, int lane) {
   if (lane == 0) {
     mbar_init(&bars[0], 1); mbar_init(&bars[1], 1); mbar_init(&bars[2], 1);
     fence_mbar_init();
@@ -416,83 +430,14 @@ __global__ void __launch_bounds__(128, 7) k_replay_fast(const __grid_constant__ 
   }
   __syncwarp();
   mbar_wait(&bars[2], 0);
-
-  FastBook<LT> fb; fb.blob = base; fb.lane = lane;
+}
+// ... and back: the header fields of the launch, then one bulk store.  `hdr_extra()`: header fields of the kernel's own, written by
+// lane 0 with the others
+template <class LT, class HdrExtra>
+__device__ __forceinline__ void replay_blob_store(unsigned char* gblob, unsigned char* base, int lane, int now_step, const FastState& f, HdrExtra hdr_extra) {
   BookHdr* h = reinterpret_cast<BookHdr*>(base);
-  FastState f; f.err = h->err; f.dead = h->dead; f.bail = 0; f.bail_vol = 0;
-  fast_refresh_best(fb, f);
-  const lobsim_stream_t* stp = &p.streams[h->stream_id];
-  const lobsim_msg_t* __restrict__ st_msgs = stp->msgs;
-  const uint32_t* __restrict__ st_step_off = stp->step_off;
-  int now_step = h->now_step;
-  const int T = p.T;
-  const int n_grid = (int)stp->n_grid_steps;   // steps beyond the end: the existing ones are run, the first one past the end sets END_OF_STREAM
-  if ((now_step < 0 || now_step > n_grid) && !f.dead && T > 0) { f.err |= LOBSIM_ERR_END_OF_STREAM; f.dead = 1; }
-  unsigned g = 0, g_end_all = 0;
-  if (!f.dead && T > 0) { g = __ldg(&st_step_off[now_step]); g_end_all = __ldg(&st_step_off[min((long long)now_step + T, (long long)n_grid)]); }
-  const unsigned tile0 = g / MSG_TILE;
-  unsigned next_issue = 0, next_wait = 0;
-  auto issue_tile = [&]() {
-    const unsigned first = (tile0 + next_issue) * MSG_TILE;
-    if (first >= g_end_all) return;
-    if (lane == 0) {
-      const unsigned n_total = (unsigned)stp->n_msgs;
-      const unsigned cnt = n_total - first < MSG_TILE ? n_total - first : MSG_TILE;
-      uint64_t* bar = &bars[next_issue & 1];
-      mbar_expect_tx(bar, cnt * 16);
-      tma_load(msgbuf + (next_issue & 1) * MSG_TILE_BYTES, st_msgs + first, cnt * 16, bar);
-    }
-    next_issue++;
-  };
-  auto wait_tile = [&]() { mbar_wait(&bars[next_wait & 1], (next_wait >> 1) & 1); next_wait++; };
-  if (g < g_end_all) { issue_tile(); issue_tile(); }
   __syncwarp();
-  const int steps_per_sec = ec.steps_per_sec;
-  int sub = now_step >= 0 ? now_step % steps_per_sec : 0;   // position inside the current second
-
-#pragma unroll 1
-  for (int t = 0; t < T && !f.dead; t++) {
-    if (now_step >= n_grid) { f.err |= LOBSIM_ERR_END_OF_STREAM; f.dead = 1; break; }
-    const unsigned g_step_end = __ldg(&st_step_off[now_step + 1]);
-#pragma unroll 1
-    while (g < g_step_end) {
-      const unsigned tile = g / MSG_TILE - tile0;
-      if (tile == next_wait) wait_tile();
-      const unsigned tile_end = (g / MSG_TILE + 1) * MSG_TILE;
-      const unsigned lim = g_step_end < tile_end ? g_step_end : tile_end;
-      const uint4* mp = reinterpret_cast<const uint4*>(msgbuf + (tile & 1) * MSG_TILE_BYTES) + (g % MSG_TILE);
-      const unsigned cnt = lim - g;
-#pragma unroll 1
-      for (unsigned i = 0; i < cnt; i++) {
-        const uint4 m = mp[i];
-        fast_message(fb, f, (int)m.x, (int)m.y, m.z, m.w);
-        if (f.dead) break;
-      }
-      if (f.dead) break;
-      g = lim;
-      if (g == tile_end) { __syncwarp(); issue_tile(); }
-    }
-    if (f.dead) break;
-    now_step++;
-    if (++sub == steps_per_sec) {                            // whole second: outer-level resync, OrderbookSimulator.py:86-87
-      sub = 0;
-      if (c.resync && (!p.resync_last_only || t == T - 1)) {
-        const double prop = ec.outer_prop;
-        const double bb = f.best0 == INT32_MIN ? 0.0 : (double)f.best0;
-        const double bs = f.best1 == INT32_MAX ? (double)INFINITY : (double)f.best1;
-        if (bb < (double)h->min_buy + prop * (double)h->init_buy_range || bs > (double)h->max_sell - prop * (double)h->init_sell_range) {
-          const int sec = now_step / steps_per_sec;
-          if (sec <= (int)stp->n_seconds && stp->snap_valid[sec]) {
-            const int32_t* row = stp->snapshots + (size_t)sec * 2 * c.n_levels * 2;
-            fast_resync(fb, f, row, c.n_levels);   // straight-line: a replay book holds no agent orders
-          }
-        }
-      }
-    }
-  }
-  while (next_wait < next_issue) wait_tile();                // drain TMA loads still in flight (aborted episode)
-  __syncwarp();
-  if (lane == 0) { h->now_step = now_step; h->err = f.err; h->dead = f.dead; }
+  if (lane == 0) { h->now_step = now_step; h->err = f.err; h->dead = f.dead; hdr_extra(); }
   __syncwarp();
   fence_proxy_async();
   __syncwarp();
@@ -500,11 +445,24 @@ __global__ void __launch_bounds__(128, 7) k_replay_fast(const __grid_constant__ 
   __syncwarp();
 }
 
+// Whole second: the outer-level resync test of OrderbookSimulator.py:86-87 for a book with the best prices best0 / best1 -- the
+// snapshot row of the second that now_step ends when a best price has left the inner part of the book's initial range and the
+// stream has a snapshot of that second, else nullptr.
+__device__ __forceinline__ const int32_t* resync_row(const EnvConst& ec, const BookHdr* h, const lobsim_stream_t* stp, int best0, int best1, int now_step, int steps_per_sec) {
+  const double prop = ec.outer_prop;
+  const double bb = best0 == INT32_MIN ? 0.0 : (double)best0;
+  const double bs = best1 == INT32_MAX ? (double)INFINITY : (double)best1;
+  if (bb < (double)h->min_buy + prop * (double)h->init_buy_range || bs > (double)h->max_sell - prop * (double)h->init_sell_range) {
+    const int sec = now_step / steps_per_sec;
+    if (sec <= (int)stp->n_seconds && stp->snap_valid[sec]) return stp->snapshots + (size_t)sec * 2 * ec.cfg.n_levels * 2;
+  }
+  return nullptr;
+}
 __device__ __forceinline__ bool hdr_is_flat(const BookHdr* h) { return h->cnt[0][0] < 0; }
 // ====================================================================================================================
-//  the replay HYBRID kernel (deep layouts): k_replay_fast with the hybrid book of book_hybrid.cuh -- the levels near the touch in
-//  a flat order pool, the rest in the sorted arrays -- for every book that can take that form, the sorted straight-line path for
-//  the others.  The blob in HBM is the canonical sorted layout on entry and on exit.
+//  the replay HYBRID kernel (deep layouts): the hybrid book of book_hybrid.cuh -- the levels near the touch in a flat order pool,
+//  the rest in the sorted arrays -- for every book that can take that form, the sorted straight-line path for the others.  One grid
+//  step at a time: the pools are topped up at every step boundary.  The blob in HBM is the canonical sorted layout on entry and on exit.
 // ====================================================================================================================
 template <class LT>
 __global__ void __launch_bounds__(128, 3) k_replay_hyb(const __grid_constant__ AdvParams p, const __grid_constant__ EnvConst ec) {
@@ -517,14 +475,7 @@ __global__ void __launch_bounds__(128, 3) k_replay_hyb(const __grid_constant__ A
   unsigned char* msgbuf = base + LT::agent_off;
   uint64_t* bars = reinterpret_cast<uint64_t*>(msgbuf + 2 * MSG_TILE_BYTES);
   unsigned char* gblob = p.blobs + (size_t)env * LT::blob_bytes;
-  if (lane == 0) {
-    mbar_init(&bars[0], 1); mbar_init(&bars[1], 1); mbar_init(&bars[2], 1);
-    fence_mbar_init();
-    mbar_expect_tx(&bars[2], (uint32_t)LT::agent_off);
-    tma_load(base, gblob, (uint32_t)LT::agent_off, &bars[2]);
-  }
-  __syncwarp();
-  mbar_wait(&bars[2], 0);
+  replay_blob_load<LT>(base, gblob, bars, lane);
 
   FastBook<LT> fb; fb.blob = base; fb.lane = lane;
   BookHdr* h = reinterpret_cast<BookHdr*>(base);
@@ -534,36 +485,19 @@ __global__ void __launch_bounds__(128, 3) k_replay_hyb(const __grid_constant__ A
   HybState hs; hs.n0 = hs.n1 = 0; hs.floor0 = INT32_MIN; hs.floor1 = INT32_MAX; hs.seq = 0;
   bool hyb = false;
   const lobsim_stream_t* stp = &p.streams[h->stream_id];
-  const lobsim_msg_t* __restrict__ st_msgs = stp->msgs;
+  MsgTiles mt(stp);
   const uint32_t* __restrict__ st_step_off = stp->step_off;
   int now_step = h->now_step;
   const int T = p.T;
   const int n_grid = (int)stp->n_grid_steps;
-  if ((now_step < 0 || now_step > n_grid) && !f.dead && T > 0) { f.err |= LOBSIM_ERR_END_OF_STREAM; f.dead = 1; }
-  unsigned g = 0, g_end_all = 0;
-  if (!f.dead && T > 0) { g = __ldg(&st_step_off[now_step]); g_end_all = __ldg(&st_step_off[min((long long)now_step + T, (long long)n_grid)]); }
+  unsigned g, g_end_all;
+  stream_window(st_step_off, n_grid, now_step, T, f.err, f.dead, g, g_end_all);
   auto try_enter = [&]() {
     if (hyb_enter(fb, f, hs)) hyb = true;
     else if (hs.n0 | hs.n1) { hyb_leave(fb, f, hs); hs.n0 = hs.n1 = 0; }      // one side was moved, the other could not be: put it back
   };
   if (g < g_end_all) try_enter();
-  const unsigned tile0 = g / MSG_TILE;
-  unsigned next_issue = 0, next_wait = 0;
-  auto issue_tile = [&]() {
-    const unsigned first = (tile0 + next_issue) * MSG_TILE;
-    if (first >= g_end_all) return;
-    if (lane == 0) {
-      const unsigned n_total = (unsigned)stp->n_msgs;
-      const unsigned cnt = n_total - first < MSG_TILE ? n_total - first : MSG_TILE;
-      uint64_t* bar = &bars[next_issue & 1];
-      mbar_expect_tx(bar, cnt * 16);
-      tma_load(msgbuf + (next_issue & 1) * MSG_TILE_BYTES, st_msgs + first, cnt * 16, bar);
-    }
-    next_issue++;
-  };
-  auto wait_tile = [&]() { mbar_wait(&bars[next_wait & 1], (next_wait >> 1) & 1); next_wait++; };
-  if (g < g_end_all) { issue_tile(); issue_tile(); }
-  __syncwarp();
+  mt.start(msgbuf, bars, lane, g, g_end_all);
   const int steps_per_sec = ec.steps_per_sec;
   int sub = now_step >= 0 ? now_step % steps_per_sec : 0;
 
@@ -573,8 +507,8 @@ __global__ void __launch_bounds__(128, 3) k_replay_hyb(const __grid_constant__ A
     const unsigned g_step_end = __ldg(&st_step_off[now_step + 1]);
 #pragma unroll 1
     while (g < g_step_end) {
-      const unsigned tile = g / MSG_TILE - tile0;
-      if (tile == next_wait) wait_tile();
+      const unsigned tile = mt.rel(g);
+      if (tile == mt.next_wait) mt.wait();
       const unsigned tile_end = (g / MSG_TILE + 1) * MSG_TILE;
       const unsigned lim = g_step_end < tile_end ? g_step_end : tile_end;
       const uint4* mp = reinterpret_cast<const uint4*>(msgbuf + (tile & 1) * MSG_TILE_BYTES) + (g % MSG_TILE);
@@ -612,7 +546,7 @@ __global__ void __launch_bounds__(128, 3) k_replay_hyb(const __grid_constant__ A
       }
       if (f.dead) break;
       g = lim;
-      if (g == tile_end) { __syncwarp(); issue_tile(); }
+      if (g == tile_end) { __syncwarp(); mt.issue(); }
     }
     if (f.dead) break;
     now_step++;
@@ -620,18 +554,11 @@ __global__ void __launch_bounds__(128, 3) k_replay_hyb(const __grid_constant__ A
     if (++sub == steps_per_sec) {                            // whole second: outer-level resync, OrderbookSimulator.py:86-87
       sub = 0;
       if (c.resync && (!p.resync_last_only || t == T - 1)) {
-        const double prop = ec.outer_prop;
-        const double bb = f.best0 == INT32_MIN ? 0.0 : (double)f.best0;
-        const double bs = f.best1 == INT32_MAX ? (double)INFINITY : (double)f.best1;
-        if (bb < (double)h->min_buy + prop * (double)h->init_buy_range || bs > (double)h->max_sell - prop * (double)h->init_sell_range) {
-          const int sec = now_step / steps_per_sec;
-          if (sec <= (int)stp->n_seconds && stp->snap_valid[sec]) {
-            const int32_t* row = stp->snapshots + (size_t)sec * 2 * c.n_levels * 2;
-            if (hyb && !flat_resync_needed(h, row, c.n_levels, lane)) hyb_update_trackers(fb, hs);
-            else {
-              if (hyb) { hyb_leave(fb, f, hs); hyb = false; hs.n0 = hs.n1 = 0; }
-              fast_resync(fb, f, row, c.n_levels);
-            }
+        if (const int32_t* row = resync_row(ec, h, stp, f.best0, f.best1, now_step, steps_per_sec)) {
+          if (hyb && !flat_resync_needed(h, row, c.n_levels, lane)) hyb_update_trackers(fb, hs);
+          else {
+            if (hyb) { hyb_leave(fb, f, hs); hyb = false; hs.n0 = hs.n1 = 0; }
+            fast_resync(fb, f, row, c.n_levels);
           }
         }
       }
@@ -639,14 +566,8 @@ __global__ void __launch_bounds__(128, 3) k_replay_hyb(const __grid_constant__ A
     }
   }
   if (hyb) hyb_leave(fb, f, hs);
-  while (next_wait < next_issue) wait_tile();
-  __syncwarp();
-  if (lane == 0) { h->now_step = now_step; h->err = f.err; h->dead = f.dead; }
-  __syncwarp();
-  fence_proxy_async();
-  __syncwarp();
-  if (lane == 0) { tma_store(gblob, base, (uint32_t)LT::agent_off); tma_store_wait(); }
-  __syncwarp();
+  mt.drain();
+  replay_blob_store<LT>(gblob, base, lane, now_step, f, []() {});
 }
 
 // ---- the flat form of a blob in HBM (book_flat.cuh): header with cnt[0] = {-1, n0}, cnt[1] = {seq, n1}; per side the order pool
@@ -717,69 +638,43 @@ __global__ void __launch_bounds__(128) k_to_sorted(unsigned char* blobs, int n_e
 }
 
 // ====================================================================================================================
-//  the replay FLAT kernel: k_replay_fast with the flat order pools of book_flat.cuh for every book that fits them (at most
-//  FLAT_CAP resting orders per side), the sorted straight-line path for the others -- per book, re-decided every second.
-//  The blob in HBM is the canonical sorted layout on entry and on exit.
+//  the straight-line replay kernels: T x (messages of the step + [resync]) with the straight-line message paths, one pass per
+//  second.  Used by lobsim_replay when no fill log is requested, no agent order can be resting and the book capacities match one
+//  of the compiled StaticLayouts.  kPools (k_replay_flat): the flat order pools of book_flat.cuh for every book that fits them (at
+//  most FLAT_CAP resting orders per side), the sorted straight-line path of book_fast.cuh for the others -- per book, re-decided
+//  every second.  Without (k_replay_fast): the sorted path for every book.  The blob in HBM is the canonical sorted layout on
+//  entry and on exit.
 // ====================================================================================================================
-#ifndef LOBSIM_REPLAY_FLAT_MIN_BLOCKS
-#define LOBSIM_REPLAY_FLAT_MIN_BLOCKS 7      // 72 registers: 28 resident warps per SM with the 64/256/32 blob (8 = 64 registers: A/B in profiles/)
-#endif
-template <class LT>
-__global__ void __launch_bounds__(128, LOBSIM_REPLAY_FLAT_MIN_BLOCKS) k_replay_flat(const __grid_constant__ AdvParams p, const __grid_constant__ EnvConst ec) {
+template <class LT, bool kPools>
+__device__ __forceinline__ void replay_straight(const AdvParams& p, const EnvConst& ec) {
   extern __shared__ __align__(128) unsigned char smem[];
   const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
   const int env = blockIdx.x * (blockDim.x >> 5) + warp;
   if (env >= p.n_sel) return;
   const lobsim_cfg_t& c = ec.cfg;
-  // a replay book holds no agent orders: the agent tables at the end of the blob stay in HBM (deep books are shared-memory bound:
-  // 128/1536/64 capacities = 8 instead of 7 resident books per SM)
   unsigned char* base = warp_smem_base(smem, warp, p.warp_smem);
   unsigned char* msgbuf = base + LT::agent_off;
   uint64_t* bars = reinterpret_cast<uint64_t*>(msgbuf + 2 * MSG_TILE_BYTES);
   unsigned char* gblob = p.blobs + (size_t)env * LT::blob_bytes;
-  if (lane == 0) {
-    mbar_init(&bars[0], 1); mbar_init(&bars[1], 1); mbar_init(&bars[2], 1);
-    fence_mbar_init();
-    mbar_expect_tx(&bars[2], (uint32_t)LT::agent_off);
-    tma_load(base, gblob, (uint32_t)LT::agent_off, &bars[2]);
-  }
-  __syncwarp();
-  mbar_wait(&bars[2], 0);
+  replay_blob_load<LT>(base, gblob, bars, lane);
 
   FastBook<LT> fb; fb.blob = base; fb.lane = lane;
   BookHdr* h = reinterpret_cast<BookHdr*>(base);
   FastState f; f.err = h->err; f.dead = h->dead; f.bail = 0; f.bail_vol = 0;
-  if (!hdr_is_flat(h)) fast_refresh_best(fb, f);
+  if (!kPools || !hdr_is_flat(h)) fast_refresh_best(fb, f);
   FlatState fs; fs.n0 = fs.n1 = 0; fs.seq = 0;
   bool flat = false;
-  if (hdr_is_flat(h)) { flat_adopt<LT>(base, lane, f, fs); flat = true; }   // the blob was stored in the flat form
+  if (kPools && hdr_is_flat(h)) { flat_adopt<LT>(base, lane, f, fs); flat = true; }   // the blob was stored in the flat form
   const lobsim_stream_t* stp = &p.streams[h->stream_id];
-  const lobsim_msg_t* __restrict__ st_msgs = stp->msgs;
+  MsgTiles mt(stp);
   const uint32_t* __restrict__ st_step_off = stp->step_off;
   int now_step = h->now_step;
   const int T = p.T;
   const int n_grid = (int)stp->n_grid_steps;
-  if ((now_step < 0 || now_step > n_grid) && !f.dead && T > 0) { f.err |= LOBSIM_ERR_END_OF_STREAM; f.dead = 1; }
-  unsigned g = 0, g_end_all = 0;
-  if (!f.dead && T > 0) { g = __ldg(&st_step_off[now_step]); g_end_all = __ldg(&st_step_off[min((long long)now_step + T, (long long)n_grid)]); }
-  if (!flat && g < g_end_all && flat_fits(fb, 0)) { flat_enter(fb, fs); flat = true; }
-  const unsigned tile0 = g / MSG_TILE;
-  unsigned next_issue = 0, next_wait = 0;
-  auto issue_tile = [&]() {
-    const unsigned first = (tile0 + next_issue) * MSG_TILE;
-    if (first >= g_end_all) return;
-    if (lane == 0) {
-      const unsigned n_total = (unsigned)stp->n_msgs;
-      const unsigned cnt = n_total - first < MSG_TILE ? n_total - first : MSG_TILE;
-      uint64_t* bar = &bars[next_issue & 1];
-      mbar_expect_tx(bar, cnt * 16);
-      tma_load(msgbuf + (next_issue & 1) * MSG_TILE_BYTES, st_msgs + first, cnt * 16, bar);
-    }
-    next_issue++;
-  };
-  auto wait_tile = [&]() { mbar_wait(&bars[next_wait & 1], (next_wait >> 1) & 1); next_wait++; };
-  if (g < g_end_all) { issue_tile(); issue_tile(); }
-  __syncwarp();
+  unsigned g, g_end_all;
+  stream_window(st_step_off, n_grid, now_step, T, f.err, f.dead, g, g_end_all);
+  if (kPools && !flat && g < g_end_all && flat_fits(fb, 0)) { flat_enter(fb, fs); flat = true; }
+  mt.start(msgbuf, bars, lane, g, g_end_all);
   const int steps_per_sec = ec.steps_per_sec;
   int sub = now_step >= 0 ? now_step % steps_per_sec : 0;
 
@@ -793,31 +688,33 @@ __global__ void __launch_bounds__(128, LOBSIM_REPLAY_FLAT_MIN_BLOCKS) k_replay_f
     const unsigned g_pass_end = __ldg(&st_step_off[now_step + k]);
 #pragma unroll 1
     while (g < g_pass_end) {
-      const unsigned tile = g / MSG_TILE - tile0;
-      if (tile == next_wait) wait_tile();
+      const unsigned tile = mt.rel(g);
+      if (tile == mt.next_wait) mt.wait();
       const unsigned tile_end = (g / MSG_TILE + 1) * MSG_TILE;
       const unsigned lim = g_pass_end < tile_end ? g_pass_end : tile_end;
       const uint4* mp = reinterpret_cast<const uint4*>(msgbuf + (tile & 1) * MSG_TILE_BYTES) + (g % MSG_TILE);
       const unsigned cnt = lim - g;
       unsigned i = 0;
-      if (flat) {
-        // the volumes of the whole segment (<= 32 messages, one per lane) are checked at once; the per-message test is one predicate
-        const bool bad_vol = __any_sync(FULL_MASK, (unsigned)lane < cnt && (int)mp[(unsigned)lane < cnt ? lane : 0].y <= 0);
-        unsigned off = 0;                                    // (the loop walks a byte offset: no index arithmetic per message)
-        const unsigned off_end = cnt * 16u;
-        auto run = [&](auto vchk) {                          // (two copies of the loop: the one that runs has no volume test)
+      if constexpr (kPools) {
+        if (flat) {
+          // the volumes of the whole segment (<= 32 messages, one per lane) are checked at once; the per-message test is one predicate
+          const bool bad_vol = __any_sync(FULL_MASK, (unsigned)lane < cnt && (int)mp[(unsigned)lane < cnt ? lane : 0].y <= 0);
+          unsigned off = 0;                                  // (the loop walks a byte offset: no index arithmetic per message)
+          const unsigned off_end = cnt * 16u;
+          auto run = [&](auto vchk) {                        // (two copies of the loop: the one that runs has no volume test)
 #pragma unroll 1
-          for (; off != off_end; off += 16u) {
-            const uint4 m = *reinterpret_cast<const uint4*>(reinterpret_cast<const unsigned char*>(mp) + off);
-            if (flat_message<LT, decltype(vchk)::value>(base, lane, f, fs, (int)m.x, (int)m.y, m.z, m.w)) return true;   // pool full
+            for (; off != off_end; off += 16u) {
+              const uint4 m = *reinterpret_cast<const uint4*>(reinterpret_cast<const unsigned char*>(mp) + off);
+              if (flat_message<LT, decltype(vchk)::value>(base, lane, f, fs, (int)m.x, (int)m.y, m.z, m.w)) return true;   // pool full
                                                              // (this message runs on the sorted book) or f.dead: EmptyOrderbookError
-          }
-          return false;
-        };
-        const bool stopped = __builtin_expect(bad_vol, 0) ? run(std::true_type{}) : run(std::false_type{});
-        i = off >> 4;
-        f.bail = 0;                                          // (not read: `stopped` without f.dead is the full pool)
-        if (stopped && !f.dead) { flat_leave(fb, fs); flat = false; }
+            }
+            return false;
+          };
+          const bool stopped = __builtin_expect(bad_vol, 0) ? run(std::true_type{}) : run(std::false_type{});
+          i = off >> 4;
+          f.bail = 0;                                        // (not read: `stopped` without f.dead is the full pool)
+          if (stopped && !f.dead) { flat_leave(fb, fs); flat = false; }
+        }
       }
       if (!flat && !f.dead) {
 #pragma unroll 1
@@ -829,7 +726,7 @@ __global__ void __launch_bounds__(128, LOBSIM_REPLAY_FLAT_MIN_BLOCKS) k_replay_f
       }
       if (f.dead) { g += i; break; }                        // g: the message the book died of
       g = lim;
-      if (g == tile_end) { __syncwarp(); issue_tile(); }
+      if (g == tile_end) { __syncwarp(); mt.issue(); }
     }
     if (f.dead) {                                            // now_step: the step that holds message g (a step without messages holds none)
       while (__ldg(&st_step_off[now_step + 1]) <= g) now_step++;
@@ -839,34 +736,35 @@ __global__ void __launch_bounds__(128, LOBSIM_REPLAY_FLAT_MIN_BLOCKS) k_replay_f
     if (sub == steps_per_sec) {                              // whole second: outer-level resync, OrderbookSimulator.py:86-87
       sub = 0;
       if (c.resync && (!p.resync_last_only || t == T)) {
-        const double prop = ec.outer_prop;
-        const double bb = f.best0 == INT32_MIN ? 0.0 : (double)f.best0;
-        const double bs = f.best1 == INT32_MAX ? (double)INFINITY : (double)f.best1;
-        if (bb < (double)h->min_buy + prop * (double)h->init_buy_range || bs > (double)h->max_sell - prop * (double)h->init_sell_range) {
-          const int sec = now_step / steps_per_sec;
-          if (sec <= (int)stp->n_seconds && stp->snap_valid[sec]) {
-            const int32_t* row = stp->snapshots + (size_t)sec * 2 * c.n_levels * 2;
-            if (flat && !flat_resync_needed(h, row, c.n_levels, lane)) flat_update_trackers<LT>(base, lane, fs);
-            else {
-              if (flat) { flat_leave(fb, fs); flat = false; }
-              fast_resync(fb, f, row, c.n_levels);
-            }
+        if (const int32_t* row = resync_row(ec, h, stp, f.best0, f.best1, now_step, steps_per_sec)) {
+          if (flat && !flat_resync_needed(h, row, c.n_levels, lane)) flat_update_trackers<LT>(base, lane, fs);
+          else {
+            if (flat) { flat_leave(fb, fs); flat = false; }
+            fast_resync(fb, f, row, c.n_levels);
           }
         }
       }
-      if (flat && fs.seq > 0xE0000000u) { flat_leave(fb, fs); flat = false; }   // renumber the time-priority stamps long before they wrap
-      if (!flat && flat_fits(fb, 8)) { flat_enter(fb, fs); flat = true; }   // back to the flat pools once the book has shrunk
+      if constexpr (kPools) {
+        if (flat && fs.seq > 0xE0000000u) { flat_leave(fb, fs); flat = false; }   // renumber the time-priority stamps long before they wrap
+        if (!flat && flat_fits(fb, 8)) { flat_enter(fb, fs); flat = true; }   // back to the flat pools once the book has shrunk
+      }
     }
   }
   if (flat && !p.allow_flat) { flat_leave(fb, fs); flat = false; }   // the caller wants the canonical sorted layout in HBM
-  while (next_wait < next_issue) wait_tile();                // drain TMA loads still in flight (aborted episode)
-  __syncwarp();
-  if (lane == 0) { h->now_step = now_step; h->err = f.err; h->dead = f.dead; if (flat) flat_mark(h, fs); }
-  __syncwarp();
-  fence_proxy_async();
-  __syncwarp();
-  if (lane == 0) { tma_store(gblob, base, (uint32_t)LT::agent_off); tma_store_wait(); }
-  __syncwarp();
+  mt.drain();
+  replay_blob_store<LT>(gblob, base, lane, now_step, f, [&]() { if (flat) flat_mark(h, fs); });
+}
+
+#ifndef LOBSIM_REPLAY_FLAT_MIN_BLOCKS
+#define LOBSIM_REPLAY_FLAT_MIN_BLOCKS 7      // 72 registers: 28 resident warps per SM with the 64/256/32 blob (8 = 64 registers: A/B in profiles/)
+#endif
+template <class LT>
+__global__ void __launch_bounds__(128, LOBSIM_REPLAY_FLAT_MIN_BLOCKS) k_replay_flat(const __grid_constant__ AdvParams p, const __grid_constant__ EnvConst ec) {
+  replay_straight<LT, true>(p, ec);
+}
+template <class LT>
+__global__ void __launch_bounds__(128, 7) k_replay_fast(const __grid_constant__ AdvParams p, const __grid_constant__ EnvConst ec) {
+  replay_straight<LT, false>(p, ec);
 }
 
 // ====================================================================================================================
@@ -996,7 +894,7 @@ __global__ void __launch_bounds__(32 * LOBSIM_ENVFAST_WARPS, env_min_blocks<LT>(
   }
   fast_refresh_best(fb, f);
   const lobsim_stream_t* stp = &p.streams[stream_id];
-  const lobsim_msg_t* __restrict__ st_msgs = stp->msgs;
+  MsgTiles mt(stp);
   const uint32_t* __restrict__ st_step_off = stp->step_off;
   StepSave* sv = reinterpret_cast<StepSave*>(bars + 4);
   int now_step = h->now_step;
@@ -1031,27 +929,9 @@ __global__ void __launch_bounds__(32 * LOBSIM_ENVFAST_WARPS, env_min_blocks<LT>(
 
   // ---- message pipeline ----------------------------------------------------------------------------------------------
   const int T = p.T;
-  const int n_grid = (int)stp->n_grid_steps;   // steps beyond the end: the existing ones are run, the first one past the end sets END_OF_STREAM
-  if ((now_step < 0 || now_step > n_grid) && !f.dead && T > 0) { f.err |= LOBSIM_ERR_END_OF_STREAM; f.dead = 1; }
-  unsigned g = 0, g_end_all = 0;
-  if (!f.dead && T > 0) { g = __ldg(&st_step_off[now_step]); g_end_all = __ldg(&st_step_off[min((long long)now_step + T, (long long)n_grid)]); }
-  const unsigned tile0 = g / MSG_TILE;
-  unsigned next_issue = 0, next_wait = 0;
-  auto issue_tile = [&]() {
-    const unsigned first = (tile0 + next_issue) * MSG_TILE;
-    if (first >= g_end_all) return;
-    if (lane == 0) {
-      const unsigned n_total = (unsigned)stp->n_msgs;
-      const unsigned cnt = n_total - first < MSG_TILE ? n_total - first : MSG_TILE;
-      uint64_t* bar = &bars[next_issue & 1];
-      mbar_expect_tx(bar, cnt * 16);
-      tma_load(msgbuf + (next_issue & 1) * MSG_TILE_BYTES, st_msgs + first, cnt * 16, bar);
-    }
-    next_issue++;
-  };
-  auto wait_tile = [&]() { mbar_wait(&bars[next_wait & 1], (next_wait >> 1) & 1); next_wait++; };
-  if (g < g_end_all) { issue_tile(); issue_tile(); }
-  __syncwarp();
+  unsigned g, g_end_all;
+  stream_window(st_step_off, (int)stp->n_grid_steps, now_step, T, f.err, f.dead, g, g_end_all);
+  mt.start(msgbuf, bars, lane, g, g_end_all);
   if (SYNC) __syncthreads();
   const int steps_per_sec = ec.steps_per_sec;
   int sub = now_step >= 0 ? now_step % steps_per_sec : 0;
@@ -1104,13 +984,13 @@ __global__ void __launch_bounds__(32 * LOBSIM_ENVFAST_WARPS, env_min_blocks<LT>(
           is_agent = true;
         } else {
           if (f.dead || g >= g_step_end) break;
-          const unsigned tile = g / MSG_TILE - tile0;
-          if (tile == next_wait) wait_tile();
+          const unsigned tile = mt.rel(g);
+          if (tile == mt.next_wait) mt.wait();
           const uint4 m = *reinterpret_cast<const uint4*>(msgbuf + (tile & 1) * MSG_TILE_BYTES + (g % MSG_TILE) * 16);
           oprice = (int)m.x; vol = (int)m.y; ref = m.z; type = (int)(m.w & 7u); side = (int)((m.w >> 3) & 1u);
           is_agent = false;
           g++;
-          if (g % MSG_TILE == 0) { __syncwarp(); issue_tile(); }
+          if (g % MSG_TILE == 0) { __syncwarp(); mt.issue(); }
         }
         if (!f.dead) fast_order_full<LT, true>(fb, f, type, side, oprice, vol, ref, is_agent);
       }
@@ -1166,7 +1046,7 @@ __global__ void __launch_bounds__(32 * LOBSIM_ENVFAST_WARPS, env_min_blocks<LT>(
     if (lane < F) o[lane] = feat_cur;
     if (c.inc_prev_action_in_obs && lane < ec.action_dim) o[F + lane] = 0.0;
   }
-  while (next_wait < next_issue) wait_tile();
+  mt.drain();
 
   // ---- shared memory -> HBM: the header and the occupied part of the arrays; every issuing lane commits and waits for its own copy
   __syncwarp();

@@ -1,5 +1,5 @@
 // layouts.h -- the book capacities {levels, orders, agent orders per side} that have compiled straight-line kernels
-// (k_replay_fast / k_env_fast, book_fast.cuh).  Any other capacity triple runs on the general runtime-layout kernel
+// (k_replay_flat / k_replay_fast / k_replay_hyb / k_env_fast, kernels.cuh).  Any other capacity triple runs on the general runtime-layout kernel
 // k_advance (same results, about 2-3x the instructions per order); lobsim_kernel_path() tells which one a handle got.
 //
 // Each entry is compiled as its own translation units (fast_layout.cu with -DLOBSIM_LAYOUT_INDEX=i, see build.py), in

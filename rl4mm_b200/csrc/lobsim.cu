@@ -35,8 +35,7 @@ struct FastLayoutOps {
   int NL, NO, NA;
   cudaError_t (*attrs)(int dyn_replay, int dyn_env);
   cudaError_t (*attrs_rare)(int dyn_env);
-  void (*replay)(int grid, int block, size_t dyn, cudaStream_t stream, const AdvParams& p, const EnvConst& ec);
-  void (*replay_flat)(int grid, int block, size_t dyn, cudaStream_t stream, const AdvParams& p, const EnvConst& ec);
+  void (*replay)(ReplayKind kind, int grid, int block, size_t dyn, cudaStream_t stream, const AdvParams& p, const EnvConst& ec);
   void (*to_sorted)(unsigned char* blobs, int n_envs, cudaStream_t stream);
   void (*env)(bool sync, int grid, int block, size_t dyn, cudaStream_t stream, const AdvParams& p, const EnvConst& ec);
   void (*env_rare)(bool sync, int grid, int block, size_t dyn, cudaStream_t stream, const AdvParams& p, const EnvConst& ec);
@@ -44,14 +43,13 @@ struct FastLayoutOps {
 #define X(i, nl, no, na)                                                                                                   \
   cudaError_t lobsim_fast##i##_attrs(int, int);                                                                            \
   cudaError_t lobsim_fast##i##_attrs_rare(int);                                                                            \
-  void lobsim_fast##i##_replay(int, int, size_t, cudaStream_t, const AdvParams&, const EnvConst&);                         \
-  void lobsim_fast##i##_replay_flat(int, int, size_t, cudaStream_t, const AdvParams&, const EnvConst&);                    \
+  void lobsim_fast##i##_replay(ReplayKind, int, int, size_t, cudaStream_t, const AdvParams&, const EnvConst&);             \
   void lobsim_fast##i##_to_sorted(unsigned char*, int, cudaStream_t);                                                      \
   void lobsim_fast##i##_env(bool, int, int, size_t, cudaStream_t, const AdvParams&, const EnvConst&);                      \
   void lobsim_fast##i##_env_rare(bool, int, int, size_t, cudaStream_t, const AdvParams&, const EnvConst&);
 LOBSIM_FAST_LAYOUTS(X)
 #undef X
-#define X(i, nl, no, na) {nl, no, na, lobsim_fast##i##_attrs, lobsim_fast##i##_attrs_rare, lobsim_fast##i##_replay, lobsim_fast##i##_replay_flat, lobsim_fast##i##_to_sorted, lobsim_fast##i##_env, lobsim_fast##i##_env_rare},
+#define X(i, nl, no, na) {nl, no, na, lobsim_fast##i##_attrs, lobsim_fast##i##_attrs_rare, lobsim_fast##i##_replay, lobsim_fast##i##_to_sorted, lobsim_fast##i##_env, lobsim_fast##i##_env_rare},
 static const FastLayoutOps g_fast_layouts[LOBSIM_N_FAST_LAYOUTS] = {LOBSIM_FAST_LAYOUTS(X)};
 #undef X
 static const FastLayoutOps* find_fast_layout(const Layout& L) {
@@ -210,9 +208,7 @@ struct lobsim {
   lobsim_msg_t* st_msgs = nullptr; uint64_t st_msgs_cap = 0;
   bool has_reset = false;
   bool force_general = false;         // LOBSIM_FORCE_GENERAL=1: always use the runtime-layout kernels (testing)
-  int replay_hybrid = -1;             // k_replay_hyb (book_hybrid.cuh) as the replay launch of a deep compiled layout (NL >= 64, NO >= 512):
-                                      // -1 (default) when NO >= 1024, LOBSIM_REPLAY_HYBRID=1 on every such layout, =0 never
-  bool replay_flat = true;            // LOBSIM_REPLAY_FLAT=0: the replay fast path keeps every book in the sorted level arrays (A/B, testing)
+  ReplayKind replay_kind = REPLAY_FLAT; // the replay kernel of a compiled layout (lobsim_create, from LOBSIM_REPLAY_FLAT / _HYBRID)
   bool flat_blobs = true;             // LOBSIM_FLAT_BLOBS=0: the fast kernels never keep a book in the flat order pools across launches
                                       // (the flat replay converts back at the end of every launch)
   lobsim_order_t* po_orders = nullptr; uint32_t* po_refs = nullptr; lobsim_fill_t* po_fills = nullptr; int32_t* po_nf = nullptr;   // lobsim_process_orders staging
@@ -286,8 +282,6 @@ int lobsim_create(const lobsim_cfg_t* cfg, int device, lobsim_t** out) {
   if (!h) return fail(LOBSIM_E_NOMEM, "out of host memory");
   h->cfg = *cfg; h->device = device;
   { const char* e = getenv("LOBSIM_FORCE_GENERAL"); h->force_general = e && e[0] == '1'; }
-  { const char* e = getenv("LOBSIM_REPLAY_FLAT"); h->replay_flat = !(e && e[0] == '0'); }
-  { const char* e = getenv("LOBSIM_REPLAY_HYBRID"); h->replay_hybrid = e && e[0] == '1' ? 1 : e && e[0] == '0' ? 0 : -1; }
   { const char* e = getenv("LOBSIM_FLAT_BLOBS"); h->flat_blobs = !(e && e[0] == '0'); }
   h->rare_paths = cfg->step_reward.kind == LOBSIM_REWARD_ROLLING_SHARPE || cfg->terminal_reward.kind == LOBSIM_REWARD_ROLLING_SHARPE;
   for (int i = 0; i < cfg->n_features; i++) h->rare_paths = h->rare_paths || cfg->features[i].norm_len > 0;
@@ -336,6 +330,12 @@ int lobsim_create(const lobsim_cfg_t* cfg, int device, lobsim_t** out) {
   CUDA_TRY((cudaFuncSetAttribute(k_advance<false, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, h->warps_per_cta * h->warp_smem)));
   h->fast = h->force_general ? nullptr : find_fast_layout(h->L);
   if (h->fast) {
+    // LOBSIM_REPLAY_FLAT=0: sorted level arrays only.  Otherwise the hybrid book on a deep layout (NL >= 64, NO >= 512) when
+    // LOBSIM_REPLAY_HYBRID=1, or by default when NO >= 1024 (=0: never); the flat order pools on every other layout.
+    const char* ef = getenv("LOBSIM_REPLAY_FLAT"); const char* eh = getenv("LOBSIM_REPLAY_HYBRID");
+    const int hybrid = eh && eh[0] == '1' ? 1 : eh && eh[0] == '0' ? 0 : -1;
+    if (ef && ef[0] == '0') h->replay_kind = REPLAY_SORTED;
+    else if (h->fast->NL >= 64 && h->fast->NO >= 512 && (hybrid > 0 || (hybrid < 0 && h->fast->NO >= 1024))) h->replay_kind = REPLAY_HYBRID;
     CUDA_TRY(h->fast->attrs(h->replay_warps_per_cta * h->replay_warp_smem, h->env_warps_per_cta * h->warp_smem));
     if (h->rare_paths) CUDA_TRY(h->fast->attrs_rare(h->env_warps_per_cta * h->warp_smem));
   } else if (!h->force_general) {
@@ -493,17 +493,14 @@ static int launch_advance(lobsim* h, const AdvParams& p, cudaStream_t stream) {
 
 static int launch_replay_fast(lobsim* h, const AdvParams& p, cudaStream_t stream) {
   if (h->streams.empty()) return fail(LOBSIM_E_STATE, "no stream loaded");
-  if (!h->fast) return 1;
   CUDA_TRY(cudaSetDevice(h->device));
   const int wpc = h->replay_warps_per_cta, grid = (p.n_sel + wpc - 1) / wpc;
   if (grid <= 0) return LOBSIM_OK;
   AdvParams pr = p;
   pr.warp_smem = h->replay_warp_smem;
-  pr.hybrid = h->replay_flat && h->fast->NL >= 64 && h->fast->NO >= 512 && (h->replay_hybrid > 0 || (h->replay_hybrid < 0 && h->fast->NO >= 1024)) ? 1 : 0;
-  if (pr.hybrid) pr.allow_flat = 0;
-  if (!h->replay_flat || pr.hybrid) { int rc = ensure_sorted(h, stream); if (rc) return rc; }
+  if (h->replay_kind != REPLAY_FLAT) { int rc = ensure_sorted(h, stream); if (rc) return rc; }
   else if (p.allow_flat) h->maybe_flat = true;
-  (h->replay_flat ? h->fast->replay_flat : h->fast->replay)(grid, wpc * 32, (size_t)wpc * h->replay_warp_smem, stream, pr, h->ec);
+  h->fast->replay(h->replay_kind, grid, wpc * 32, (size_t)wpc * h->replay_warp_smem, stream, pr, h->ec);
   CUDA_TRY(cudaGetLastError());
   h->launches++;
   return LOBSIM_OK;
@@ -633,10 +630,7 @@ int lobsim_replay(lobsim_t* h, int32_t n_steps, void* stream) {
   AdvParams p; base_params(h, p);
   p.T = n_steps; p.agent_kind = LOBSIM_AGENT_NONE;
   // fast path: no fill log requested and no agent order can be resting in any book
-  if (!h->fill_log && !h->agent_orders_possible && h->fast) {
-    int rc = launch_replay_fast(h, p, (cudaStream_t)stream);
-    if (rc != 1) return rc; // 1: no compiled StaticLayout matches these capacities
-  }
+  if (!h->fill_log && !h->agent_orders_possible && h->fast) return launch_replay_fast(h, p, (cudaStream_t)stream);
   return launch_advance<false, true>(h, p, (cudaStream_t)stream);
 }
 
