@@ -254,11 +254,8 @@ __device__ __forceinline__ void record_external(WarpState& w, int dir, int vol) 
 
 // ---- Exchange.submit_order (no-cross branch), Exchange.py:74-83 ------------------------------------------------
 // returns the agent id given to the order, 0xffffffff for an external order that rested, 0 on overflow
-// TR == false is the replay fast path: no agent orders can rest in the book, fills are not recorded.
-template <bool TR>
 __device__ __forceinline__ uint32_t rest_order(const Book& b, WarpState& w, int side, int price, int vol, uint32_t ref, bool is_agent) {
-  if (!TR) is_agent = false;
-  int nag = TR ? NAG(w, side) : 0;
+  int nag = NAG(w, side);
   if (is_agent && nag >= b.L.NA) { w.err |= LOBSIM_ERR_AGENT_OVERFLOW; return 0; }
   if (NORD(w, side) >= b.L.NO) { w.err |= LOBSIM_ERR_ORDER_OVERFLOW; return 0; }
   bool found;
@@ -278,9 +275,7 @@ __device__ __forceinline__ uint32_t rest_order(const Book& b, WarpState& w, int 
 
 // ---- Exchange.submit_order / execute_order, Exchange.py:71-120 --------------------------------------------------
 // is_limit: LimitOrder (crosses only while price allows, remainder rests); else MarketOrder.
-template <bool TR>
 __device__ __forceinline__ uint32_t submit_or_execute(const Book& b, WarpState& w, int side, int price, int vol, uint32_t ref, bool is_limit, bool is_agent) {
-  if (!TR) is_agent = false;
   int rem = vol;
   const int opp = side ^ 1;
   while (rem > 0) {
@@ -294,7 +289,7 @@ __device__ __forceinline__ uint32_t submit_or_execute(const Book& b, WarpState& 
     if (is_limit && !(side == 0 ? price >= bp : price <= bp)) break;     // _does_order_cross_spread :188-194
     int start = level_start(b, opp, j);
     uint2 head = b.ord(opp)[start];
-    const bool hagent = TR && (head.y & LOBSIM_REF_AGENT) != 0;
+    const bool hagent = (head.y & LOBSIM_REF_AGENT) != 0;
     __syncwarp();
     if (is_agent && hagent) { // cannot fill our own order => delete it, :91-94
       remove_entries(b, w, opp, j, start, 1);
@@ -309,7 +304,7 @@ __device__ __forceinline__ uint32_t submit_or_execute(const Book& b, WarpState& 
       agent_reduce(b, w, opp, head.y & 0x7fffffffu, v, false);
       record_internal(w, opp, bp, v);
       log_fill(b, w, 0, opp, bp, v, 0, head.y);
-    } else if (TR) {
+    } else {
       record_external(w, opp, v);
       log_fill(b, w, 1, opp, bp, v, 0, head.y);
     }
@@ -319,15 +314,13 @@ __device__ __forceinline__ uint32_t submit_or_execute(const Book& b, WarpState& 
       log_fill(b, w, 0, side, bp, v, 1, head.y);
     }
   }
-  if (rem > 0 && is_limit) return rest_order<TR>(b, w, side, price, rem, ref, is_agent); // :116-119 / :74-83
+  if (rem > 0 && is_limit) return rest_order(b, w, side, price, rem, ref, is_agent); // :116-119 / :74-83
   return 0;
 }
 
 // ---- Exchange.remove_order, Exchange.py:122-147 ------------------------------------------------------------------
 // has_vol == false: Deletion with volume None (full delete).
-template <bool TR>
 __device__ __forceinline__ void remove_order(const Book& b, WarpState& w, int side, int price, int vol, bool has_vol, uint32_t ref, bool is_agent) {
-  if (!TR) is_agent = false;
   bool found;
   int j = find_level(b, side, NLV(w, side), price, found);
   if (!found) return;                                  // KeyError => continue, :129-132
@@ -355,12 +348,11 @@ __device__ __forceinline__ void remove_order(const Book& b, WarpState& w, int si
 }
 
 // ---- Exchange.process_order, Exchange.py:58-69: the ONE call site of the general book routines in a kernel ---------
-template <bool TR>
 __device__ __forceinline__ void process_order(const Book& b, WarpState& w, int type, int side, int price, int vol, uint32_t ref, bool is_agent) {
   if (w.dead) return;
   if (vol <= 0) { w.err |= LOBSIM_ERR_BAD_VOLUME; return; }
-  if (type == LOBSIM_MSG_LIMIT || type == LOBSIM_MSG_MARKET) submit_or_execute<TR>(b, w, side, price, vol, ref, type == LOBSIM_MSG_LIMIT, is_agent);
-  else remove_order<TR>(b, w, side, price, vol, true, ref, is_agent);
+  if (type == LOBSIM_MSG_LIMIT || type == LOBSIM_MSG_MARKET) submit_or_execute(b, w, side, price, vol, ref, type == LOBSIM_MSG_LIMIT, is_agent);
+  else remove_order(b, w, side, price, vol, true, ref, is_agent);
 }
 
 // ---- Orderbook properties, rl4mm/orderbook/models.py:72-101 -------------------------------------------------------
@@ -380,25 +372,20 @@ __device__ __forceinline__ double microprice(int bb, int bs, int bv, int sv, dou
 }
 
 // ---- WarpState <-> header ----------------------------------------------------------------------------------------
-// FULL == false (replay fast path): only the book counters live in registers; portfolio / agent fields stay in the
-// header untouched.
-template <bool FULL>
 __device__ __forceinline__ void load_state(const Book& b, WarpState& w) {
   const BookHdr* h = b.hdr();
   w.nlv0 = h->cnt[0][0]; w.nlv1 = h->cnt[1][0]; w.nord0 = h->cnt[0][1]; w.nord1 = h->cnt[1][1];
   w.err = h->err; w.dead = h->dead;
-  w.nag0 = w.nag1 = 0; w.next_agent_id = 0; w.inventory = 0; w.cash = 0.0;
-  if (FULL) { w.nag0 = h->nag[0]; w.nag1 = h->nag[1]; w.next_agent_id = h->next_agent_id; w.inventory = h->inventory; w.cash = h->cash; }
+  w.nag0 = h->nag[0]; w.nag1 = h->nag[1]; w.next_agent_id = h->next_agent_id; w.inventory = h->inventory; w.cash = h->cash;
   w.n_ext0 = w.n_ext1 = w.vol_ext0 = w.vol_ext1 = w.n_int0 = w.n_int1 = w.vol_int0 = w.vol_int1 = 0;
 }
-template <bool FULL>
 __device__ __forceinline__ void store_state(const Book& b, const WarpState& w) {
   __syncwarp();
   if (b.lane == 0) {
     BookHdr* h = b.hdr();
     h->cnt[0][0] = w.nlv0; h->cnt[1][0] = w.nlv1; h->cnt[0][1] = w.nord0; h->cnt[1][1] = w.nord1;
     h->err = w.err; h->dead = w.dead;
-    if (FULL) { h->nag[0] = w.nag0; h->nag[1] = w.nag1; h->next_agent_id = w.next_agent_id; h->inventory = w.inventory; h->cash = w.cash; }
+    h->nag[0] = w.nag0; h->nag[1] = w.nag1; h->next_agent_id = w.next_agent_id; h->inventory = w.inventory; h->cash = w.cash;
   }
   __syncwarp();
 }

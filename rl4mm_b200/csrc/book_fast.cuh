@@ -424,7 +424,7 @@ __device__ __forceinline__ void fast_find_any(const FastBook<LT>& fb, unsigned c
   }
   __syncwarp();
 }
-// Exchange.submit_order, no-cross branch (Exchange.py:74-83) = book.cuh rest_order<false>: same result, same overflow flags
+// Exchange.submit_order, no-cross branch (Exchange.py:74-83) = book.cuh rest_order: same result, same overflow flags
 template <class LT, bool TR>
 __device__ __forceinline__ void fast_rest_any(const FastBook<LT>& fb, FastState& f, int side, int price, int vol, uint32_t ref, bool is_agent) {
   if (!TR) is_agent = false;
@@ -481,7 +481,7 @@ __device__ __forceinline__ void fast_rest_any(const FastBook<LT>& fb, FastState&
   __syncwarp();
   fast_refresh_best(fb, f);
 }
-// Exchange.remove_order (Exchange.py:122-147) = book.cuh remove_order<false> with a volume
+// Exchange.remove_order (Exchange.py:122-147) = book.cuh remove_order with a volume
 template <class LT, bool TR>
 __device__ __forceinline__ void fast_remove_any(const FastBook<LT>& fb, FastState& f, int side, int price, int vol, uint32_t ref, bool is_agent) {
   if (!TR) is_agent = false;

@@ -19,25 +19,12 @@
 #pragma once
 #include "book_flat.cuh"
 
-#ifndef HYB_COLD_ATTR
-#define HYB_COLD_ATTR __forceinline__   // the cold-array routines: inline (measured: 3.47e9 msgs/s vs 2.75e9 out of line, BASELINE config 5)
-#endif
-#ifndef HYB_REFILL_ATTR
-#define HYB_REFILL_ATTR __noinline__    // the level moves: out of line (inline: 2.71e9)
-#endif
-#ifndef HYB_SPILL_ATTR
-#define HYB_SPILL_ATTR __noinline__
-#endif
 #define HYB_CAP 128
 #define HYB_NCH 4
 #define HYB_BAIL_DONE 4          // leave the hybrid form; the order itself is complete
-#ifndef HYB_REFILL_BELOW
 #define HYB_REFILL_BELOW 96      // refill the pool from the cold levels at step boundaries when it holds fewer orders than this
                                  // (measured on BASELINE config 5: 16/64 3.39e9, 32/80 3.48e9, 96/120 3.65e9 msgs/s)
-#endif
-#ifndef HYB_REFILL_TO
 #define HYB_REFILL_TO 120
-#endif
 
 template <class LT>
 __host__ __device__ constexpr bool hyb_layout() { return LT::NO >= 512 && LT::NL >= 64; }
@@ -57,9 +44,10 @@ struct HybState {
 };
 
 // ---- cold -> hot: the best cold level moves into the pool (if the pool has room).  Keeps f.best of the side current. ----------
-// (out of line: called from half a dozen places of hyb_order, rarely)   returns {orders moved or -1, the level's price}
+// (out of line: called from half a dozen places of hyb_order, rarely; inline: 2.71e9 msgs/s, BASELINE config 5)
+// returns {orders moved or -1, the level's price}
 template <class LT, int S>
-static __device__ HYB_REFILL_ATTR int2 hyb_refill_fn(unsigned char* blob, int lane, int n, unsigned seq) {
+static __device__ __noinline__ int2 hyb_refill_fn(unsigned char* blob, int lane, int n, unsigned seq) {
   FastBook<LT> fb; fb.blob = blob; fb.lane = lane;
   unsigned char* sb = fb.side(S);
   __syncwarp();
@@ -92,16 +80,17 @@ __device__ __forceinline__ bool hyb_refill_one(const FastBook<LT>& fb, FastState
   return true;
 }
 
-// the any-depth routines of book_fast.cuh on the cold arrays, out of line (one copy for both sides); return the error bits
+// the any-depth routines of book_fast.cuh on the cold arrays (one copy for both sides); return the error bits.  Inline (measured:
+// 3.47e9 msgs/s vs 2.75e9 out of line, BASELINE config 5)
 template <class LT>
-static __device__ HYB_COLD_ATTR uint32_t hyb_cold_rest_fn(unsigned char* blob, int lane, int side, int price, int vol, uint32_t ref) {
+static __device__ __forceinline__ uint32_t hyb_cold_rest_fn(unsigned char* blob, int lane, int side, int price, int vol, uint32_t ref) {
   FastBook<LT> fb; fb.blob = blob; fb.lane = lane;
   FastState t; t.err = 0; t.dead = 0; t.bail = 0; t.bail_vol = 0; t.best0 = t.best1 = 0;
   fast_rest_any<LT, false>(fb, t, side, price, vol, ref, false);
   return t.err;
 }
 template <class LT>
-static __device__ HYB_COLD_ATTR uint32_t hyb_cold_remove_fn(unsigned char* blob, int lane, int side, int price, int vol, uint32_t ref) {
+static __device__ __forceinline__ uint32_t hyb_cold_remove_fn(unsigned char* blob, int lane, int side, int price, int vol, uint32_t ref) {
   FastBook<LT> fb; fb.blob = blob; fb.lane = lane;
   FastState t; t.err = 0; t.dead = 0; t.bail = 0; t.bail_vol = 0; t.best0 = t.best1 = 0;
   fast_remove_any<LT, false>(fb, t, side, price, vol, ref, false);
@@ -110,7 +99,7 @@ static __device__ HYB_COLD_ATTR uint32_t hyb_cold_remove_fn(unsigned char* blob,
 
 // ---- hot -> cold: the worst hot level, in time priority, becomes the best cold level.  false: no room in the cold arrays. --------
 template <class LT, int S>
-static __device__ HYB_SPILL_ATTR int hyb_spill_fn(unsigned char* blob, int lane, int n) {   // returns the new pool size, or -1
+static __device__ __noinline__ int hyb_spill_fn(unsigned char* blob, int lane, int n) {   // returns the new pool size, or -1
   FastBook<LT> fb; fb.blob = blob; fb.lane = lane;
   unsigned char* sb = fb.side(S);
   uint4* pool = hyb_pool<LT>(blob, S);

@@ -64,7 +64,6 @@ __device__ __forceinline__ bool near_exiting(const Book& b, const WarpState& w, 
 
 // ---- OrderbookSimulator.update_outer_levels, OrderbookSimulator.py:105-135 ---------------------------------------
 // scratch: per-warp shared int2[2*NA] for the agent orders that are cancelled and re-queued behind the aggregates.
-template <bool TR>
 __device__ __forceinline__ void update_outer_levels_impl(const Book& b, WarpState& w, const lobsim_cfg_t& c, const int32_t* __restrict__ row, int2* scratch) {
   BookHdr* h = b.hdr();
   const int L = c.n_levels;
@@ -75,7 +74,7 @@ __device__ __forceinline__ void update_outer_levels_impl(const Book& b, WarpStat
       int price = __ldg(&row[(side * L + lvl) * 2]), vol = __ldg(&row[(side * L + lvl) * 2 + 1]);
       if (price == LOBSIM_NO_PRICE) continue;
       if (!(side == 0 ? price < min_buy : price > max_sell)) continue; // _initial_prices_filter_function :99-103
-      for (int i = 0; TR && i < NAG(w, side);) { // internal orders at this price: cancel now, re-queue later (:116-129)
+      for (int i = 0; i < NAG(w, side);) { // internal orders at this price: cancel now, re-queue later (:116-129)
         int ap = b.aprice(side)[i], av = b.avol(side)[i];
         uint32_t id = b.aid(side)[i];
         __syncwarp();
@@ -83,7 +82,7 @@ __device__ __forceinline__ void update_outer_levels_impl(const Book& b, WarpStat
         if (b.lane == 0) scratch[nrepl] = make_int2(price, av);
         nrepl++;
         int before = NAG(w, side);
-        remove_order<TR>(b, w, side, price, av, true, LOBSIM_REF_AGENT | id, true);
+        remove_order(b, w, side, price, av, true, LOBSIM_REF_AGENT | id, true);
         if (NAG(w, side) == before) agent_remove_at(b, w, side, i); // keep internal and central consistent
       }
       bool found;
@@ -103,9 +102,9 @@ __device__ __forceinline__ void update_outer_levels_impl(const Book& b, WarpStat
     if (side == 0) nrepl_buy = nrepl;
   }
   __syncwarp();
-  for (int i = 0; TR && i < nrepl; i++) { // :132-133
+  for (int i = 0; i < nrepl; i++) { // :132-133
     int2 r = scratch[i];
-    submit_or_execute<TR>(b, w, i < nrepl_buy ? 0 : 1, r.x, r.y, 0, true, true);
+    submit_or_execute(b, w, i < nrepl_buy ? 0 : 1, r.x, r.y, 0, true, true);
   }
   if (b.lane == 0) { // :134-135 (Exchange.orderbook_price_range, Exchange.py:160-170)
     if (w.nlv0 && b.lvp(0)[0] < h->min_buy) h->min_buy = b.lvp(0)[0];
@@ -115,9 +114,8 @@ __device__ __forceinline__ void update_outer_levels_impl(const Book& b, WarpStat
 }
 
 // cold wrapper: a real function call keeps the second copy of the book routines out of the kernel's hot code
-template <bool TR>
 static __device__ __noinline__ WarpState update_outer_levels(const Book b, WarpState w, const lobsim_cfg_t* c, const int32_t* row, int2* scratch) {
-  update_outer_levels_impl<TR>(b, w, *c, row, scratch);
+  update_outer_levels_impl(b, w, *c, row, scratch);
   return w;
 }
 

@@ -1,7 +1,8 @@
-// fast_layout.cu -- ONE compiled StaticLayout of the straight-line kernels (k_replay_flat / k_replay_fast / k_replay_hyb /
-// k_env_fast, kernels.cuh).
+// fast_layout.cu -- ONE compiled StaticLayout of the straight-line kernels (kernels.cuh): the three instantiations of
+// replay_straight (k_replay_flat / k_replay_fast / k_replay_hyb), k_to_sorted and k_env_fast.
 // Compiled once per entry of layouts.h and per part (-DLOBSIM_LAYOUT_INDEX=i -DLOBSIM_TU_PART=p, build.py), in parallel:
-//   part 0: the replay kernels + the env kernels without the z-score / RollingSharpe code
+//   part 0: the replay kernels (k_replay_hyb only for the deep layouts of hyb_layout()) + the env kernels without the z-score /
+//           RollingSharpe code
 //   part 1: the env kernels with that code (RARE)
 // lobsim.cu calls the launchers below through the FastLayoutOps table.
 #include "kernels.cuh"

@@ -201,9 +201,8 @@ struct MsgTiles {
 // ====================================================================================================================
 //  the advance kernel: [reset] + T x ([agent orders] + messages of the step + [resync] + [features, reward])
 // ====================================================================================================================
-// kEnv: agent + features + rewards (HistoricalOrderbookEnvironment.step); kTrack: fills / flows / agent orders are
-// tracked (always with kEnv; the pure replay fast path <false,false> is used when no agent order can be resting).
-template <bool kEnv, bool kTrack>
+// kEnv: agent + features + rewards (HistoricalOrderbookEnvironment.step); fills / flows / agent orders are tracked either way.
+template <bool kEnv>
 __global__ void __launch_bounds__(128, kEnv ? LOBSIM_ENV_MIN_BLOCKS : 4) k_advance(const __grid_constant__ AdvParams p, const __grid_constant__ EnvConst ec) {
   extern __shared__ __align__(128) unsigned char smem[];
   const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
@@ -236,7 +235,7 @@ __global__ void __launch_bounds__(128, kEnv ? LOBSIM_ENV_MIN_BLOCKS : 4) k_advan
   if (!p.blob_in_global) mbar_wait(&bars[2], 0);
 
   WarpState w;
-  load_state<kTrack>(b, w);
+  load_state(b, w);
   w.fill_log = p.fill_log ? p.fill_log + (size_t)env * p.fill_cap : nullptr;
   w.fill_cap = p.fill_cap; w.n_fills = 0;
   const long long inventory_in = w.inventory; const double cash_in = w.cash;
@@ -245,7 +244,7 @@ __global__ void __launch_bounds__(128, kEnv ? LOBSIM_ENV_MIN_BLOCKS : 4) k_advan
 
   // ---- reset prologue ----------------------------------------------------------------------------------------------
   int stream_id = h->stream_id;
-  if (kTrack && p.reset_mode) {
+  if (p.reset_mode) {
     stream_id = p.reset_stream_ids[sel];
     int start = p.reset_steps[sel] - (p.reset_mode == 2 ? c.warmup_steps : 0);
     if (stream_id < 0 || stream_id >= p.n_streams) { stream_id = 0; start = -1; }
@@ -349,7 +348,7 @@ __global__ void __launch_bounds__(128, kEnv ? LOBSIM_ENV_MIN_BLOCKS : 4) k_advan
           g++;
           if (g % MSG_TILE == 0) { __syncwarp(); mt.issue(); } // tile consumed: refill its buffer
         }
-        process_order<kTrack>(b, w, type, side, price, vol, ref, is_agent);
+        process_order(b, w, type, side, price, vol, ref, is_agent);
       }
     }
     if (!w.dead) {
@@ -360,7 +359,7 @@ __global__ void __launch_bounds__(128, kEnv ? LOBSIM_ENV_MIN_BLOCKS : 4) k_advan
         if (rel % 1000000 == 0 && near_exiting(b, w, c)) {
           long long sec = rel / 1000000;
           if (sec <= (long long)stp->n_seconds && stp->snap_valid[sec]) {
-            w = update_outer_levels<kTrack>(b, w, &ec.cfg, stp->snapshots + (size_t)sec * 2 * c.n_levels * 2, scratch);
+            w = update_outer_levels(b, w, &ec.cfg, stp->snapshots + (size_t)sec * 2 * c.n_levels * 2, scratch);
                     }
         }
       }
@@ -408,7 +407,7 @@ __global__ void __launch_bounds__(128, kEnv ? LOBSIM_ENV_MIN_BLOCKS : 4) k_advan
     h->price = price;
     if (p.fill_count) p.fill_count[env] = w.n_fills;
   }
-  store_state<kTrack>(b, w);
+  store_state(b, w);
   fence_proxy_async();
   __syncwarp();
   if (lane == 0 && !p.blob_in_global) { tma_store(gblob, base, (uint32_t)p.L.blob_bytes); tma_store_wait(); }
@@ -459,116 +458,6 @@ __device__ __forceinline__ const int32_t* resync_row(const EnvConst& ec, const B
   return nullptr;
 }
 __device__ __forceinline__ bool hdr_is_flat(const BookHdr* h) { return h->cnt[0][0] < 0; }
-// ====================================================================================================================
-//  the replay HYBRID kernel (deep layouts): the hybrid book of book_hybrid.cuh -- the levels near the touch in a flat order pool,
-//  the rest in the sorted arrays -- for every book that can take that form, the sorted straight-line path for the others.  One grid
-//  step at a time: the pools are topped up at every step boundary.  The blob in HBM is the canonical sorted layout on entry and on exit.
-// ====================================================================================================================
-template <class LT>
-__global__ void __launch_bounds__(128, 3) k_replay_hyb(const __grid_constant__ AdvParams p, const __grid_constant__ EnvConst ec) {
-  extern __shared__ __align__(128) unsigned char smem[];
-  const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
-  const int env = blockIdx.x * (blockDim.x >> 5) + warp;
-  if (env >= p.n_sel) return;
-  const lobsim_cfg_t& c = ec.cfg;
-  unsigned char* base = warp_smem_base(smem, warp, p.warp_smem);
-  unsigned char* msgbuf = base + LT::agent_off;
-  uint64_t* bars = reinterpret_cast<uint64_t*>(msgbuf + 2 * MSG_TILE_BYTES);
-  unsigned char* gblob = p.blobs + (size_t)env * LT::blob_bytes;
-  replay_blob_load<LT>(base, gblob, bars, lane);
-
-  FastBook<LT> fb; fb.blob = base; fb.lane = lane;
-  BookHdr* h = reinterpret_cast<BookHdr*>(base);
-  FastState f; f.err = h->err; f.dead = h->dead; f.bail = 0; f.bail_vol = 0;
-  if (hdr_is_flat(h)) flat_leave_fn<LT>(base, lane, h->cnt[0][1], h->cnt[1][1]);   // (a blob stored by the flat kernels)
-  fast_refresh_best(fb, f);
-  HybState hs; hs.n0 = hs.n1 = 0; hs.floor0 = INT32_MIN; hs.floor1 = INT32_MAX; hs.seq = 0;
-  bool hyb = false;
-  const lobsim_stream_t* stp = &p.streams[h->stream_id];
-  MsgTiles mt(stp);
-  const uint32_t* __restrict__ st_step_off = stp->step_off;
-  int now_step = h->now_step;
-  const int T = p.T;
-  const int n_grid = (int)stp->n_grid_steps;
-  unsigned g, g_end_all;
-  stream_window(st_step_off, n_grid, now_step, T, f.err, f.dead, g, g_end_all);
-  auto try_enter = [&]() {
-    if (hyb_enter(fb, f, hs)) hyb = true;
-    else if (hs.n0 | hs.n1) { hyb_leave(fb, f, hs); hs.n0 = hs.n1 = 0; }      // one side was moved, the other could not be: put it back
-  };
-  if (g < g_end_all) try_enter();
-  mt.start(msgbuf, bars, lane, g, g_end_all);
-  const int steps_per_sec = ec.steps_per_sec;
-  int sub = now_step >= 0 ? now_step % steps_per_sec : 0;
-
-#pragma unroll 1
-  for (int t = 0; t < T && !f.dead; t++) {
-    if (now_step >= n_grid) { f.err |= LOBSIM_ERR_END_OF_STREAM; f.dead = 1; break; }
-    const unsigned g_step_end = __ldg(&st_step_off[now_step + 1]);
-#pragma unroll 1
-    while (g < g_step_end) {
-      const unsigned tile = mt.rel(g);
-      if (tile == mt.next_wait) mt.wait();
-      const unsigned tile_end = (g / MSG_TILE + 1) * MSG_TILE;
-      const unsigned lim = g_step_end < tile_end ? g_step_end : tile_end;
-      const uint4* mp = reinterpret_cast<const uint4*>(msgbuf + (tile & 1) * MSG_TILE_BYTES) + (g % MSG_TILE);
-      const unsigned cnt = lim - g;
-      unsigned i = 0;
-      int redo_vol = 0;
-      // the volumes of the whole segment (<= 32 messages, one per lane) at once: a segment with a bad one (never in valid data) runs on
-      // the sorted book, whose routines test every order (assert order.volume > 0, Exchange.py:59-60)
-      if (hyb && __any_sync(FULL_MASK, (unsigned)lane < cnt && (int)mp[(unsigned)lane < cnt ? lane : 0].y <= 0)) {
-        hyb_leave(fb, f, hs); hyb = false; hs.n0 = hs.n1 = 0;
-      }
-      if (hyb) {
-#pragma unroll 1
-        for (; i < cnt; i++) {
-          const uint4 m = mp[i];
-          if (hyb_message<LT>(fb, f, hs, (int)m.x, (int)m.y, m.z, m.w)) break;
-        }
-        if (f.bail) {                                        // this book cannot stay hybrid: back to the sorted form
-          const int why = f.bail, rest = f.bail_vol;
-          f.bail = 0; f.bail_vol = 0;
-          hyb_leave(fb, f, hs); hyb = false; hs.n0 = hs.n1 = 0;
-          if (why == FLAT_BAIL_FULL) redo_vol = rest;        // the unfinished part of message i runs on the sorted book
-          else i++;
-        }
-      }
-      if (!hyb && !f.dead) {
-#pragma unroll 1
-        for (; i < cnt; i++) {
-          const uint4 m = mp[i];
-          const int v = redo_vol ? redo_vol : (int)m.y;
-          redo_vol = 0;
-          fast_message(fb, f, (int)m.x, v, m.z, m.w);
-          if (f.dead) break;
-        }
-      }
-      if (f.dead) break;
-      g = lim;
-      if (g == tile_end) { __syncwarp(); mt.issue(); }
-    }
-    if (f.dead) break;
-    now_step++;
-    if (hyb) hyb_top_up(fb, f, hs);
-    if (++sub == steps_per_sec) {                            // whole second: outer-level resync, OrderbookSimulator.py:86-87
-      sub = 0;
-      if (c.resync && (!p.resync_last_only || t == T - 1)) {
-        if (const int32_t* row = resync_row(ec, h, stp, f.best0, f.best1, now_step, steps_per_sec)) {
-          if (hyb && !flat_resync_needed(h, row, c.n_levels, lane)) hyb_update_trackers(fb, hs);
-          else {
-            if (hyb) { hyb_leave(fb, f, hs); hyb = false; hs.n0 = hs.n1 = 0; }
-            fast_resync(fb, f, row, c.n_levels);
-          }
-        }
-      }
-      if (!hyb) try_enter();
-    }
-  }
-  if (hyb) hyb_leave(fb, f, hs);
-  mt.drain();
-  replay_blob_store<LT>(gblob, base, lane, now_step, f, []() {});
-}
 
 // ---- the flat form of a blob in HBM (book_flat.cuh): header with cnt[0] = {-1, n0}, cnt[1] = {seq, n1}; per side the order pool
 //      (n x 16 B at the start of the side's order array); the agent tables as always.  Parts: lanes 0-1 the pools, 2-7 the agent tables.
@@ -638,15 +527,38 @@ __global__ void __launch_bounds__(128) k_to_sorted(unsigned char* blobs, int n_e
 }
 
 // ====================================================================================================================
-//  the straight-line replay kernels: T x (messages of the step + [resync]) with the straight-line message paths, one pass per
-//  second.  Used by lobsim_replay when no fill log is requested, no agent order can be resting and the book capacities match one
-//  of the compiled StaticLayouts.  kPools (k_replay_flat): the flat order pools of book_flat.cuh for every book that fits them (at
-//  most FLAT_CAP resting orders per side), the sorted straight-line path of book_fast.cuh for the others -- per book, re-decided
-//  every second.  Without (k_replay_fast): the sorted path for every book.  The blob in HBM is the canonical sorted layout on
-//  entry and on exit.
+//  the straight-line replay kernels: T x (messages of the step + [resync]) with the straight-line message paths.  Used by
+//  lobsim_replay when no fill log is requested, no agent order can be resting and the book capacities match one of the compiled
+//  StaticLayouts.  kForm is the form a book runs in where it can (per book, re-decided every second); the others run on the sorted
+//  straight-line path of book_fast.cuh:
+//    REPLAY_SORTED (k_replay_fast): the sorted path for every book;
+//    REPLAY_FLAT   (k_replay_flat): the flat order pools of book_flat.cuh for every book that fits them (at most FLAT_CAP resting
+//                  orders per side);
+//    REPLAY_HYBRID (k_replay_hyb, deep layouts): the hybrid book of book_hybrid.cuh -- the levels near the touch in a flat order
+//                  pool, the rest in the sorted arrays -- for every book that can take that form.
+//  The blob in HBM is the canonical sorted layout on entry, and on exit unless the flat form may be stored (p.allow_flat).  The
+//  kind of a handle is fixed in lobsim_create, only REPLAY_FLAT launches store the flat form, and the host converts every blob
+//  to the sorted form (ensure_sorted) before a launch of any other kind: so only the REPLAY_FLAT kernel meets a flat blob.
 // ====================================================================================================================
-template <class LT, bool kPools>
+// (forced-inline functions, not lambdas: with lambdas the compiler schedules k_replay_flat differently)
+// sorted -> the pool form of kForm, where the book can take it (the flat pools: with `slack` orders to spare per side)
+template <class LT, ReplayKind kForm>
+__device__ __forceinline__ void pool_enter(const FastBook<LT>& fb, FastState& f, FlatState& fs, HybState& hs, bool& flat, int slack) {
+  if constexpr (kForm == REPLAY_HYBRID) {
+    if (hyb_enter(fb, f, hs)) flat = true;
+    else if (hs.n0 | hs.n1) { hyb_leave(fb, f, hs); hs.n0 = hs.n1 = 0; }   // one side was moved, the other could not be: put it back
+  } else if (flat_fits(fb, slack)) { flat_enter(fb, fs); flat = true; }
+}
+// pool form -> sorted
+template <class LT, ReplayKind kForm>
+__device__ __forceinline__ void pool_leave(const FastBook<LT>& fb, FastState& f, FlatState& fs, HybState& hs, bool& flat) {
+  if constexpr (kForm == REPLAY_HYBRID) { hyb_leave(fb, f, hs); hs.n0 = hs.n1 = 0; }
+  else flat_leave(fb, fs);
+  flat = false;
+}
+template <class LT, ReplayKind kForm>
 __device__ __forceinline__ void replay_straight(const AdvParams& p, const EnvConst& ec) {
+  constexpr bool kHyb = kForm == REPLAY_HYBRID;
   extern __shared__ __align__(128) unsigned char smem[];
   const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
   const int env = blockIdx.x * (blockDim.x >> 5) + warp;
@@ -661,10 +573,12 @@ __device__ __forceinline__ void replay_straight(const AdvParams& p, const EnvCon
   FastBook<LT> fb; fb.blob = base; fb.lane = lane;
   BookHdr* h = reinterpret_cast<BookHdr*>(base);
   FastState f; f.err = h->err; f.dead = h->dead; f.bail = 0; f.bail_vol = 0;
-  if (!kPools || !hdr_is_flat(h)) fast_refresh_best(fb, f);
+  if (kForm != REPLAY_FLAT || !hdr_is_flat(h)) fast_refresh_best(fb, f);
+  // flat: the book is in the pool form of kForm (fs: the flat pools; hs: the hybrid book's pools near the touch)
   FlatState fs; fs.n0 = fs.n1 = 0; fs.seq = 0;
+  HybState hs; hs.n0 = hs.n1 = 0; hs.floor0 = INT32_MIN; hs.floor1 = INT32_MAX; hs.seq = 0;
   bool flat = false;
-  if (kPools && hdr_is_flat(h)) { flat_adopt<LT>(base, lane, f, fs); flat = true; }   // the blob was stored in the flat form
+  if (kForm == REPLAY_FLAT && hdr_is_flat(h)) { flat_adopt<LT>(base, lane, f, fs); flat = true; }   // the blob was stored in the flat form
   const lobsim_stream_t* stp = &p.streams[h->stream_id];
   MsgTiles mt(stp);
   const uint32_t* __restrict__ st_step_off = stp->step_off;
@@ -673,18 +587,20 @@ __device__ __forceinline__ void replay_straight(const AdvParams& p, const EnvCon
   const int n_grid = (int)stp->n_grid_steps;
   unsigned g, g_end_all;
   stream_window(st_step_off, n_grid, now_step, T, f.err, f.dead, g, g_end_all);
-  if (kPools && !flat && g < g_end_all && flat_fits(fb, 0)) { flat_enter(fb, fs); flat = true; }
+  if (kForm != REPLAY_SORTED && !flat && g < g_end_all) pool_enter<LT, kForm>(fb, f, fs, hs, flat, 0);
   mt.start(msgbuf, bars, lane, g, g_end_all);
   const int steps_per_sec = ec.steps_per_sec;
   int sub = now_step >= 0 ? now_step % steps_per_sec : 0;
 
   // One pass per second, or per part of a second where the launch (T) or the stream begins or ends inside one: a replay book holds
   // no agent orders, so nothing happens at a step boundary that is not a second boundary, and the message segments run across
-  // steps.  now_step advances by the steps a pass covered; where a book dies, it is recovered from the step offsets of that pass.
+  // steps.  The hybrid book walks one grid step per pass instead: its pools are topped up at every step boundary.  now_step
+  // advances by the steps a pass covered; where a book dies, it is recovered from the step offsets of that pass.
 #pragma unroll 1
   for (int t = 0; t < T && !f.dead;) {
-    const int k = min(min(steps_per_sec - sub, T - t), n_grid - now_step);   // steps of this pass
-    if (k <= 0) { f.err |= LOBSIM_ERR_END_OF_STREAM; f.dead = 1; break; }
+    const int left = n_grid - now_step;                      // grid steps left in the stream
+    const int k = kHyb ? 1 : min(min(steps_per_sec - sub, T - t), left);   // steps of this pass
+    if (min(k, left) <= 0) { f.err |= LOBSIM_ERR_END_OF_STREAM; f.dead = 1; break; }   // (k <= left in the other forms)
     const unsigned g_pass_end = __ldg(&st_step_off[now_step + k]);
 #pragma unroll 1
     while (g < g_pass_end) {
@@ -695,7 +611,8 @@ __device__ __forceinline__ void replay_straight(const AdvParams& p, const EnvCon
       const uint4* mp = reinterpret_cast<const uint4*>(msgbuf + (tile & 1) * MSG_TILE_BYTES) + (g % MSG_TILE);
       const unsigned cnt = lim - g;
       unsigned i = 0;
-      if constexpr (kPools) {
+      int redo_vol = 0;                                      // (hybrid) the unfinished part of message i, for the sorted book
+      if constexpr (kForm == REPLAY_FLAT) {
         if (flat) {
           // the volumes of the whole segment (<= 32 messages, one per lane) are checked at once; the per-message test is one predicate
           const bool bad_vol = __any_sync(FULL_MASK, (unsigned)lane < cnt && (int)mp[(unsigned)lane < cnt ? lane : 0].y <= 0);
@@ -715,12 +632,33 @@ __device__ __forceinline__ void replay_straight(const AdvParams& p, const EnvCon
           f.bail = 0;                                        // (not read: `stopped` without f.dead is the full pool)
           if (stopped && !f.dead) { flat_leave(fb, fs); flat = false; }
         }
+      } else if constexpr (kHyb) {
+        // the volumes of the whole segment at once: a segment with a bad one (never in valid data) runs on the sorted book, whose
+        // routines test every order (assert order.volume > 0, Exchange.py:59-60)
+        if (flat && __any_sync(FULL_MASK, (unsigned)lane < cnt && (int)mp[(unsigned)lane < cnt ? lane : 0].y <= 0))
+          pool_leave<LT, kForm>(fb, f, fs, hs, flat);
+        if (flat) {
+#pragma unroll 1
+          for (; i < cnt; i++) {
+            const uint4 m = mp[i];
+            if (hyb_message<LT>(fb, f, hs, (int)m.x, (int)m.y, m.z, m.w)) break;
+          }
+          if (f.bail) {                                      // this book cannot stay hybrid: back to the sorted form
+            const int why = f.bail, rest = f.bail_vol;
+            f.bail = 0; f.bail_vol = 0;
+            pool_leave<LT, kForm>(fb, f, fs, hs, flat);
+            if (why == FLAT_BAIL_FULL) redo_vol = rest;      // the unfinished part of message i runs on the sorted book
+            else i++;
+          }
+        }
       }
       if (!flat && !f.dead) {
 #pragma unroll 1
         for (; i < cnt; i++) {
           const uint4 m = mp[i];
-          fast_message(fb, f, (int)m.x, (int)m.y, m.z, m.w);
+          int v = (int)m.y;
+          if constexpr (kHyb) { if (redo_vol) v = redo_vol; redo_vol = 0; }
+          fast_message(fb, f, (int)m.x, v, m.z, m.w);
           if (f.dead) break;
         }
       }
@@ -733,52 +671,59 @@ __device__ __forceinline__ void replay_straight(const AdvParams& p, const EnvCon
       break;
     }
     now_step += k; t += k; sub += k;
+    if constexpr (kHyb) { if (flat) hyb_top_up(fb, f, hs); }
     if (sub == steps_per_sec) {                              // whole second: outer-level resync, OrderbookSimulator.py:86-87
       sub = 0;
       if (c.resync && (!p.resync_last_only || t == T)) {
         if (const int32_t* row = resync_row(ec, h, stp, f.best0, f.best1, now_step, steps_per_sec)) {
-          if (flat && !flat_resync_needed(h, row, c.n_levels, lane)) flat_update_trackers<LT>(base, lane, fs);
-          else {
-            if (flat) { flat_leave(fb, fs); flat = false; }
+          if (flat && !flat_resync_needed(h, row, c.n_levels, lane)) {
+            if constexpr (kHyb) hyb_update_trackers(fb, hs);
+            else flat_update_trackers<LT>(base, lane, fs);
+          } else {
+            if (flat) pool_leave<LT, kForm>(fb, f, fs, hs, flat);
             fast_resync(fb, f, row, c.n_levels);
           }
         }
       }
-      if constexpr (kPools) {
-        if (flat && fs.seq > 0xE0000000u) { flat_leave(fb, fs); flat = false; }   // renumber the time-priority stamps long before they wrap
-        if (!flat && flat_fits(fb, 8)) { flat_enter(fb, fs); flat = true; }   // back to the flat pools once the book has shrunk
+      if constexpr (kForm != REPLAY_SORTED) {
+        // (flat pools) renumber the time-priority stamps long before they wrap
+        if (kForm == REPLAY_FLAT && flat && fs.seq > 0xE0000000u) pool_leave<LT, kForm>(fb, f, fs, hs, flat);
+        if (!flat) pool_enter<LT, kForm>(fb, f, fs, hs, flat, 8);   // back to the pool form once the book has shrunk
       }
     }
   }
-  if (flat && !p.allow_flat) { flat_leave(fb, fs); flat = false; }   // the caller wants the canonical sorted layout in HBM
+  // the hybrid form never goes to HBM; the flat form only where the caller allows it
+  if (flat && (kHyb || !p.allow_flat)) pool_leave<LT, kForm>(fb, f, fs, hs, flat);
   mt.drain();
   replay_blob_store<LT>(gblob, base, lane, now_step, f, [&]() { if (flat) flat_mark(h, fs); });
 }
 
-#ifndef LOBSIM_REPLAY_FLAT_MIN_BLOCKS
-#define LOBSIM_REPLAY_FLAT_MIN_BLOCKS 7      // 72 registers: 28 resident warps per SM with the 64/256/32 blob (8 = 64 registers: A/B in profiles/)
-#endif
+// 72 registers: 28 resident warps per SM with the 64/256/32 blob (8 blocks = 64 registers: A/B in profiles/)
 template <class LT>
-__global__ void __launch_bounds__(128, LOBSIM_REPLAY_FLAT_MIN_BLOCKS) k_replay_flat(const __grid_constant__ AdvParams p, const __grid_constant__ EnvConst ec) {
-  replay_straight<LT, true>(p, ec);
+__global__ void __launch_bounds__(128, 7) k_replay_flat(const __grid_constant__ AdvParams p, const __grid_constant__ EnvConst ec) {
+  replay_straight<LT, REPLAY_FLAT>(p, ec);
 }
 template <class LT>
 __global__ void __launch_bounds__(128, 7) k_replay_fast(const __grid_constant__ AdvParams p, const __grid_constant__ EnvConst ec) {
-  replay_straight<LT, false>(p, ec);
+  replay_straight<LT, REPLAY_SORTED>(p, ec);
+}
+template <class LT>
+__global__ void __launch_bounds__(128, 3) k_replay_hyb(const __grid_constant__ AdvParams p, const __grid_constant__ EnvConst ec) {
+  replay_straight<LT, REPLAY_HYBRID>(p, ec);
 }
 
 // ====================================================================================================================
-//  the env fast kernel: k_advance<true,true> with the straight-line tracked order path (book_fast.cuh fast_order<LT,true>)
+//  the env fast kernel: k_advance<true> with the straight-line tracked order path (book_fast.cuh fast_order<LT,true>)
 //  and all per-env scalars (counters, portfolio, per-step flow) in the shared-memory header instead of registers.
 // ====================================================================================================================
 static __device__ __noinline__ uint32_t reset_book_cold(unsigned char* blob, const Layout* L, int lane, const lobsim_cfg_t* c, const lobsim_stream_t* st, int stream_id, int start_step) {
   Book b; b.blob = blob; b.L = *L; b.lane = lane;
   WarpState w;
   __syncwarp();
-  load_state<true>(b, w);
+  load_state(b, w);
   w.fill_log = nullptr; w.fill_cap = 0; w.n_fills = 0;
   init_book_from_snapshot(b, w, *c, *st, stream_id, start_step);
-  store_state<true>(b, w);
+  store_state(b, w);
   return pack_errdead(w.err, w.dead);
 }
 

@@ -82,7 +82,7 @@ __global__ void __launch_bounds__(32) k_process_orders(const __grid_constant__ O
       for (int i = lane; i < p.L.blob_bytes / 16; i += 32) dst[i] = src[i];
     }
     __syncwarp();
-    load_state<true>(b, w);
+    load_state(b, w);
     inventory_in = w.inventory; cash_in = w.cash;
     w.fill_log = p.fills ? p.fills + total_fills : nullptr;
     w.fill_cap = p.max_fills - total_fills; w.n_fills = 0;
@@ -90,7 +90,7 @@ __global__ void __launch_bounds__(32) k_process_orders(const __grid_constant__ O
   auto store_env = [&](int env) {
     // Exchange.process_order only returns the fills: the portfolio belongs to the env and moves in its step (HOE.py:280-289)
     w.inventory = inventory_in; w.cash = cash_in;
-    store_state<true>(b, w);
+    store_state(b, w);
     if (!p.blob_in_global) {
       uint4* dst = reinterpret_cast<uint4*>(p.blobs + (size_t)env * p.L.blob_bytes);
       const uint4* src = reinterpret_cast<const uint4*>(smem);
@@ -109,8 +109,8 @@ __global__ void __launch_bounds__(32) k_process_orders(const __grid_constant__ O
     if (!w.dead) {
       if (has_vol && o.volume <= 0) w.err |= LOBSIM_ERR_BAD_VOLUME;
       else if (o.type == LOBSIM_MSG_LIMIT || o.type == LOBSIM_MSG_MARKET)
-        id = submit_or_execute<true>(b, w, o.direction, o.price, o.volume, is_agent ? 0u : o.ref, o.type == LOBSIM_MSG_LIMIT, is_agent);
-      else remove_order<true>(b, w, o.direction, o.price, o.volume, has_vol, is_agent ? (LOBSIM_REF_AGENT | (o.ref & 0x7fffffffu)) : o.ref, is_agent);
+        id = submit_or_execute(b, w, o.direction, o.price, o.volume, is_agent ? 0u : o.ref, o.type == LOBSIM_MSG_LIMIT, is_agent);
+      else remove_order(b, w, o.direction, o.price, o.volume, has_vol, is_agent ? (LOBSIM_REF_AGENT | (o.ref & 0x7fffffffu)) : o.ref, is_agent);
     }
     if (p.refs_out && lane == 0) p.refs_out[k] = id;
   }
@@ -326,8 +326,8 @@ int lobsim_create(const lobsim_cfg_t* cfg, int device, lobsim_t** out) {
   h->warps_per_cta = best_wpc(4, 1.0, h->warp_smem);
   h->replay_warps_per_cta = best_wpc(4, 1.0, h->replay_warp_smem);
   h->env_warps_per_cta = best_wpc(LOBSIM_ENVFAST_WARPS, 0.95, h->warp_smem);   // (deep 128/1024/64 books: 5 warps x 2 CTAs = 10 resident, +11 % over 8 x 1)
-  CUDA_TRY((cudaFuncSetAttribute(k_advance<true, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, h->warps_per_cta * h->warp_smem)));
-  CUDA_TRY((cudaFuncSetAttribute(k_advance<false, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, h->warps_per_cta * h->warp_smem)));
+  CUDA_TRY((cudaFuncSetAttribute(k_advance<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, h->warps_per_cta * h->warp_smem)));
+  CUDA_TRY((cudaFuncSetAttribute(k_advance<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, h->warps_per_cta * h->warp_smem)));
   h->fast = h->force_general ? nullptr : find_fast_layout(h->L);
   if (h->fast) {
     // LOBSIM_REPLAY_FLAT=0: sorted level arrays only.  Otherwise the hybrid book on a deep layout (NL >= 64, NO >= 512) when
@@ -347,8 +347,8 @@ int lobsim_create(const lobsim_cfg_t* cfg, int device, lobsim_t** out) {
               h->L.NL, h->L.NO, h->L.NA);
     }
   }
-  CUDA_TRY((cudaFuncSetAttribute(k_advance<true, true>, cudaFuncAttributePreferredSharedMemoryCarveout, cudaSharedmemCarveoutMaxShared)));
-  CUDA_TRY((cudaFuncSetAttribute(k_advance<false, true>, cudaFuncAttributePreferredSharedMemoryCarveout, cudaSharedmemCarveoutMaxShared)));
+  CUDA_TRY((cudaFuncSetAttribute(k_advance<true>, cudaFuncAttributePreferredSharedMemoryCarveout, cudaSharedmemCarveoutMaxShared)));
+  CUDA_TRY((cudaFuncSetAttribute(k_advance<false>, cudaFuncAttributePreferredSharedMemoryCarveout, cudaSharedmemCarveoutMaxShared)));
   if (!h->blob_in_global) CUDA_TRY(cudaFuncSetAttribute(k_process_orders, cudaFuncAttributeMaxDynamicSharedMemorySize, h->L.blob_bytes));
   // feature rings
   memset(&h->ec, 0, sizeof h->ec);
@@ -477,7 +477,7 @@ static int ensure_sorted(lobsim* h, cudaStream_t stream) {
 
 } // extern "C"
 
-template <bool kEnv, bool kTrack>
+template <bool kEnv>
 static int launch_advance(lobsim* h, const AdvParams& p, cudaStream_t stream) {
   { int rc = ensure_sorted(h, stream); if (rc) return rc; }
   if (h->streams.empty()) return fail(LOBSIM_E_STATE, "no stream loaded");
@@ -485,7 +485,7 @@ static int launch_advance(lobsim* h, const AdvParams& p, cudaStream_t stream) {
   int wpc = h->warps_per_cta;
   int grid = (p.n_sel + wpc - 1) / wpc;
   if (grid <= 0) return LOBSIM_OK;
-  k_advance<kEnv, kTrack><<<grid, wpc * 32, (size_t)wpc * h->warp_smem, stream>>>(p, h->ec);
+  k_advance<kEnv><<<grid, wpc * 32, (size_t)wpc * h->warp_smem, stream>>>(p, h->ec);
   CUDA_TRY(cudaGetLastError());
   h->launches++;
   return LOBSIM_OK;
@@ -510,7 +510,7 @@ static int launch_replay_fast(lobsim* h, const AdvParams& p, cudaStream_t stream
 // the general runtime-layout kernel otherwise
 static int launch_env(lobsim* h, const AdvParams& p, cudaStream_t stream) {
   if (h->streams.empty()) return fail(LOBSIM_E_STATE, "no stream loaded");
-  if (!h->fast) return launch_advance<true, true>(h, p, stream);
+  if (!h->fast) return launch_advance<true>(h, p, stream);
   CUDA_TRY(cudaSetDevice(h->device));
   const int wpc = h->env_warps_per_cta;
   const size_t dyn = (size_t)wpc * h->warp_smem;
@@ -540,7 +540,7 @@ int lobsim_reset_book(lobsim_t* h, const int32_t* env_ids, int32_t n, const int3
   p.env_ids = env_ids; p.n_sel = env_ids ? n : h->cfg.n_envs;
   p.T = 0; p.reset_mode = 1; p.reset_stream_ids = stream_ids; p.reset_steps = start_steps; p.agent_kind = LOBSIM_AGENT_NONE;
   if (!env_ids) h->agent_orders_possible = false; // every book is a fresh snapshot again
-  return launch_advance<false, true>(h, p, (cudaStream_t)stream);
+  return launch_advance<false>(h, p, (cudaStream_t)stream);
 }
 
 int lobsim_reset(lobsim_t* h, const int32_t* env_ids, int32_t n, const int32_t* stream_ids, const int32_t* episode_start_steps, double* obs_out, void* stream) {
@@ -631,14 +631,14 @@ int lobsim_replay(lobsim_t* h, int32_t n_steps, void* stream) {
   p.T = n_steps; p.agent_kind = LOBSIM_AGENT_NONE;
   // fast path: no fill log requested and no agent order can be resting in any book
   if (!h->fill_log && !h->agent_orders_possible && h->fast) return launch_replay_fast(h, p, (cudaStream_t)stream);
-  return launch_advance<false, true>(h, p, (cudaStream_t)stream);
+  return launch_advance<false>(h, p, (cudaStream_t)stream);
 }
 
 int lobsim_forward_step(lobsim_t* h, int32_t n_steps, void* stream) {
   if (!h || n_steps < 0) return fail(LOBSIM_E_INVALID, "bad argument");
   AdvParams p; base_params(h, p);
   p.T = n_steps; p.agent_kind = LOBSIM_AGENT_NONE; p.resync_last_only = 1;
-  return launch_advance<false, true>(h, p, (cudaStream_t)stream);
+  return launch_advance<false>(h, p, (cudaStream_t)stream);
 }
 
 int lobsim_set_book(lobsim_t* h, int32_t env, const lobsim_book_entry_t* buy, int32_t n_buy, const lobsim_book_entry_t* sell, int32_t n_sell) {
