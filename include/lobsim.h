@@ -347,6 +347,20 @@ int lobsim_dump_book(lobsim_t* h, int32_t env, int32_t side, lobsim_book_entry_t
 /* the agent's internal book side (Exchange.internal_orderbook), ascending internal id */
 int lobsim_dump_agent_orders(lobsim_t* h, int32_t env, int32_t side, lobsim_book_entry_t* out_host, int32_t capacity);
 
+/* L2 depth of every env's central book on the device, in one launch: the L2 projection of lobsim_dump_book
+ * (rl4mm/extras/orderbook_comparison.py:6-19) for all envs and both sides at once.  Outputs are [n_envs][2][depth],
+ * side 0 = buy, level 0 = the best level (highest buy / lowest sell price), the layout of the stream snapshots:
+ *   price_dev        int32  level price, LOBSIM_NO_PRICE for an absent level
+ *   volume_dev       int64  sum of the resting volumes at that price (agent orders and snapshot aggregates included), 0 if absent
+ *   orders_dev       int32  number of resting orders at that price (queue length); may be NULL
+ *   agent_volume_dev int64  the part of volume that belongs to the agent's own orders (ref & LOBSIM_REF_AGENT), i.e.
+ *                           _get_volumes_at_prices (HOE.py:324) at the central levels; may be NULL
+ * 1 <= depth <= max_levels_per_side.  Stream-ordered on `stream`.  The call reads every book in the form it is in and changes
+ * no state: no book form conversion, no host synchronisation, no allocation, exactly one kernel launch -- it may run between
+ * any two launches and inside a captured CUDA graph.                                                             */
+int lobsim_get_depth_dev(lobsim_t* h, int32_t depth, int32_t* price_dev, int64_t* volume_dev, int32_t* orders_dev,
+                         int64_t* agent_volume_dev, void* stream);
+
 int lobsim_get_state(lobsim_t* h, int32_t first_env, int32_t n, lobsim_env_state_t* out_host);
 int lobsim_get_state_dev(lobsim_t* h, lobsim_env_state_t* out_dev, void* stream);
 /* fills recorded by the last step / rollout / replay / process_orders call of env `env` */

@@ -159,6 +159,142 @@ __global__ void k_get_state(const unsigned char* blobs, Layout L, int first, int
   out[i] = s;
 }
 
+// ====================================================================================================================
+//  per-env L2 depth (one warp per env, reads the blob in HBM in whichever form it is in: no conversion, no state change)
+// ====================================================================================================================
+struct DepthOut {   // [n_envs][2][depth] each; orders and agent_volume may be null
+  int32_t* price; int64_t* volume; int32_t* orders; int64_t* agent_volume;
+};
+
+// exact warp sum of per-lane partial sums below 2^34 (at most 4 volumes below 2^32 each): two 32-bit warp reductions
+__device__ __forceinline__ long long warp_sum_u34(unsigned long long s) {
+  const unsigned lo = __reduce_add_sync(FULL_MASK, (unsigned)(s & 0xffffu));
+  const unsigned hi = __reduce_add_sync(FULL_MASK, (unsigned)(s >> 16));
+  return ((long long)hi << 16) + lo;
+}
+
+// Level k of a side (best first) is produced by lane k % 32 and written by the whole warp every 32 levels, so that the stores
+// are coalesced.  Levels [found, depth) are absent: LOBSIM_NO_PRICE and zeros.
+__global__ void __launch_bounds__(128) k_book_depth(const unsigned char* blobs, Layout L, int n_envs, int depth, DepthOut out) {
+  const int lane = threadIdx.x & 31;
+  const int env = blockIdx.x * (blockDim.x >> 5) + (threadIdx.x >> 5);
+  if (env >= n_envs) return;
+  const unsigned char* blob = blobs + (size_t)env * L.blob_bytes;
+  const BookHdr* h = reinterpret_cast<const BookHdr*>(blob);
+  const bool flat = h->cnt[0][0] < 0;
+  const bool want_agent = out.agent_volume != nullptr;
+  for (int side = 0; side < 2; side++) {
+    const size_t base = ((size_t)env * 2 + side) * depth;
+    const unsigned char* sb = blob + L.side_off + side * L.side_stride;
+    int lp = LOBSIM_NO_PRICE, lc = 0;    // this lane's level of the current group of 32
+    long long lv = 0, la = 0;
+    auto flush = [&](int k0, int m) {
+      if (lane < m) {
+        const size_t o = base + k0 + lane;
+        out.price[o] = lp; out.volume[o] = lv;
+        if (out.orders) out.orders[o] = lc;
+        if (want_agent) out.agent_volume[o] = la;
+      }
+    };
+    int found = 0;
+    if (flat) {
+      // flat form (book_flat.cuh): an unordered pool of n <= 128 orders {price, ref, volume, seq}, at most 4 per lane in
+      // registers; level k = the best price strictly worse than level k - 1
+      const uint4* pool = reinterpret_cast<const uint4*>(sb + L.ord_off);
+      const int n = h->cnt[side][1];
+      int pr[4]; unsigned vol[4]; unsigned valid = 0, agent = 0;
+#pragma unroll
+      for (int c = 0; c < 4; c++) {
+        pr[c] = 0; vol[c] = 0;
+        if (c * 32 + lane < n) {
+          const uint4 e = pool[c * 32 + lane];
+          pr[c] = (int)e.x; vol[c] = e.z;
+          valid |= 1u << c;
+          if (e.y & LOBSIM_REF_AGENT) agent |= 1u << c;
+        }
+      }
+      int prev = 0;
+      for (; found < depth; found++) {
+        int best = side ? INT32_MAX : INT32_MIN;
+        bool any = false;
+#pragma unroll
+        for (int c = 0; c < 4; c++) {
+          const bool cand = ((valid >> c) & 1) && (found == 0 || (side ? pr[c] > prev : pr[c] < prev));
+          if (cand) { best = side ? min(best, pr[c]) : max(best, pr[c]); any = true; }
+        }
+        if (!__any_sync(FULL_MASK, any)) break;
+        best = side ? __reduce_min_sync(FULL_MASK, best) : __reduce_max_sync(FULL_MASK, best);
+        unsigned long long sv = 0, sa = 0;
+        unsigned cnt = 0;
+#pragma unroll
+        for (int c = 0; c < 4; c++) {
+          if (((valid >> c) & 1) && pr[c] == best) {
+            sv += vol[c]; cnt++;
+            if ((agent >> c) & 1) sa += vol[c];
+          }
+        }
+        const long long v = warp_sum_u34(sv);
+        const int nord = (int)__reduce_add_sync(FULL_MASK, cnt);
+        const long long a = want_agent ? warp_sum_u34(sa) : 0;
+        if (lane == (found & 31)) { lp = best; lv = v; lc = nord; la = a; }
+        if ((found & 31) == 31) flush(found & ~31, 32);
+        prev = best;
+      }
+      if (found & 31) flush(found & ~31, found & 31);
+    } else {
+      // sorted form (book.cuh): levels worst -> best, the best `depth` levels are the contiguous order range ending at
+      // lvend[nlv - 1]; per group of 32 levels, the orders of the group are read coalesced, 32 at a time, and each order is
+      // summed into the level that holds it
+      const int32_t* lvp = reinterpret_cast<const int32_t*>(sb);
+      const uint16_t* lvend = reinterpret_cast<const uint16_t*>(sb + L.lvend_off);
+      const uint2* ord = reinterpret_cast<const uint2*>(sb + L.ord_off);
+      const int nlv = h->cnt[side][0];
+      found = min(depth, nlv);
+      for (int k0 = 0; k0 < found; k0 += 32) {
+        const int m = min(32, found - k0);
+        int lo = 0, hi = 0;
+        lp = LOBSIM_NO_PRICE; lv = 0; la = 0;
+        if (lane < m) {
+          const int j = nlv - 1 - k0 - lane;
+          lp = lvp[j]; hi = lvend[j]; lo = j ? lvend[j - 1] : 0;
+        }
+        lc = hi - lo;
+        const int first = __shfl_sync(FULL_MASK, lo, m - 1), last = __shfl_sync(FULL_MASK, hi, 0);
+        for (int i0 = first; i0 < last; i0 += 32) {
+          const int i = i0 + lane;
+          const bool in = i < last;
+          const uint2 o = in ? ord[i] : make_uint2(0u, 0u);
+          // the level of the group that holds order i: the number of levels whose segment starts above i (segment starts
+          // fall with the lane, and i >= the start of level m - 1)
+          int own = 0;
+#pragma unroll
+          for (int s = 16; s; s >>= 1) {
+            const int t = own + s - 1;
+            const int lo_t = __shfl_sync(FULL_MASK, lo, t);
+            if (t < m && lo_t > i) own += s;
+          }
+          unsigned todo = __ballot_sync(FULL_MASK, in);
+          while (todo) {
+            const int lvl = __shfl_sync(FULL_MASK, own, __ffs(todo) - 1);
+            const bool mine = in && own == lvl;
+            const long long v = warp_sum_u34(mine ? o.x : 0u);
+            const long long a = want_agent ? warp_sum_u34(mine && (o.y & LOBSIM_REF_AGENT) ? o.x : 0u) : 0;
+            if (lane == lvl) { lv += v; la += a; }
+            todo &= ~__ballot_sync(FULL_MASK, mine);
+          }
+        }
+        flush(k0, m);
+      }
+    }
+    for (int k = found + lane; k < depth; k += 32) {
+      const size_t o = base + k;
+      out.price[o] = LOBSIM_NO_PRICE; out.volume[o] = 0;
+      if (out.orders) out.orders[o] = 0;
+      if (want_agent) out.agent_volume[o] = 0;
+    }
+  }
+}
+
 __global__ void k_init_blobs(unsigned char* blobs, Layout L, int n, long long inventory, double cash) {
   int i = blockIdx.x * blockDim.x + threadIdx.x;
   if (i >= n) return;
@@ -704,6 +840,19 @@ int lobsim_get_state_dev(lobsim_t* h, lobsim_env_state_t* out_dev, void* stream)
   if (!h || !out_dev) return fail(LOBSIM_E_INVALID, "null argument");
   CUDA_TRY(cudaSetDevice(h->device));
   k_get_state<<<(h->cfg.n_envs + 127) / 128, 128, 0, (cudaStream_t)stream>>>(h->blobs, h->L, 0, h->cfg.n_envs, out_dev);
+  CUDA_TRY(cudaGetLastError());
+  h->launches++;
+  return LOBSIM_OK;
+}
+
+int lobsim_get_depth_dev(lobsim_t* h, int32_t depth, int32_t* price_dev, int64_t* volume_dev, int32_t* orders_dev,
+                         int64_t* agent_volume_dev, void* stream) {
+  if (!h || !price_dev || !volume_dev) return fail(LOBSIM_E_INVALID, "null argument");
+  if (depth < 1 || depth > h->cfg.max_levels_per_side) return fail(LOBSIM_E_INVALID, "depth must be in [1, max_levels_per_side]");
+  CUDA_TRY(cudaSetDevice(h->device));
+  // reads flat and sorted blobs as they are (no ensure_sorted): one launch, no synchronisation, no allocation
+  const DepthOut out = {price_dev, volume_dev, orders_dev, agent_volume_dev};
+  k_book_depth<<<(h->cfg.n_envs + 3) / 4, 128, 0, (cudaStream_t)stream>>>(h->blobs, h->L, h->cfg.n_envs, depth, out);
   CUDA_TRY(cudaGetLastError());
   h->launches++;
   return LOBSIM_OK;

@@ -195,6 +195,37 @@ class LobSim:
         lib().lobsim_dump_agent_orders(self._h, env, side, np_ptr(out), n)
         return out
 
+    def book_depth(self, depth: int, orders: bool = False, agent: bool = False, out=None, stream=None):
+        """L2 depth of every env's central book, read on the device in one launch (lobsim_get_depth_dev): the L2
+        projection of ``dump_book`` (rl4mm/extras/orderbook_comparison.py:6-19) for all envs at once.
+
+        Returns torch CUDA tensors ``price`` int32 [N, 2, depth] (side 0 = buy, level 0 = best; absent levels
+        ``abi.NO_PRICE``) and ``volume`` int64 [N, 2, depth] (agent orders and snapshot aggregates included), then
+        ``orders`` int32 [N, 2, depth] (resting orders per level) if ``orders``, then ``agent_volume`` int64 [N, 2, depth]
+        (the agent's own part of ``volume``, HOE.py:324) if ``agent``.  ``out``: a tuple of preallocated tensors in that
+        order, filled and returned instead (for CUDA graph capture).  No host synchronisation; the books are read in
+        whatever form they are in and left unchanged."""
+        depth = int(depth)
+        if not 1 <= depth <= self.cfg.max_levels_per_side:
+            raise LobsimError(f"depth must be in [1, max_levels_per_side = {self.cfg.max_levels_per_side}], got {depth}")
+        want = [torch.int32, torch.int64] + ([torch.int32] if orders else []) + ([torch.int64] if agent else [])
+        shape = (self.n_envs, 2, depth)
+        if out is None:
+            out = tuple(torch.empty(shape, dtype=dt, device=self.device) for dt in want)
+        else:
+            out = tuple(out)
+            if len(out) != len(want):
+                raise ValueError(f"out: expected {len(want)} tensors (price, volume[, orders][, agent_volume])")
+            for t, dt in zip(out, want):
+                if t.dtype != dt or tuple(t.shape) != shape or t.device != self.device or not t.is_contiguous():
+                    raise ValueError(f"out: expected contiguous {dt} tensors of shape {shape} on {self.device}")
+        price, volume = out[0], out[1]
+        n_orders = out[2] if orders else None
+        agent_volume = out[-1] if agent else None
+        check(lib().lobsim_get_depth_dev(self._h, depth, _dptr(price), _dptr(volume), _dptr(n_orders), _dptr(agent_volume),
+                                         self._stream_arg(stream)))
+        return out
+
     def state(self, first: int = 0, n: Optional[int] = None) -> np.ndarray:
         n = self.n_envs - first if n is None else n
         out = np.zeros(n, abi.ENV_STATE_DTYPE)

@@ -344,6 +344,12 @@ class HistoricalOrderbookEnvironment:
         """Hot-loop variant: torch CUDA tensors in and out, no host round trip, no error polling."""
         return self.sim.step(actions)
 
+    def book_depth(self, depth: int, orders: bool = False, agent: bool = False, out=None, stream=None):
+        """Depth observations: the L2 book of every env read on the device in one launch (``LobSim.book_depth``), torch
+        CUDA tensors price int32 / volume int64 [n_envs, 2, depth] (+ orders, agent_volume when asked for).  Batched and
+        not squeezed, also when n_envs == 1; no host round trip, so it may sit next to ``step_torch`` in a CUDA graph."""
+        return self.sim.book_depth(depth, orders=orders, agent=agent, out=out, stream=stream)
+
     def rollout(self, agent, T: int):
         """``generate_trajectory`` (rl4mm/gym/utils.py:100-117) for T steps of every env, fused on the device when the
         agent has a device implementation (FixedActionAgent, Teradactyl); returns torch tensors obs, act, rew, done."""

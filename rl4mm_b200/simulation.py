@@ -187,6 +187,11 @@ class OrderbookSimulator:
         self.now_is = until
         return filled
 
+    def book_depth(self, depth: int, orders: bool = False, agent: bool = False, out=None, stream=None):
+        """L2 depth of EVERY env of the underlying LobSim (``LobSim.book_depth``): torch CUDA tensors [n_envs, 2, depth],
+        batched and not squeezed, also when n_envs == 1 or this simulator is a view of one env (index with ``self.env``)."""
+        return self.sim.book_depth(depth, orders=orders, agent=agent, out=out, stream=stream)
+
     @property
     def min_buy_price(self) -> int:
         return int(self.sim.state(self.env, 1)[0]["min_buy_price"])
