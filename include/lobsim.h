@@ -361,6 +361,29 @@ int lobsim_dump_agent_orders(lobsim_t* h, int32_t env, int32_t side, lobsim_book
 int lobsim_get_depth_dev(lobsim_t* h, int32_t depth, int32_t* price_dev, int64_t* volume_dev, int32_t* orders_dev,
                          int64_t* agent_volume_dev, void* stream);
 
+/* The agent's resting orders of every env on the device, in one launch, with their queue positions in the central book
+ * (Exchange._find_queue_position, Exchange.py:196-217): lobsim_dump_agent_orders for all envs and both sides at once.
+ * count_dev is [n_envs][2], the other outputs are [n_envs][2][max_orders]; side 0 = buy, and the slots of a side hold its
+ * orders in ascending internal id (the order of lobsim_dump_agent_orders):
+ *   count_dev        int32  the side's number of agent orders, also when it exceeds max_orders (then only the first
+ *                           max_orders are written)
+ *   price_dev        int32  order price; LOBSIM_NO_PRICE in an unused slot
+ *   volume_dev       int32  remaining volume; 0 in an unused slot
+ *   id_dev           int32  internal agent id (the order's ref is LOBSIM_REF_AGENT | id); 0 in an unused slot
+ *   level_dev        int32  index of the order's price among the central levels of its side, 0 = the best level (the
+ *                           numbering of lobsim_get_depth_dev); may be NULL
+ *   ahead_orders_dev int32  number of resting orders in front of it in the FIFO at its price (external orders, snapshot
+ *                           aggregates and the agent's own earlier orders alike); may be NULL
+ *   ahead_volume_dev int64  their summed volume; may be NULL
+ * Unused slots have level -1 and nothing ahead.  An order the central book lacks (possible only in a book flagged with a
+ * capacity error) also gets level -1 and nothing ahead.  1 <= max_orders <= max_agent_orders.  Stream-ordered on `stream`.
+ * Like lobsim_get_depth_dev, the call reads every book in the form it is in and changes no state: no book form conversion,
+ * no host synchronisation, no allocation, exactly one kernel launch -- it may run between any two launches and inside a
+ * captured CUDA graph.                                                                                           */
+int lobsim_get_agent_orders_dev(lobsim_t* h, int32_t max_orders, int32_t* count_dev, int32_t* price_dev, int32_t* volume_dev,
+                                int32_t* id_dev, int32_t* level_dev, int32_t* ahead_orders_dev, int64_t* ahead_volume_dev,
+                                void* stream);
+
 int lobsim_get_state(lobsim_t* h, int32_t first_env, int32_t n, lobsim_env_state_t* out_host);
 int lobsim_get_state_dev(lobsim_t* h, lobsim_env_state_t* out_dev, void* stream);
 /* fills recorded by the last step / rollout / replay / process_orders call of env `env` */

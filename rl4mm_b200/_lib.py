@@ -55,6 +55,7 @@ def lib():
         "lobsim_dump_book": (C.c_int, [vp, i32, i32, vp, i32]),
         "lobsim_dump_agent_orders": (C.c_int, [vp, i32, i32, vp, i32]),
         "lobsim_get_depth_dev": (C.c_int, [vp, i32, vp, vp, vp, vp, vp]),
+        "lobsim_get_agent_orders_dev": (C.c_int, [vp, i32, vp, vp, vp, vp, vp, vp, vp, vp]),
         "lobsim_get_state": (C.c_int, [vp, i32, i32, vp]),
         "lobsim_get_state_dev": (C.c_int, [vp, vp, vp]),
         "lobsim_get_fills": (C.c_int, [vp, i32, vp, i32, C.POINTER(i32)]),
@@ -84,7 +85,7 @@ EXPORTED_SYMBOLS = [
     "lobsim_last_error", "lobsim_abi_version", "lobsim_state_bytes", "lobsim_create", "lobsim_destroy",
     "lobsim_load_stream", "lobsim_reset", "lobsim_step", "lobsim_step_host", "lobsim_rollout", "lobsim_rollout_info", "lobsim_rollout_agents", "lobsim_replay",
     "lobsim_replay_host", "lobsim_forward_step", "lobsim_set_book", "lobsim_reset_book", "lobsim_process_orders", "lobsim_dump_book",
-    "lobsim_dump_agent_orders", "lobsim_get_depth_dev", "lobsim_get_state", "lobsim_get_state_dev", "lobsim_get_fills", "lobsim_errors",
+    "lobsim_dump_agent_orders", "lobsim_get_depth_dev", "lobsim_get_agent_orders_dev", "lobsim_get_state", "lobsim_get_state_dev", "lobsim_get_fills", "lobsim_errors",
     "lobsim_obs_dim", "lobsim_action_dim", "lobsim_launch_count", "lobsim_kernel_path", "lobsim_source_hash",
 ]
 

@@ -295,6 +295,116 @@ __global__ void __launch_bounds__(128) k_book_depth(const unsigned char* blobs, 
   }
 }
 
+// ====================================================================================================================
+//  per-env agent orders and their queue positions (one warp per env, reads the blob in HBM as it is: no state change)
+// ====================================================================================================================
+struct AgentOrdersOut {   // count [n_envs][2], the others [n_envs][2][max_orders]; level, ahead_orders, ahead_volume may be null
+  int32_t* count; int32_t* price; int32_t* volume; int32_t* id; int32_t* level; int32_t* ahead_orders; int64_t* ahead_volume;
+};
+
+// Slot k of a side is the k-th entry of the side's agent table (ascending internal id).  The slots are handled 32 at a time,
+// one per lane, and stored coalesced.  Queue position of the group's orders: each lane finds its order's level among the best
+// 32 levels of the side, held one per lane (a 5-step shuffle search; a binary search over the level prices below them); then
+// every distinct level of the group is walked once, 32 FIFO entries per round, carrying the volume of the rounds before, until
+// all of the group's orders at that level are found (the agent's orders are matched by ballot over the round's agent
+// entries).  Per distinct level, that walk is the only dependent load.  An order whose level or FIFO entry is missing (a book flagged with a capacity
+// error) gets level -1 and nothing ahead.  Nine CTAs per SM leave 56 registers, which it needs without spilling (at the 48 of
+// ten, ptxas spills the per-side set-up).
+__global__ void __launch_bounds__(128, 9) k_agent_orders(const unsigned char* blobs, Layout L, int n_envs, int max_orders, AgentOrdersOut out) {
+  const int lane = threadIdx.x & 31;
+  const int env = blockIdx.x * (blockDim.x >> 5) + (threadIdx.x >> 5);
+  if (env >= n_envs) return;
+  const unsigned char* blob = blobs + (size_t)env * L.blob_bytes;
+  const BookHdr* h = reinterpret_cast<const BookHdr*>(blob);
+  // a flat blob holds no agent order (the replay that leaves blobs flat runs only while none can rest): its agent table is
+  // not read, and its nag (0) is the count
+  const bool flat = h->cnt[0][0] < 0;
+  const bool want_queue = out.level || out.ahead_orders || out.ahead_volume;
+  if (lane < 2) out.count[env * 2 + lane] = h->nag[lane];
+  for (int side = 0; side < 2; side++) {
+    const size_t base = ((size_t)env * 2 + side) * max_orders;
+    const int m = flat ? 0 : min(h->nag[side], max_orders);
+    const int32_t* ap = reinterpret_cast<const int32_t*>(blob + L.agent_off + side * L.NA * 12);
+    const int32_t* av = ap + L.NA;
+    const uint32_t* ai = reinterpret_cast<const uint32_t*>(ap + 2 * L.NA);
+    const unsigned char* sb = blob + L.side_off + side * L.side_stride;
+    const int32_t* lvp = reinterpret_cast<const int32_t*>(sb);
+    const uint16_t* lvend = reinterpret_cast<const uint16_t*>(sb + L.lvend_off);
+    const uint2* ord = reinterpret_cast<const uint2*>(sb + L.ord_off);
+    for (int k0 = 0; k0 < max_orders; k0 += 32) {
+      const int k = k0 + lane;
+      const bool in = k < m;
+      const size_t o = base + k;
+      int price = LOBSIM_NO_PRICE;
+      uint32_t id = 0;
+      if (in) { price = ap[k]; id = ai[k]; }
+      if (k < max_orders) { out.price[o] = price; out.volume[o] = in ? av[k] : 0; out.id[o] = (int32_t)id; }
+      if (!want_queue) continue;
+      int lvl = -1, ahead_n = 0;
+      long long ahead_v = 0;
+      if (k0 < m) {
+        // the best 32 levels of the side, lane t = level t (best first): prices and FIFO ends, one coalesced load each
+        const int nlv = h->cnt[side][0], ntop = min(nlv, 32);
+        int tp = 0, tend = 0;
+        if (lane < ntop) { tp = lvp[nlv - 1 - lane]; tend = lvend[nlv - 1 - lane]; }
+        // t: the number of top levels better than the order's price (their keys fall with the lane)
+        const int key = key_of(side, in ? price : 0);
+        int t = 0;
+#pragma unroll
+        for (int s = 16; s; s >>= 1) {
+          const int c = t + s - 1;
+          const int pc = __shfl_sync(FULL_MASK, tp, c);
+          if (c < ntop && key_of(side, pc) > key) t += s;
+        }
+        const int pt = __shfl_sync(FULL_MASK, tp, t);
+        if (t < ntop && key_of(side, pt) > key) t++;        // (t = 31 only: the 32nd level is better too, so all 32 are)
+        const int et = __shfl_sync(FULL_MASK, tend, t & 31), en = __shfl_sync(FULL_MASK, tend, (t + 1) & 31);
+        // j, [seg0, seg1): the index of the order's level in lvp (worst -> best) and its FIFO segment; j = -1 if the side has
+        // no level at its price.  The start of level j is the end of the next worse level: lane t + 1's, or a load past the top.
+        int j = -1, seg0 = 0, seg1 = 0;
+        if (in && t < ntop) {
+          if (pt == price) { j = nlv - 1 - t; seg1 = et; seg0 = j == 0 ? 0 : t < 31 ? en : lvend[j - 1]; }
+        } else if (in && nlv > 32) {   // worse than the 32nd level: binary search over the others (keys ascending)
+          int lo = 0, hi = nlv - 32;
+          while (lo < hi) { const int mid = (lo + hi) >> 1; if (key_of(side, lvp[mid]) < key) lo = mid + 1; else hi = mid; }
+          if (lo < nlv - 32 && lvp[lo] == price) { j = lo; seg0 = j ? lvend[j - 1] : 0; seg1 = lvend[j]; }
+        }
+        unsigned todo = __ballot_sync(FULL_MASK, j >= 0);
+        while (todo) {
+          const int src = __ffs(todo) - 1;
+          const int jl = __shfl_sync(FULL_MASK, j, src);
+          const int first = __shfl_sync(FULL_MASK, seg0, src), last = __shfl_sync(FULL_MASK, seg1, src);
+          unsigned wait = __ballot_sync(FULL_MASK, j == jl);   // the group's orders at level jl not yet found in its FIFO
+          todo &= ~wait;
+          long long before = 0;                                // volume of the FIFO entries of the earlier rounds
+          for (int i0 = first; i0 < last && wait; i0 += 32) {
+            const int i = i0 + lane;
+            const uint2 o = i < last ? ord[i] : make_uint2(0u, 0u);
+            unsigned agents = __ballot_sync(FULL_MASK, (o.y & LOBSIM_REF_AGENT) != 0);
+            while (agents) {
+              const int p = __ffs(agents) - 1;
+              agents &= agents - 1;
+              const uint32_t ref = __shfl_sync(FULL_MASK, o.y, p);
+              const unsigned hit = __ballot_sync(FULL_MASK, ((wait >> lane) & 1) && ref == (LOBSIM_REF_AGENT | id));
+              if (hit) {
+                const long long v = before + warp_sum_u34(lane < p ? o.x : 0u);
+                if ((hit >> lane) & 1) { lvl = nlv - 1 - jl; ahead_n = i0 + p - first; ahead_v = v; }
+                wait &= ~hit;
+              }
+            }
+            before += warp_sum_u34(o.x);
+          }
+        }
+      }
+      if (k < max_orders) {
+        if (out.level) out.level[o] = lvl;
+        if (out.ahead_orders) out.ahead_orders[o] = ahead_n;
+        if (out.ahead_volume) out.ahead_volume[o] = ahead_v;
+      }
+    }
+  }
+}
+
 __global__ void k_init_blobs(unsigned char* blobs, Layout L, int n, long long inventory, double cash) {
   int i = blockIdx.x * blockDim.x + threadIdx.x;
   if (i >= n) return;
@@ -853,6 +963,20 @@ int lobsim_get_depth_dev(lobsim_t* h, int32_t depth, int32_t* price_dev, int64_t
   // reads flat and sorted blobs as they are (no ensure_sorted): one launch, no synchronisation, no allocation
   const DepthOut out = {price_dev, volume_dev, orders_dev, agent_volume_dev};
   k_book_depth<<<(h->cfg.n_envs + 3) / 4, 128, 0, (cudaStream_t)stream>>>(h->blobs, h->L, h->cfg.n_envs, depth, out);
+  CUDA_TRY(cudaGetLastError());
+  h->launches++;
+  return LOBSIM_OK;
+}
+
+int lobsim_get_agent_orders_dev(lobsim_t* h, int32_t max_orders, int32_t* count_dev, int32_t* price_dev, int32_t* volume_dev,
+                                int32_t* id_dev, int32_t* level_dev, int32_t* ahead_orders_dev, int64_t* ahead_volume_dev,
+                                void* stream) {
+  if (!h || !count_dev || !price_dev || !volume_dev || !id_dev) return fail(LOBSIM_E_INVALID, "null argument");
+  if (max_orders < 1 || max_orders > h->cfg.max_agent_orders) return fail(LOBSIM_E_INVALID, "max_orders must be in [1, max_agent_orders]");
+  CUDA_TRY(cudaSetDevice(h->device));
+  // reads flat and sorted blobs as they are (no ensure_sorted): one launch, no synchronisation, no allocation
+  const AgentOrdersOut out = {count_dev, price_dev, volume_dev, id_dev, level_dev, ahead_orders_dev, ahead_volume_dev};
+  k_agent_orders<<<(h->cfg.n_envs + 3) / 4, 128, 0, (cudaStream_t)stream>>>(h->blobs, h->L, h->cfg.n_envs, max_orders, out);
   CUDA_TRY(cudaGetLastError());
   h->launches++;
   return LOBSIM_OK;

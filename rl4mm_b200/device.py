@@ -226,6 +226,40 @@ class LobSim:
                                          self._stream_arg(stream)))
         return out
 
+    def agent_orders(self, max_orders: Optional[int] = None, queue: bool = True, out=None, stream=None):
+        """The agent's resting orders of every env and their queue positions, read on the device in one launch
+        (lobsim_get_agent_orders_dev): ``dump_agent_orders`` for all envs at once, plus where each order stands in the central
+        book (Exchange._find_queue_position, Exchange.py:196-217).
+
+        Returns torch CUDA tensors ``count`` int32 [N, 2] (agent orders per side, also beyond ``max_orders``, which
+        defaults to ``cfg.max_agent_orders``), then ``price``, ``volume`` and ``id`` (the internal agent id) int32
+        [N, 2, max_orders]: side 0 = buy, slots in ascending id, unused slots ``abi.NO_PRICE`` / 0 / 0.  With ``queue``
+        also ``level`` int32 (0 = the best central level of the side, -1 for an unused slot), ``ahead_orders`` int32 and
+        ``ahead_volume`` int64 (the resting orders in front of the order in the FIFO at its price, and their volume).
+        ``out``: a tuple of preallocated tensors in that order, filled and returned instead (for CUDA graph capture).  No
+        host synchronisation; the books are read in whatever form they are in and left unchanged."""
+        A = self.cfg.max_agent_orders if max_orders is None else int(max_orders)
+        if not 1 <= A <= self.cfg.max_agent_orders:
+            raise LobsimError(f"max_orders must be in [1, max_agent_orders = {self.cfg.max_agent_orders}], got {A}")
+        N = self.n_envs
+        want = [((N, 2), torch.int32)] + [((N, 2, A), torch.int32)] * 3
+        if queue:
+            want += [((N, 2, A), torch.int32)] * 2 + [((N, 2, A), torch.int64)]
+        if out is None:
+            out = tuple(torch.empty(shape, dtype=dt, device=self.device) for shape, dt in want)
+        else:
+            out = tuple(out)
+            if len(out) != len(want):
+                raise ValueError(f"out: expected {len(want)} tensors (count, price, volume, id"
+                                 + (", level, ahead_orders, ahead_volume)" if queue else ")"))
+            for t, (shape, dt) in zip(out, want):
+                if t.dtype != dt or tuple(t.shape) != shape or t.device != self.device or not t.is_contiguous():
+                    raise ValueError(f"out: expected a contiguous {dt} tensor of shape {shape} on {self.device}")
+        q = out[4:] if queue else (None, None, None)
+        check(lib().lobsim_get_agent_orders_dev(self._h, A, *(_dptr(t) for t in out[:4]), *(_dptr(t) for t in q),
+                                                self._stream_arg(stream)))
+        return out
+
     def state(self, first: int = 0, n: Optional[int] = None) -> np.ndarray:
         n = self.n_envs - first if n is None else n
         out = np.zeros(n, abi.ENV_STATE_DTYPE)

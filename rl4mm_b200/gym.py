@@ -350,6 +350,13 @@ class HistoricalOrderbookEnvironment:
         not squeezed, also when n_envs == 1; no host round trip, so it may sit next to ``step_torch`` in a CUDA graph."""
         return self.sim.book_depth(depth, orders=orders, agent=agent, out=out, stream=stream)
 
+    def agent_orders(self, max_orders=None, queue: bool = True, out=None, stream=None):
+        """The agent's resting orders of every env and their queue positions, read on the device in one launch
+        (``LobSim.agent_orders``): torch CUDA tensors count [n_envs, 2], price / volume / id [n_envs, 2, max_orders] (+ level,
+        ahead_orders, ahead_volume with ``queue``).  Batched and not squeezed, also when n_envs == 1; no host round trip, so
+        it may sit next to ``step_torch`` in a CUDA graph."""
+        return self.sim.agent_orders(max_orders=max_orders, queue=queue, out=out, stream=stream)
+
     def rollout(self, agent, T: int):
         """``generate_trajectory`` (rl4mm/gym/utils.py:100-117) for T steps of every env, fused on the device when the
         agent has a device implementation (FixedActionAgent, Teradactyl); returns torch tensors obs, act, rew, done."""

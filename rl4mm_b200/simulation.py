@@ -192,6 +192,11 @@ class OrderbookSimulator:
         batched and not squeezed, also when n_envs == 1 or this simulator is a view of one env (index with ``self.env``)."""
         return self.sim.book_depth(depth, orders=orders, agent=agent, out=out, stream=stream)
 
+    def agent_orders(self, max_orders=None, queue: bool = True, out=None, stream=None):
+        """The agent's orders and queue positions in EVERY env of the underlying LobSim (``LobSim.agent_orders``), batched
+        and not squeezed, also when n_envs == 1 or this simulator is a view of one env (index with ``self.env``)."""
+        return self.sim.agent_orders(max_orders=max_orders, queue=queue, out=out, stream=stream)
+
     @property
     def min_buy_price(self) -> int:
         return int(self.sim.state(self.env, 1)[0]["min_buy_price"])
