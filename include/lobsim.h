@@ -87,6 +87,7 @@ typedef struct {
 
 /* ---- features: rl4mm/features/Features.py ------------------------------------------------------------------- */
 #define LOBSIM_MAX_FEATURES 16
+#define LOBSIM_MAX_NORM_LEN 10000000   /* longest rolling z-score history (max_norm_len) */
 enum {
   LOBSIM_FEAT_SPREAD = 0,             /* Features.py:113 */
   LOBSIM_FEAT_BOOK_IMBALANCE = 1,     /* :132 */

@@ -551,6 +551,9 @@ __device__ __forceinline__ void feature_update_raw(const lobsim_feature_t& fc, F
 //   * noise-dominated window (|std| <= 1e-8 |mean|, e.g. [p + 1e-06, p, p, ...] for a price p ~ 4e6): the numpy arithmetic
 //     is replayed over the ring, O(history) like the reference, because there the result IS the rounding error.
 // mode 0: x_i, mode 1: (x_i - mean)^2, mode 2: the constant cval (no memory access)
+// Frames of the explicit post-order stack below: one per level of numpy's split tree (leaf included).  A child holds at most
+// n/2 + 8 entries, so the tree of n <= LOBSIM_MAX_NORM_LEN (10 M) entries is 18 levels deep (tests/test_zscore_cpu.py).
+#define NP_PAIRWISE_STACK 18
 static __device__ __noinline__ double np_pairwise_sum_ring(const double* hist, int maxlen, int start, int n, int mode, double mean, double cval) {
   auto el = [&](int i) -> double {
     if (mode == 2) return cval;
@@ -580,7 +583,7 @@ static __device__ __noinline__ double np_pairwise_sum_ring(const double* hist, i
     return res;
   };
   if (n <= 128) return leaf(0, n);
-  int f_off[16], f_n[16], f_stage[16]; double f_left[16];   // explicit post-order stack: depth <= log2(n / 64) (n < 2^21)
+  int f_off[NP_PAIRWISE_STACK], f_n[NP_PAIRWISE_STACK], f_stage[NP_PAIRWISE_STACK]; double f_left[NP_PAIRWISE_STACK];
   int sp = 1; double ret = 0.0;
   f_off[0] = 0; f_n[0] = n; f_stage[0] = 0; f_left[0] = 0.0;
   while (sp > 0) {
@@ -648,10 +651,13 @@ static __device__ __noinline__ double feature_normalise(NormState* fg, double* h
   f.nS2max = fmax(f.nS2max, f.nS2);
   double m1 = f.nS1 / (double)n, msq = f.nS2 / (double)n;
   double var = msq - m1 * m1;
-  // the running sums carry an absolute error ~ eps * nS2max: recompute them exactly (around the current mean) when that is
-  // not negligible against n * var -- a dominant entry (e.g. the 1e-06 offset of the first one) left the window, or the mean
-  // drifted far from the centre -- when a NaN got in, and once per lap of the ring
-  if (!(var * (double)n > 1e-6 * f.nS2max) || (head == 0 && n == maxlen)) {
+  // the running sums carry an absolute error ~ eps * nS2max per update, and it accumulates: recompute them exactly (around
+  // the current mean) when nS2max exceeds 100 n * var -- a dominant entry (e.g. the 1e-06 offset of the first one) left the
+  // window or dominates it, or the mean drifted far from the centre -- when a NaN got in, and every 512 updates (ring
+  // positions 0, 512, ...: once per lap of a shorter ring).  This keeps the normal-regime z-score within 256 eps * kappa of
+  // the exact one (tests/test_gpu_zscore.py); a bound of 1e6 n * var and one recentre per lap left windows of 1 000 to
+  // 20 000 entries up to 400 eps * kappa off.
+  if (!(var * (double)n > 1e-2 * f.nS2max) || (head & 511) == 0) {
     double centre = f.nK + m1;
     if (!isfinite(centre)) centre = isfinite(value) ? value : 0.0;
     zscore_recenter(f, hist, maxlen, start, n, centre);

@@ -500,7 +500,7 @@ static int validate_cfg(const lobsim_cfg_t* c) {
     if (f.kind == LOBSIM_FEAT_AMIHUD_LAMBDA && (f.iparam < 1 || f.iparam > 16383 || f.lookback % f.iparam || f.lookback / f.iparam < 2 || f.lookback / f.iparam > 65535))
       return fail(LOBSIM_E_INVALID, "AMIHUD_LAMBDA: lookback must be (true_lookback + 1) * slowing_factor with true_lookback >= 1");
     if (f.update_us <= 0 || f.update_us > 60000000 || f.lookback < 0) return fail(LOBSIM_E_INVALID, "bad feature update_us / lookback");
-    if (f.norm_len < 0 || f.norm_len > 10000000) return fail(LOBSIM_E_INVALID, "bad feature norm_len");
+    if (f.norm_len < 0 || f.norm_len > LOBSIM_MAX_NORM_LEN) return fail(LOBSIM_E_INVALID, "bad feature norm_len");
     if (f.kind == LOBSIM_FEAT_TIME_OF_DAY && f.iparam <= 0) return fail(LOBSIM_E_INVALID, "TIME_OF_DAY needs n_buckets > 0");
     if ((f.kind == LOBSIM_FEAT_VOLATILITY || f.kind == LOBSIM_FEAT_TRADE_DIR_IMBALANCE || f.kind == LOBSIM_FEAT_TRADE_VOL_IMBALANCE) && f.lookback < 1)
       return fail(LOBSIM_E_INVALID, "windowed feature needs lookback >= 1");
