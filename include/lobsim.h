@@ -335,6 +335,24 @@ int lobsim_reset_book(lobsim_t* h, const int32_t* env_ids_dev, int32_t n, const 
 int lobsim_process_orders(lobsim_t* h, const lobsim_order_t* orders_host, int32_t n, lobsim_fill_t* fills_out_host,
                           int32_t max_fills, int32_t* n_fills_out, uint32_t* refs_out_host);
 
+/* Exchange.process_order (Exchange.py:58-69) for EVERY env at once, on the device: row i of orders_dev is env i's own list,
+ * applied in order, exactly as lobsim_process_orders would apply the same orders of env i.
+ *   orders_dev   lobsim_order_t [n_envs][max_orders], 16-byte aligned; the `env` field is ignored (the row is the env)
+ *   count_dev    int32 [n_envs]: orders of each row to apply; values outside [0, max_orders] are clamped
+ *   refs_dev     uint32 [n_envs][max_orders], may be NULL: as refs_out_host of lobsim_process_orders (agent id of an agent
+ *                order that rested, 0xffffffff for an external order that rested, 0 otherwise; 0 beyond the row's count)
+ *   fills_dev    lobsim_fill_t [n_envs][max_fills], may be NULL when max_fills == 0: each env's fills in emission order
+ *   n_fills_dev  int32 [n_envs], may be NULL: each env's number of fills, also when it exceeds max_fills (then only the first
+ *                max_fills are written and the env gets LOBSIM_ERR_FILL_LOG_FULL, as with lobsim_process_orders).  With
+ *                max_fills == 0 no fill is logged or counted (n_fills 0), as with lobsim_process_orders.
+ * Like lobsim_process_orders it moves only the books and the agent tables: inventory, cash, price, the per-step flow and the
+ * handle's fill log (lobsim_get_fills) are unchanged.  An env with count 0 is not read or written.  A dead env (sticky
+ * EMPTY_BOOK etc.) ignores its orders.  Orders with a type outside 1..4 or a direction outside 0..1 are skipped (ref 0).
+ * Stream-ordered on `stream`: no host synchronisation, no allocation, exactly one kernel launch -- it may run between any two
+ * launches and inside a captured CUDA graph.  1 <= max_orders, 0 <= max_fills.                                              */
+int lobsim_submit_orders_dev(lobsim_t* h, int32_t max_orders, const lobsim_order_t* orders_dev, const int32_t* count_dev,
+                             uint32_t* refs_dev, int32_t max_fills, lobsim_fill_t* fills_dev, int32_t* n_fills_dev, void* stream);
+
 /* Exchange(central_orderbook=..., internal_orderbook=...) (Exchange.py:40-49) / `exchange.central_orderbook = book`:
  * replaces env's books by the given L3 entries (per side: best level first, FIFO order inside a level, exactly the
  * lobsim_dump_book format; ref = LOBSIM_REF_AGENT | id marks the agent's own orders, which also form the internal

@@ -124,6 +124,43 @@ assert ORDER_DTYPE.itemsize == 32 and FILL_DTYPE.itemsize == 24 and BOOK_ENTRY_D
 assert ENV_STATE_DTYPE.itemsize == 80, ENV_STATE_DTYPE.itemsize
 
 
+def _order_field(x, shape, device):
+    """One field of pack_orders as int32 [N, K]: a tensor (broadcast) or a scalar; values are taken modulo 2^32 (refs >= 2^31)."""
+    import torch
+
+    if isinstance(x, torch.Tensor):
+        if x.dtype.is_floating_point or x.dtype.is_complex:
+            raise TypeError(f"pack_orders: integer tensors only, got {x.dtype}")
+        v = x.to(torch.int64)
+        v = torch.where(v >= 2**31, v - 2**32, v).to(torch.int32)
+        return v.expand(shape)
+    x = int(x)
+    return torch.full(shape, x - 2**32 if x >= 2**31 else x, dtype=torch.int32, device=device)
+
+
+def pack_orders(type, direction, price, volume, is_external=0, ref=0):
+    """The orders of N envs, K per env, as the int32 tensor [N, K, 8] that is a ``lobsim_order_t`` array in ORDER_DTYPE field
+    order (the input of ``LobSim.submit_orders``).  Each argument is an integer tensor of shape [N, K] (or broadcastable to it)
+    or a scalar; the tensors must be on one device, which the result is on, and at least one must be given.  ``env`` is set to
+    the row index, so that the rows concatenated env by env are also a valid ``process_orders`` list; ``reserved`` is 0."""
+    import torch
+
+    fields = (type, direction, price, volume, is_external, ref)
+    tensors = [f for f in fields if isinstance(f, torch.Tensor)]
+    if not tensors:
+        raise ValueError("pack_orders: at least one argument must be an [N, K] tensor")
+    device = tensors[0].device
+    if any(t.device != device for t in tensors):
+        raise ValueError("pack_orders: all tensors must be on one device")
+    shape = torch.broadcast_shapes(*(t.shape for t in tensors))
+    if len(shape) != 2:
+        raise ValueError(f"pack_orders: the fields must broadcast to [N, K], got {tuple(shape)}")
+    n, k = shape
+    env = torch.arange(n, dtype=torch.int32, device=device)[:, None].expand(n, k)
+    cols = [env] + [_order_field(f, shape, device) for f in fields] + [torch.zeros(shape, dtype=torch.int32, device=device)]
+    return torch.stack(cols, dim=-1).contiguous()
+
+
 def default_cfg(**kw) -> Cfg:
     """A Cfg with the reference's defaults (HOE.py:54-81, OrderbookSimulator.py:24-35); override with kwargs."""
     cfg = Cfg()

@@ -1,8 +1,8 @@
 // fast_layout.cu -- ONE compiled StaticLayout of the straight-line kernels (kernels.cuh): the three instantiations of
-// replay_straight (k_replay_flat / k_replay_fast / k_replay_hyb), k_to_sorted and k_env_fast.
+// replay_straight (k_replay_flat / k_replay_fast / k_replay_hyb), k_to_sorted, k_env_fast and k_submit_orders.
 // Compiled once per entry of layouts.h and per part (-DLOBSIM_LAYOUT_INDEX=i -DLOBSIM_TU_PART=p, build.py), in parallel:
 //   part 0: the replay kernels (k_replay_hyb only for the deep layouts of hyb_layout()) + the env kernels without the z-score /
-//           RollingSharpe code
+//           RollingSharpe code + k_submit_orders
 //   part 1: the env kernels with that code (RARE)
 // lobsim.cu calls the launchers below through the FastLayoutOps table.
 #include "kernels.cuh"
@@ -47,7 +47,12 @@ cudaError_t FN(_attrs)(int dyn_replay, int dyn_env) {
   if constexpr (hyb_layout<LT>()) { if (e == cudaSuccess) e = set_attr((const void*)k_replay_hyb<LT>, dyn_replay); }
   if (e == cudaSuccess) e = cudaFuncSetAttribute((const void*)k_to_sorted<LT>, cudaFuncAttributeMaxDynamicSharedMemorySize, 4 * LT::blob_bytes <= 227 * 1024 ? 4 * LT::blob_bytes : LT::blob_bytes);
   if (e == cudaSuccess) e = env_attrs<false>(dyn_env);
+  if (e == cudaSuccess) e = cudaFuncSetAttribute((const void*)k_submit_orders<LT>, cudaFuncAttributeMaxDynamicSharedMemorySize, LOBSIM_SUBMIT_WARPS * submit_warp_bytes<LT>());
   return e;
+}
+void FN(_submit)(const SubmitParams& p, cudaStream_t stream) {
+  const int grid = (p.n_envs + LOBSIM_SUBMIT_WARPS - 1) / LOBSIM_SUBMIT_WARPS;
+  k_submit_orders<LT><<<grid, 32 * LOBSIM_SUBMIT_WARPS, (size_t)LOBSIM_SUBMIT_WARPS * submit_warp_bytes<LT>(), stream>>>(p);
 }
 void FN(_replay)(ReplayKind kind, int grid, int block, size_t dyn, cudaStream_t stream, const AdvParams& p, const EnvConst& ec) {
   if constexpr (hyb_layout<LT>()) {

@@ -1008,3 +1008,167 @@ __global__ void __launch_bounds__(32 * LOBSIM_ENVFAST_WARPS, env_min_blocks<LT>(
   if (lane <= 12) { tma_store_commit(); tma_store_wait(); }
   __syncwarp();
 }
+
+// ====================================================================================================================
+//  lobsim_submit_orders_dev: Exchange.process_order for every env's own row of orders, one warp per env -- k_submit_orders<LT>
+//  (the compiled layouts) and k_submit_orders_general (lobsim.cu: every other handle)
+// ====================================================================================================================
+struct SubmitParams {
+  unsigned char* blobs; Layout L; int32_t n_envs; int32_t blob_in_global;
+  int32_t max_orders;
+  const lobsim_order_t* orders;   // [n_envs][max_orders], 16-byte aligned
+  const int32_t* count;           // [n_envs]
+  uint32_t* refs;                 // [n_envs][max_orders] or null
+  int32_t max_fills;
+  lobsim_fill_t* fills;           // [n_envs][max_fills]; null when max_fills == 0 (then no fill is logged or counted)
+  int32_t* n_fills;               // [n_envs] or null
+};
+
+// the number of orders of env's row: count clamped to [0, max_orders]
+__device__ __forceinline__ int submit_count(const SubmitParams& p, int env) {
+  const int n = p.count[env];
+  return n < 0 ? 0 : n > p.max_orders ? p.max_orders : n;
+}
+
+// The first n orders of env's row, in order, through apply(order) -> its ref (warp-collective, uniform).  The row is read 32
+// orders at a time, one per lane (two 16-byte loads), and each order is broadcast to the warp; the refs of a group are stored
+// by the lanes that read the orders, and the refs beyond n are 0.  Orders with a type outside 1..4 or a direction outside 0..1
+// are skipped (ref 0).
+template <class Apply>
+__device__ __forceinline__ void submit_row(const SubmitParams& p, int env, int n, int lane, Apply apply) {
+  const int4* row = reinterpret_cast<const int4*>(p.orders + (size_t)env * p.max_orders);
+  uint32_t* refs = p.refs ? p.refs + (size_t)env * p.max_orders : nullptr;
+  const int kend = refs ? p.max_orders : n;
+#pragma unroll 1
+  for (int k0 = 0; k0 < kend; k0 += 32) {
+    const int m = min(32, n - k0);
+    int4 a = make_int4(0, 0, 0, 0), c = a;   // {env, type, direction, price}, {volume, is_external, ref, reserved}
+    if (lane < m) { a = row[2 * (k0 + lane)]; c = row[2 * (k0 + lane) + 1]; }
+    uint32_t my_ref = 0;
+#pragma unroll 1
+    for (int i = 0; i < m; i++) {
+      lobsim_order_t o;
+      o.env = env; o.type = __shfl_sync(FULL_MASK, a.y, i); o.direction = __shfl_sync(FULL_MASK, a.z, i);
+      o.price = __shfl_sync(FULL_MASK, a.w, i); o.volume = __shfl_sync(FULL_MASK, c.x, i);
+      o.is_external = __shfl_sync(FULL_MASK, c.y, i); o.ref = (uint32_t)__shfl_sync(FULL_MASK, c.z, i); o.reserved = 0;
+      uint32_t id = 0;
+      if ((unsigned)(o.type - LOBSIM_MSG_LIMIT) <= LOBSIM_MSG_MARKET - LOBSIM_MSG_LIMIT && (unsigned)o.direction <= 1u) id = apply(o);
+      if (lane == i) my_ref = id;
+    }
+    if (refs && k0 + lane < p.max_orders) refs[k0 + lane] = my_ref;
+  }
+}
+
+// Volume None (Exchange.py:140) on the straight-line path, which takes removals with a volume only: a removal of at least the
+// resting volume removes the whole order (:142-146), which is what volume None does -- except where book.cuh
+// remove_order(has_vol = false) differs: `ref` is not in the level and the level's head is a snapshot aggregate, which a removal
+// with a volume reduces and volume None may not (the assert of :134, BAD_VOLUME).  True in that case.
+template <class LT>
+__device__ __forceinline__ bool fast_none_hits_aggregate(const FastBook<LT>& fb, int side, int price, uint32_t ref) {
+  unsigned char* sb = fb.side(side);
+  int j, jeq;
+  fast_find_any(fb, sb, side, fb.cnt(side)->x, price, j, jeq);
+  if (jeq < 0) return false;                                 // no level: nothing happens either way (:129-132)
+  const int start = jeq > 0 ? (int)fb.LE(sb)[jeq - 1] : 0, end = fb.LE(sb)[jeq];
+  for (int base = start; base < end; base += 32) {
+    const int i = base + fb.lane;
+    if (__any_sync(FULL_MASK, i < end && fb.O(sb)[i].y == ref)) return false;
+  }
+  return fb.O(sb)[start].y == LOBSIM_REF_AGGREGATE;
+}
+
+// One order record through the tracked straight-line path (fast_order_full<LT, true>), with what that path does not report
+// itself: the ref of a limit order that rested (an agent order rested iff next_agent_id moved, and got its old value; an
+// external one iff its own side gained an order -- fills only remove orders from the opposite side) and volume None.
+template <class LT>
+__device__ __forceinline__ uint32_t fast_submit_order(const FastBook<LT>& fb, FastState& f, const lobsim_order_t& o) {
+  if (f.dead) return 0;
+  const bool is_agent = !o.is_external;
+  const int side = o.direction;
+  BookHdr* h = reinterpret_cast<BookHdr*>(fb.blob);
+  __syncwarp();
+  if (o.type == LOBSIM_MSG_DELETE || o.type == LOBSIM_MSG_CANCEL) {
+    const uint32_t ref = is_agent ? (LOBSIM_REF_AGENT | (o.ref & 0x7fffffffu)) : o.ref;
+    int vol = o.volume;
+    if (vol <= 0) {
+      if (fast_none_hits_aggregate(fb, side, o.price, ref)) { f.err |= LOBSIM_ERR_BAD_VOLUME; return 0; }
+      vol = INT32_MAX;
+    }
+    fast_order_full<LT, true>(fb, f, o.type, side, o.price, vol, ref, is_agent);
+    return 0;
+  }
+  if (o.volume <= 0) { f.err |= LOBSIM_ERR_BAD_VOLUME; return 0; }
+  const uint32_t id0 = h->next_agent_id;
+  const int n0 = fb.cnt(side)->y;
+  fast_order_full<LT, true>(fb, f, o.type, side, o.price, o.volume, is_agent ? 0u : o.ref, is_agent);
+  __syncwarp();
+  if (o.type != LOBSIM_MSG_LIMIT) return 0;
+  if (is_agent) return h->next_agent_id != id0 ? id0 : 0u;
+  return fb.cnt(side)->y == n0 + 1 ? 0xffffffffu : 0u;
+}
+
+template <class LT>
+__host__ __device__ constexpr int submit_warp_bytes() { return (LT::blob_bytes + 8 + 127) & ~127; }   // the blob and one mbarrier
+#define LOBSIM_SUBMIT_WARPS 4
+
+// The frame of k_env_fast: the header first, then only the occupied part of the blob (a flat blob left by k_replay_flat is
+// converted on load), the orders, and the occupied part back in the sorted form.  Like Exchange.process_order, the call moves
+// only the books and the agent tables: the portfolio, the per-step flow and the fill counter that fast_record_fn moves in the
+// header are restored before the store.  An env with count 0 is neither read nor written.
+template <class LT>
+__global__ void __launch_bounds__(32 * LOBSIM_SUBMIT_WARPS) k_submit_orders(const __grid_constant__ SubmitParams p) {
+  extern __shared__ __align__(128) unsigned char smem[];
+  const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
+  const int env = blockIdx.x * (blockDim.x >> 5) + warp;
+  if (env >= p.n_envs) return;
+  const int n = submit_count(p, env);
+  if (n == 0) {
+    submit_row(p, env, 0, lane, [](const lobsim_order_t&) { return 0u; });
+    if (p.n_fills && lane == 0) p.n_fills[env] = 0;
+    return;
+  }
+  unsigned char* base = smem + (size_t)warp * submit_warp_bytes<LT>();
+  uint64_t* bar = reinterpret_cast<uint64_t*>(base + LT::blob_bytes);
+  unsigned char* gblob = p.blobs + (size_t)env * LT::blob_bytes;
+  if (lane == 0) {
+    mbar_init(bar, 1);
+    fence_mbar_init();
+    mbar_expect_tx(bar, (uint32_t)sizeof(BookHdr));
+    tma_load(base, gblob, (uint32_t)sizeof(BookHdr), bar);
+  }
+  __syncwarp();
+  mbar_wait(bar, 0);
+  BookHdr* h = reinterpret_cast<BookHdr*>(base);
+  if (hdr_is_flat(h)) {
+    if (flat_body_copy<LT>(base, gblob, bar, lane, h->cnt[0][1], h->cnt[1][1])) mbar_wait(bar, 1);
+    flat_leave_fn<LT>(base, lane, h->cnt[0][1], h->cnt[1][1]);
+  } else if (blob_body_copy<LT, true>(base, gblob, bar, lane)) mbar_wait(bar, 1);
+  __syncwarp();
+  const long long inventory_in = h->inventory;
+  const double cash_in = h->cash;
+  const int flow_in = lane < 8 ? h->flow[lane] : 0, n_fills_in = h->n_fills;
+  __syncwarp();
+  if (lane == 0) h->n_fills = 0;
+  FastBook<LT> fb; fb.blob = base; fb.lane = lane;
+  FastState f; f.err = h->err; f.dead = h->dead; f.bail = 0; f.bail_vol = 0;
+  f.fill_log = p.max_fills > 0 ? p.fills + (size_t)env * p.max_fills : nullptr; f.fill_cap = p.max_fills;
+  fast_refresh_best(fb, f);
+  submit_row(p, env, n, lane, [&](const lobsim_order_t& o) { return fast_submit_order<LT>(fb, f, o); });
+  __syncwarp();
+  const int n_fills = f.fill_log ? h->n_fills : 0;
+  __syncwarp();
+  if (lane < 8) h->flow[lane] = flow_in;
+  if (lane == 0) {
+    if (n_fills > f.fill_cap) f.err |= LOBSIM_ERR_FILL_LOG_FULL;
+    h->inventory = inventory_in; h->cash = cash_in; h->n_fills = n_fills_in;
+    h->err = f.err; h->dead = f.dead;
+    if (p.n_fills) p.n_fills[env] = n_fills;
+  }
+  __syncwarp();
+  fence_proxy_async();
+  __syncwarp();
+  if (lane == 12) tma_store_part(gblob, base, (uint32_t)sizeof(BookHdr));
+  blob_body_copy<LT, false>(base, gblob, nullptr, lane);
+  if (lane <= 12) { tma_store_commit(); tma_store_wait(); }
+  __syncwarp();
+}

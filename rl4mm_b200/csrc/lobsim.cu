@@ -39,6 +39,7 @@ struct FastLayoutOps {
   void (*to_sorted)(unsigned char* blobs, int n_envs, cudaStream_t stream);
   void (*env)(bool sync, int grid, int block, size_t dyn, cudaStream_t stream, const AdvParams& p, const EnvConst& ec);
   void (*env_rare)(bool sync, int grid, int block, size_t dyn, cudaStream_t stream, const AdvParams& p, const EnvConst& ec);
+  void (*submit)(const SubmitParams& p, cudaStream_t stream);
 };
 #define X(i, nl, no, na)                                                                                                   \
   cudaError_t lobsim_fast##i##_attrs(int, int);                                                                            \
@@ -46,10 +47,11 @@ struct FastLayoutOps {
   void lobsim_fast##i##_replay(ReplayKind, int, int, size_t, cudaStream_t, const AdvParams&, const EnvConst&);             \
   void lobsim_fast##i##_to_sorted(unsigned char*, int, cudaStream_t);                                                      \
   void lobsim_fast##i##_env(bool, int, int, size_t, cudaStream_t, const AdvParams&, const EnvConst&);                      \
-  void lobsim_fast##i##_env_rare(bool, int, int, size_t, cudaStream_t, const AdvParams&, const EnvConst&);
+  void lobsim_fast##i##_env_rare(bool, int, int, size_t, cudaStream_t, const AdvParams&, const EnvConst&);            \
+  void lobsim_fast##i##_submit(const SubmitParams&, cudaStream_t);
 LOBSIM_FAST_LAYOUTS(X)
 #undef X
-#define X(i, nl, no, na) {nl, no, na, lobsim_fast##i##_attrs, lobsim_fast##i##_attrs_rare, lobsim_fast##i##_replay, lobsim_fast##i##_to_sorted, lobsim_fast##i##_env, lobsim_fast##i##_env_rare},
+#define X(i, nl, no, na) {nl, no, na, lobsim_fast##i##_attrs, lobsim_fast##i##_attrs_rare, lobsim_fast##i##_replay, lobsim_fast##i##_to_sorted, lobsim_fast##i##_env, lobsim_fast##i##_env_rare, lobsim_fast##i##_submit},
 static const FastLayoutOps g_fast_layouts[LOBSIM_N_FAST_LAYOUTS] = {LOBSIM_FAST_LAYOUTS(X)};
 #undef X
 static const FastLayoutOps* find_fast_layout(const Layout& L) {
@@ -66,6 +68,23 @@ struct OrdParams {
   const lobsim_order_t* orders; int32_t n;
   lobsim_fill_t* fills; int32_t max_fills; int32_t* n_fills; uint32_t* refs_out;
 };
+
+// One lobsim_order_t on the general book routines: the record's conventions (is_external, volume None = a DELETE / CANCEL
+// with volume <= 0, BAD_VOLUME, the agent ref encoding).  Returns what refs_out reports for it: the agent id of an agent
+// limit order that rested, 0xffffffff for an external one, 0 otherwise.  k_process_orders and k_submit_orders_general
+// both go through it.
+__device__ __forceinline__ uint32_t apply_order_record(const Book& b, WarpState& w, const lobsim_order_t& o) {
+  uint32_t id = 0;
+  const bool is_agent = !o.is_external;
+  const bool has_vol = !((o.type == LOBSIM_MSG_DELETE || o.type == LOBSIM_MSG_CANCEL) && o.volume <= 0);
+  if (!w.dead) {
+    if (has_vol && o.volume <= 0) w.err |= LOBSIM_ERR_BAD_VOLUME;
+    else if (o.type == LOBSIM_MSG_LIMIT || o.type == LOBSIM_MSG_MARKET)
+      id = submit_or_execute(b, w, o.direction, o.price, o.volume, is_agent ? 0u : o.ref, o.type == LOBSIM_MSG_LIMIT, is_agent);
+    else remove_order(b, w, o.direction, o.price, o.volume, has_vol, is_agent ? (LOBSIM_REF_AGENT | (o.ref & 0x7fffffffu)) : o.ref, is_agent);
+  }
+  return id;
+}
 
 __global__ void __launch_bounds__(32) k_process_orders(const __grid_constant__ OrdParams p) {
   extern __shared__ __align__(128) unsigned char smem[];
@@ -103,19 +122,65 @@ __global__ void __launch_bounds__(32) k_process_orders(const __grid_constant__ O
     const lobsim_order_t o = p.orders[k];
     if (o.env < 0 || o.env >= p.n_envs) continue;
     if (o.env != cur_env) { if (cur_env >= 0) store_env(cur_env); load_env(o.env); cur_env = o.env; }
-    uint32_t id = 0;
-    const bool is_agent = !o.is_external;
-    const bool has_vol = !((o.type == LOBSIM_MSG_DELETE || o.type == LOBSIM_MSG_CANCEL) && o.volume <= 0);
-    if (!w.dead) {
-      if (has_vol && o.volume <= 0) w.err |= LOBSIM_ERR_BAD_VOLUME;
-      else if (o.type == LOBSIM_MSG_LIMIT || o.type == LOBSIM_MSG_MARKET)
-        id = submit_or_execute(b, w, o.direction, o.price, o.volume, is_agent ? 0u : o.ref, o.type == LOBSIM_MSG_LIMIT, is_agent);
-      else remove_order(b, w, o.direction, o.price, o.volume, has_vol, is_agent ? (LOBSIM_REF_AGENT | (o.ref & 0x7fffffffu)) : o.ref, is_agent);
-    }
+    const uint32_t id = apply_order_record(b, w, o);
     if (p.refs_out && lane == 0) p.refs_out[k] = id;
   }
   if (cur_env >= 0) store_env(cur_env);
   if (lane == 0 && p.n_fills) *p.n_fills = total_fills;
+}
+
+// ====================================================================================================================
+//  lobsim_submit_orders_dev on the runtime layout: every other capacity triple, LOBSIM_FORCE_GENERAL=1 and deep-book mode
+// ====================================================================================================================
+__device__ __forceinline__ void copy_words(unsigned char* dst, const unsigned char* src, int n, int lane) {
+  uint32_t* d = reinterpret_cast<uint32_t*>(dst);
+  const uint32_t* s = reinterpret_cast<const uint32_t*>(src);
+  for (int i = lane; i < n; i += 32) d[i] = s[i];
+}
+// The occupied part of a sorted blob, src -> dst, by the counters of src's header: the header, per side the level prices, level
+// ends and orders up to {nlv, nord}, the agent tables up to nag.  (The level ends are copied in whole words: NL is a multiple of 4.)
+__device__ __forceinline__ void blob_copy_occupied(unsigned char* dst, const unsigned char* src, const Layout& L, int lane) {
+  const BookHdr* h = reinterpret_cast<const BookHdr*>(src);
+  for (int s = 0; s < 2; s++) {
+    const int so = L.side_off + s * L.side_stride, ao = L.agent_off + s * L.NA * 12;
+    const int nlv = min(h->cnt[s][0], L.NL), nord = min(h->cnt[s][1], L.NO), nag = min(h->nag[s], L.NA);
+    copy_words(dst + so, src + so, nlv, lane);
+    copy_words(dst + so + L.lvend_off, src + so + L.lvend_off, (nlv + 1) / 2, lane);
+    copy_words(dst + so + L.ord_off, src + so + L.ord_off, 2 * nord, lane);
+    for (int part = 0; part < 3; part++) copy_words(dst + ao + part * L.NA * 4, src + ao + part * L.NA * 4, nag, lane);
+  }
+  copy_words(dst, src, (int)sizeof(BookHdr) / 4, lane);
+  __syncwarp();
+}
+
+// One warp per env: the occupied part of the blob into shared memory (deep-book mode: the blob in place in HBM, as
+// k_process_orders does), the row's orders through apply_order_record, the occupied part back.  The portfolio is restored as in
+// k_process_orders.  An env with count 0 is neither read nor written.
+__global__ void __launch_bounds__(128) k_submit_orders_general(const __grid_constant__ SubmitParams p) {
+  extern __shared__ __align__(128) unsigned char smem[];
+  const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
+  const int env = blockIdx.x * (blockDim.x >> 5) + warp;
+  if (env >= p.n_envs) return;
+  const int n = submit_count(p, env);
+  if (n == 0) {
+    submit_row(p, env, 0, lane, [](const lobsim_order_t&) { return 0u; });
+    if (p.n_fills && lane == 0) p.n_fills[env] = 0;
+    return;
+  }
+  unsigned char* gblob = p.blobs + (size_t)env * p.L.blob_bytes;
+  Book b; b.L = p.L; b.lane = lane;
+  b.blob = p.blob_in_global ? gblob : smem + (size_t)warp * p.L.blob_bytes;
+  if (!p.blob_in_global) blob_copy_occupied(b.blob, gblob, p.L, lane);
+  WarpState w;
+  load_state(b, w);
+  const long long inventory_in = w.inventory; const double cash_in = w.cash;
+  w.fill_log = p.max_fills > 0 ? p.fills + (size_t)env * p.max_fills : nullptr;
+  w.fill_cap = p.max_fills; w.n_fills = 0;
+  submit_row(p, env, n, lane, [&](const lobsim_order_t& o) { return apply_order_record(b, w, o); });
+  w.inventory = inventory_in; w.cash = cash_in;
+  store_state(b, w);
+  if (!p.blob_in_global) blob_copy_occupied(gblob, b.blob, p.L, lane);
+  if (p.n_fills && lane == 0) p.n_fills[env] = w.n_fills;
 }
 
 // ====================================================================================================================
@@ -459,6 +524,7 @@ struct lobsim {
                                       // (the flat replay converts back at the end of every launch)
   lobsim_order_t* po_orders = nullptr; uint32_t* po_refs = nullptr; lobsim_fill_t* po_fills = nullptr; int32_t* po_nf = nullptr;   // lobsim_process_orders staging
   int po_cap = 0, po_fill_cap = 0;
+  int submit_wpc = 1;                 // warps (= books) per CTA of k_submit_orders_general
   bool blob_in_global = false;        // deep-book mode: the blob exceeds the shared memory of an SM and is worked on in place in HBM
   bool maybe_flat = false;            // some blob in HBM may be in the flat form: ensure_sorted() before anything that reads level arrays
   bool agent_orders_possible = false; // an agent order may rest in some book (disables the replay fast path)
@@ -596,6 +662,8 @@ int lobsim_create(const lobsim_cfg_t* cfg, int device, lobsim_t** out) {
   CUDA_TRY((cudaFuncSetAttribute(k_advance<true>, cudaFuncAttributePreferredSharedMemoryCarveout, cudaSharedmemCarveoutMaxShared)));
   CUDA_TRY((cudaFuncSetAttribute(k_advance<false>, cudaFuncAttributePreferredSharedMemoryCarveout, cudaSharedmemCarveoutMaxShared)));
   if (!h->blob_in_global) CUDA_TRY(cudaFuncSetAttribute(k_process_orders, cudaFuncAttributeMaxDynamicSharedMemorySize, h->L.blob_bytes));
+  h->submit_wpc = h->blob_in_global ? LOBSIM_SUBMIT_WARPS : std::max(1, std::min(LOBSIM_SUBMIT_WARPS, (max_smem - 1024) / h->L.blob_bytes));
+  if (!h->blob_in_global) CUDA_TRY(cudaFuncSetAttribute(k_submit_orders_general, cudaFuncAttributeMaxDynamicSharedMemorySize, h->submit_wpc * h->L.blob_bytes));
   // feature rings
   memset(&h->ec, 0, sizeof h->ec);
   h->ec.cfg = *cfg;
@@ -1054,6 +1122,30 @@ int lobsim_process_orders(lobsim_t* h, const lobsim_order_t* orders, int32_t n, 
   if (e == cudaSuccess && refs_out) e = cudaMemcpy(refs_out, d_refs, (size_t)n * sizeof(uint32_t), cudaMemcpyDeviceToHost);
   if (e != cudaSuccess) return fail(LOBSIM_E_CUDA, cudaGetErrorString(e));
   if (n_fills_out) *n_fills_out = nf;
+  return LOBSIM_OK;
+}
+
+int lobsim_submit_orders_dev(lobsim_t* h, int32_t max_orders, const lobsim_order_t* orders_dev, const int32_t* count_dev,
+                             uint32_t* refs_dev, int32_t max_fills, lobsim_fill_t* fills_dev, int32_t* n_fills_dev, void* stream) {
+  if (!h || !orders_dev || !count_dev) return fail(LOBSIM_E_INVALID, "null argument");
+  if (max_orders < 1) return fail(LOBSIM_E_INVALID, "max_orders must be at least 1");
+  if (max_fills < 0 || (max_fills > 0 && !fills_dev)) return fail(LOBSIM_E_INVALID, "max_fills must be >= 0, and fills_dev non-null when it is > 0");
+  if ((uintptr_t)orders_dev & 15) return fail(LOBSIM_E_INVALID, "orders_dev must be 16-byte aligned");
+  CUDA_TRY(cudaSetDevice(h->device));
+  SubmitParams p;
+  p.blobs = h->blobs; p.L = h->L; p.n_envs = h->cfg.n_envs; p.blob_in_global = h->blob_in_global ? 1 : 0;
+  p.max_orders = max_orders; p.orders = orders_dev; p.count = count_dev; p.refs = refs_dev;
+  p.max_fills = max_fills; p.fills = max_fills > 0 ? fills_dev : nullptr; p.n_fills = n_fills_dev;
+  // an agent order may rest from here on: later replays take the tracked kernel.  (No ensure_sorted: k_submit_orders converts a
+  // flat blob on load and stores it sorted; the handles of the general kernel never hold flat blobs.)
+  h->agent_orders_possible = true;
+  if (h->fast) h->fast->submit(p, (cudaStream_t)stream);
+  else {
+    const int wpc = h->submit_wpc;
+    k_submit_orders_general<<<(p.n_envs + wpc - 1) / wpc, 32 * wpc, h->blob_in_global ? 0 : (size_t)wpc * h->L.blob_bytes, (cudaStream_t)stream>>>(p);
+  }
+  CUDA_TRY(cudaGetLastError());
+  h->launches++;
   return LOBSIM_OK;
 }
 

@@ -177,6 +177,60 @@ class LobSim:
                                           np_ptr(refs)))
         return fills[: nf.value], refs
 
+    def submit_orders(self, orders: torch.Tensor, count=None, max_fills: int = 0, refs: bool = True, out=None, stream=None):
+        """Exchange.process_order (Exchange.py:58-69) for every env at once, on the device, in one launch
+        (lobsim_submit_orders_dev): row i of ``orders`` is env i's own list of orders, applied in order, exactly as
+        ``process_orders`` would apply them.
+
+        ``orders``: a contiguous int32 CUDA tensor [N, K, 8] on this handle's device, a ``lobsim_order_t`` array
+        (``abi.pack_orders`` builds one; the ``env`` field is ignored).  ``count``: the orders of each row to apply, an int32
+        tensor [N] on the device or an int (default K for every env); values outside [0, K] are clamped.  Returns ``refs``
+        uint32 [N, K] (int64 if this torch build has no uint32; None with ``refs=False``): the agent id of an agent limit
+        order that rested, 0xffffffff for an external one that rested, 0 otherwise; ``fills`` int32 [N, max_fills, 6] in
+        ``abi.FILL_DTYPE`` field order, each env's fills in emission order; ``n_fills`` int32 [N], each env's number of fills
+        (also beyond ``max_fills``, which then sets ``abi.ERR_FILL_LOG_FULL``; with ``max_fills=0`` nothing is counted).
+        ``out``: a tuple (refs, fills, n_fills) of preallocated tensors (refs None with ``refs=False``), filled and returned
+        instead (for CUDA graph capture).  No host synchronisation.
+
+        Like ``process_orders`` the call moves only the books and the agent's orders: inventory, cash and ``fills(env)`` are
+        unchanged.  It has no pass-through on ``OrderbookSimulator`` or ``HistoricalOrderbookEnvironment``: their order-id
+        convertors and ref maps are host state per env and would not see these orders."""
+        N = self.n_envs
+        if not (isinstance(orders, torch.Tensor) and orders.dtype == torch.int32 and orders.dim() == 3 and orders.shape[0] == N
+                and orders.shape[2] == 8 and orders.device == self.device and orders.is_contiguous()):
+            raise ValueError(f"orders: expected a contiguous int32 tensor of shape [{N}, K, 8] on {self.device}")
+        K = int(orders.shape[1])
+        if K < 1:
+            raise ValueError("orders: K must be at least 1")
+        max_fills = int(max_fills)
+        if max_fills < 0:
+            raise ValueError("max_fills must be >= 0")
+        if count is None or not isinstance(count, torch.Tensor):
+            count = torch.full((N,), K if count is None else int(count), dtype=torch.int32, device=self.device)
+        elif count.dtype != torch.int32 or tuple(count.shape) != (N,) or count.device != self.device or not count.is_contiguous():
+            raise ValueError(f"count: expected a contiguous int32 tensor of shape ({N},) on {self.device}")
+        u32 = getattr(torch, "uint32", None)
+        want = [((N, K), u32 or torch.int32) if refs else None, ((N, max_fills, 6), torch.int32), ((N,), torch.int32)]
+        if out is None:
+            res = tuple(torch.empty(w[0], dtype=w[1], device=self.device) if w else None for w in want)
+        else:
+            res = tuple(out)
+            if len(res) != 3:
+                raise ValueError("out: expected a tuple (refs, fills, n_fills)")
+            for t, w in zip(res, want):
+                if w is None:
+                    if t is not None:
+                        raise ValueError("out: refs must be None with refs=False")
+                elif not isinstance(t, torch.Tensor) or t.dtype != w[1] or tuple(t.shape) != w[0] or t.device != self.device \
+                        or not t.is_contiguous():
+                    raise ValueError(f"out: expected a contiguous {w[1]} tensor of shape {w[0]} on {self.device}")
+        r, fills, n_fills = res
+        check(lib().lobsim_submit_orders_dev(self._h, K, _dptr(orders), _dptr(count), _dptr(r), max_fills,
+                                             _dptr(fills) if max_fills > 0 else None, _dptr(n_fills), self._stream_arg(stream)))
+        if r is not None and u32 is None and out is None:
+            r = r.to(torch.int64) & 0xFFFFFFFF
+        return r, fills, n_fills
+
     def dump_book(self, env: int, side: int) -> np.ndarray:
         torch.cuda.synchronize(self.device)
         n = lib().lobsim_dump_book(self._h, env, side, None, 0)
