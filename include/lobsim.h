@@ -366,6 +366,40 @@ int lobsim_dump_book(lobsim_t* h, int32_t env, int32_t side, lobsim_book_entry_t
 /* the agent's internal book side (Exchange.internal_orderbook), ascending internal id */
 int lobsim_dump_agent_orders(lobsim_t* h, int32_t env, int32_t side, lobsim_book_entry_t* out_host, int32_t capacity);
 
+/* L3 of every env's central book on the device, in one launch: lobsim_dump_book for all envs and both sides.
+ *   count_dev    int32 [n_envs][2]: the side's number of resting orders, also when it exceeds max_entries (then only the
+ *                first max_entries are written)
+ *   entries_dev  lobsim_book_entry_t [n_envs][2][max_entries], 16-byte aligned: best level first, FIFO inside a level,
+ *                level = 0-based index of the price level (the lobsim_dump_book format, bit for bit); unused slots
+ *                {LOBSIM_NO_PRICE, 0, 0, -1}
+ * 1 <= max_entries <= max_orders_per_side.  Stream-ordered on `stream`.  Like lobsim_get_depth_dev, the call reads every book
+ * in the form it is in and changes no state: no book form conversion, no host synchronisation, no allocation, exactly one
+ * kernel launch -- it may run between any two launches and inside a captured CUDA graph.                          */
+int lobsim_get_book_dev(lobsim_t* h, int32_t max_entries, int32_t* count_dev, lobsim_book_entry_t* entries_dev, void* stream);
+
+/* per-env outcome of lobsim_set_book_dev (status_dev).  The checks run in this order, over both sides, and the first one
+ * that fails is reported: */
+#define LOBSIM_SETBOOK_OK 0
+#define LOBSIM_SETBOOK_SKIPPED 1       /* a negative count on either side: the env was neither read nor written          */
+#define LOBSIM_SETBOOK_E_COUNT -1      /* count > max_entries                                                           */
+#define LOBSIM_SETBOOK_E_VOLUME -2     /* a negative volume                                                             */
+#define LOBSIM_SETBOOK_E_UNSORTED -3   /* a side not sorted best level first (a price that comes back after another)    */
+#define LOBSIM_SETBOOK_E_LEVELS -4     /* more than max_levels_per_side levels                                          */
+#define LOBSIM_SETBOOK_E_ORDERS -5     /* more than max_orders_per_side orders                                          */
+#define LOBSIM_SETBOOK_E_AGENTS -6     /* more than max_agent_orders agent entries on a side                            */
+/* lobsim_set_book for every env at once, on the device: row env of entries_dev / count_dev replaces that env's books, exactly
+ * as lobsim_set_book(h, env, ...) would with the same entries (the `level` field is ignored): sorted level arrays, the agent
+ * table in ascending id (equal ids in entry order), next_agent_id = max(next_agent_id, max id + 1), dead = err = 0; the clock,
+ * the portfolio and the rest of the env's state are untouched.
+ *   entries_dev  lobsim_book_entry_t [n_envs][2][max_entries], 16-byte aligned (side 0 = buy)
+ *   count_dev    int32 [n_envs][2]: entries of each row to apply
+ *   status_dev   int32 [n_envs], required: LOBSIM_SETBOOK_OK, LOBSIM_SETBOOK_SKIPPED or a LOBSIM_SETBOOK_E_* code (the env
+ *                is left exactly as it was, its error bits included)
+ * The call returns LOBSIM_E_INVALID only for bad arguments (a NULL pointer, max_entries < 1, misalignment).  Stream-ordered
+ * on `stream`: no host synchronisation, no allocation, exactly one kernel launch.                                  */
+int lobsim_set_book_dev(lobsim_t* h, int32_t max_entries, const lobsim_book_entry_t* entries_dev, const int32_t* count_dev,
+                        int32_t* status_dev, void* stream);
+
 /* L2 depth of every env's central book on the device, in one launch: the L2 projection of lobsim_dump_book
  * (rl4mm/extras/orderbook_comparison.py:6-19) for all envs and both sides at once.  Outputs are [n_envs][2][depth],
  * side 0 = buy, level 0 = the best level (highest buy / lowest sell price), the layout of the stream snapshots:

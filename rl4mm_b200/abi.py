@@ -49,6 +49,9 @@ INFO_FIELDS = ("asset_price", "inventory", "cash", "aum", "market_spread", "best
 INFO_DIM = len(INFO_FIELDS)
 AGENT_NONE, AGENT_FIXED, AGENT_TERADACTYL, AGENT_EXTERNAL, AGENT_RANDOM = 0, 1, 2, 3, 4
 PATH_GENERAL, PATH_FAST, PATH_DEEP = 0, 1, 2
+# per-env outcome of lobsim_set_book_dev / LobSim.set_books, in the order the checks run (the first that fails is reported)
+SETBOOK_OK, SETBOOK_SKIPPED = 0, 1
+SETBOOK_E_COUNT, SETBOOK_E_VOLUME, SETBOOK_E_UNSORTED, SETBOOK_E_LEVELS, SETBOOK_E_ORDERS, SETBOOK_E_AGENTS = range(-1, -7, -1)
 
 MSG_DTYPE = np.dtype([("price", "<i4"), ("volume", "<i4"), ("ref", "<u4"), ("meta", "<u4")])
 assert MSG_DTYPE.itemsize == 16

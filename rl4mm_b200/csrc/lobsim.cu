@@ -470,6 +470,248 @@ __global__ void __launch_bounds__(128, 9) k_agent_orders(const unsigned char* bl
   }
 }
 
+// ====================================================================================================================
+//  per-env L3 book, read and replaced on the device (one warp per env, the blob in HBM in whichever form it is in)
+// ====================================================================================================================
+// Side s of env e is row (e * 2 + s) of `entries` (max_entries uint4 {price, volume, ref, level}, the lobsim_book_entry_t
+// bits): the lobsim_dump_book order, best level first and FIFO inside a level.  Unused slots are {NO_PRICE, 0, 0, -1}; the
+// count is the side's number of orders, also beyond max_entries.
+__global__ void __launch_bounds__(128) k_get_book(const unsigned char* blobs, Layout L, int n_envs, int max_entries, int32_t* count,
+                                                  uint4* entries) {
+  const int lane = threadIdx.x & 31;
+  const int env = blockIdx.x * (blockDim.x >> 5) + (threadIdx.x >> 5);
+  if (env >= n_envs) return;
+  const unsigned char* blob = blobs + (size_t)env * L.blob_bytes;
+  const BookHdr* h = reinterpret_cast<const BookHdr*>(blob);
+  const bool flat = h->cnt[0][0] < 0;
+  for (int side = 0; side < 2; side++) {
+    uint4* row = entries + ((size_t)env * 2 + side) * max_entries;
+    const unsigned char* sb = blob + L.side_off + side * L.side_stride;
+    int n;
+    if (flat) {
+      // flat form (book_flat.cuh): an unordered pool of n <= 128 orders {price, ref, volume, seq}, 4 per lane in registers.
+      // flat_leave sorts by (price, seq): an order's slot is the number of orders at better prices plus the older ones at its
+      // own price, and its level the number of distinct better prices (the oldest order of each price stands for it).
+      const uint4* pool = reinterpret_cast<const uint4*>(sb + L.ord_off);
+      n = h->cnt[side][1];
+      uint4 e[4];
+      int rank[4], older[4];
+#pragma unroll
+      for (int c = 0; c < 4; c++) {
+        e[c] = make_uint4(0u, 0u, 0u, 0u);
+        if (c * 32 + lane < n) e[c] = pool[c * 32 + lane];
+        rank[c] = 0; older[c] = 0;
+      }
+#pragma unroll
+      for (int cm = 0; cm < 4; cm++) {
+        for (int l = 0; l < 32 && cm * 32 + l < n; l++) {
+          const int pm = (int)__shfl_sync(FULL_MASK, e[cm].x, l);
+          const unsigned qm = __shfl_sync(FULL_MASK, e[cm].w, l);
+          const int m = cm * 32 + l;
+#pragma unroll
+          for (int c = 0; c < 4; c++) {
+            const int p = (int)e[c].x;
+            const bool same_older = pm == p && (qm < e[c].w || (qm == e[c].w && m < c * 32 + lane));
+            rank[c] += (side ? pm < p : pm > p) || same_older;
+            older[c] += same_older;
+          }
+        }
+      }
+      int level[4] = {0, 0, 0, 0};
+#pragma unroll
+      for (int cm = 0; cm < 4; cm++) {
+        unsigned heads = __ballot_sync(FULL_MASK, cm * 32 + lane < n && older[cm] == 0);
+        while (heads) {
+          const int pm = (int)__shfl_sync(FULL_MASK, e[cm].x, __ffs(heads) - 1);
+          heads &= heads - 1;
+#pragma unroll
+          for (int c = 0; c < 4; c++) level[c] += side ? pm < (int)e[c].x : pm > (int)e[c].x;
+        }
+      }
+#pragma unroll
+      for (int c = 0; c < 4; c++)
+        if (c * 32 + lane < n && rank[c] < max_entries) row[rank[c]] = make_uint4(e[c].x, e[c].z, e[c].y, (unsigned)level[c]);
+    } else {
+      // sorted form (book.cuh): levels worst -> best, so best-first level k is segment j = nlv - 1 - k, and output slots
+      // [total - lvend[j], total - lvend[j - 1]) hold it.  32 slots per round, one per lane; a window of 32 levels (lane t =
+      // level kb + t: its price, first ord index and end slot) gives each slot its level by a shuffle search over the end slots.
+      const int32_t* lvp = reinterpret_cast<const int32_t*>(sb);
+      const uint16_t* lvend = reinterpret_cast<const uint16_t*>(sb + L.lvend_off);
+      const uint2* ord = reinterpret_cast<const uint2*>(sb + L.ord_off);
+      const int nlv = h->cnt[side][0];
+      n = nlv > 0 ? lvend[nlv - 1] : 0;       // what dump_book walks: the segments of the nlv levels
+      const int m = min(n, max_entries);
+      int kb = 0;
+      for (int p0 = 0; p0 < m; p0 += 32) {
+        const int p = p0 + lane;
+        bool need = p < m;
+        int lvl = kb, price = 0, at = 0;
+        while (__any_sync(FULL_MASK, need)) {
+          const int wn = min(32, nlv - kb);
+          if (wn <= 0) break;
+          int tp = 0, tfirst = 0, tstart = 0, tend = INT32_MAX;
+          if (lane < wn) {
+            const int j = nlv - 1 - kb - lane;
+            tp = lvp[j]; tfirst = j ? lvend[j - 1] : 0; tstart = n - lvend[j]; tend = n - tfirst;
+          }
+          int c = 0;                               // the window's levels that end at or before slot p (end slots rise with t)
+#pragma unroll
+          for (int s = 16; s; s >>= 1) {
+            const int te = __shfl_sync(FULL_MASK, tend, c + s - 1);
+            if (te <= p) c += s;
+          }
+          if (__shfl_sync(FULL_MASK, tend, c & 31) <= p) c++;   // (c = 31 only: all 32 levels end at or before p)
+          const int cp = __shfl_sync(FULL_MASK, tp, c & 31), cf = __shfl_sync(FULL_MASK, tfirst, c & 31);
+          const int cs = __shfl_sync(FULL_MASK, tstart, c & 31);
+          if (need && c < wn) { lvl = kb + c; price = cp; at = cf + (p - cs); need = false; }
+          if (__any_sync(FULL_MASK, need)) kb += wn;
+        }
+        if (p < m) {
+          const uint2 o = ord[at];
+          row[p] = make_uint4((unsigned)price, o.x, o.y, (unsigned)lvl);
+        }
+        kb = __shfl_sync(FULL_MASK, lvl, 31);
+      }
+    }
+    for (int k = n + lane; k < max_entries; k += 32) row[k] = make_uint4((unsigned)LOBSIM_NO_PRICE, 0u, 0u, 0xffffffffu);
+    if (lane == 0) count[env * 2 + side] = n;
+  }
+}
+
+// Entries [p0, p0 + 32) of a row, one per lane: the entry (zeros beyond n), the previous entry's price `pl`, and whether the
+// entry starts a level (its price differs from pl).  `prev` carries the price of entry p0 - 1 and is advanced.
+__device__ __forceinline__ bool book_row_entry(const uint4* row, int p0, int n, int lane, int& prev, uint4& e, int& pl) {
+  const int i = p0 + lane;
+  e = i < n ? row[i] : make_uint4(0u, 0u, 0u, 0u);
+  pl = __shfl_up_sync(FULL_MASK, (int)e.x, 1);
+  if (lane == 0) pl = prev;
+  prev = __shfl_sync(FULL_MASK, (int)e.x, 31);
+  return i < n && (i == 0 || (int)e.x != pl);
+}
+
+// lobsim_set_book for every env: row (e * 2 + s) of `entries` replaces side s of env e.  Pass 1 reads both sides and runs the
+// checks of lobsim_set_book; an env that fails one is left exactly as it was.  Pass 2 writes, per side, the level prices and ends
+// (at each level start: best-first level k is index j = nlv - 1 - k, and lvend[j] = n - start(k)), then the orders (entry i of
+// level k goes to ord[lvend[j - 1] + i - start(k)], lvend[j - 1] being the end of the next worse level), then the agent table:
+// agent entries ranked by (id, entry index), as lobsim_set_book's std::sort.  Last the header: counts, nag, next_agent_id,
+// dead = err = 0 (a flat blob's header becomes a sorted one).
+__global__ void __launch_bounds__(128) k_set_book(unsigned char* blobs, Layout L, int n_envs, int max_entries, const uint4* entries,
+                                                  const int32_t* count, int32_t* status) {
+  const int lane = threadIdx.x & 31;
+  const int env = blockIdx.x * (blockDim.x >> 5) + (threadIdx.x >> 5);
+  if (env >= n_envs) return;
+  const int cnt[2] = {count[env * 2], count[env * 2 + 1]};
+  if (cnt[0] < 0 || cnt[1] < 0) {
+    if (lane == 0) status[env] = LOBSIM_SETBOOK_SKIPPED;
+    return;
+  }
+  unsigned char* blob = blobs + (size_t)env * L.blob_bytes;
+  unsigned fails = 0;                         // bit c - 1: check c failed on a side
+  int nlv[2] = {0, 0}, nag[2] = {0, 0}, afirst[2] = {INT32_MAX, INT32_MAX}, alast[2] = {-1, -1};
+  unsigned max_id = 0;
+  for (int side = 0; side < 2; side++) {
+    const int n = cnt[side];
+    if (n > max_entries) { fails |= 1u; continue; }
+    const uint4* row = entries + ((size_t)env * 2 + side) * max_entries;
+    int prev = 0;
+    bool neg = false, unsorted = false;
+    for (int p0 = 0; p0 < n; p0 += 32) {
+      uint4 e;
+      int pl;
+      const bool start = book_row_entry(row, p0, n, lane, prev, e, pl);
+      const bool agent = p0 + lane < n && (e.z & LOBSIM_REF_AGENT);
+      neg |= p0 + lane < n && (int)e.y < 0;
+      // a new level must be strictly worse than the one before it (so a price never comes back)
+      unsorted |= start && p0 + lane > 0 && (side ? (int)e.x < pl : (int)e.x > pl);
+      nlv[side] += __popc(__ballot_sync(FULL_MASK, start));
+      const unsigned am = __ballot_sync(FULL_MASK, agent);
+      nag[side] += __popc(am);
+      if (am) { afirst[side] = min(afirst[side], p0); alast[side] = p0; }
+      if (agent) max_id = max(max_id, e.z & 0x7fffffffu);
+    }
+    if (__any_sync(FULL_MASK, neg)) fails |= 2u;
+    if (__any_sync(FULL_MASK, unsorted)) fails |= 4u;
+    if (nlv[side] > L.NL) fails |= 8u;
+    if (n > L.NO) fails |= 16u;
+    if (nag[side] > L.NA) fails |= 32u;
+  }
+  if (fails) {
+    if (lane == 0) status[env] = -(__ffs(fails));
+    return;
+  }
+  const unsigned le_mask = 0xffffffffu >> (31 - lane);      // lanes <= this lane
+  for (int side = 0; side < 2; side++) {
+    const int n = cnt[side];
+    const uint4* row = entries + ((size_t)env * 2 + side) * max_entries;
+    unsigned char* sb = blob + L.side_off + side * L.side_stride;
+    int32_t* lvp = reinterpret_cast<int32_t*>(sb);
+    uint16_t* lvend = reinterpret_cast<uint16_t*>(sb + L.lvend_off);
+    uint2* ord = reinterpret_cast<uint2*>(sb + L.ord_off);
+    int prev = 0, below = 0;
+    for (int p0 = 0; p0 < n; p0 += 32) {     // level prices and ends
+      uint4 e;
+      int pl;
+      const bool start = book_row_entry(row, p0, n, lane, prev, e, pl);
+      const unsigned sm = __ballot_sync(FULL_MASK, start);
+      if (start) {
+        const int j = nlv[side] - below - __popc(sm & le_mask);
+        lvp[j] = (int)e.x; lvend[j] = (uint16_t)(n - (p0 + lane));
+      }
+      below += __popc(sm);
+    }
+    __syncwarp();
+    prev = 0; below = 0;
+    int level_start = 0;                     // start of the level in progress at the chunk's first entry
+    for (int p0 = 0; p0 < n; p0 += 32) {     // orders
+      uint4 e;
+      int pl;
+      const bool start = book_row_entry(row, p0, n, lane, prev, e, pl);
+      const unsigned sm = __ballot_sync(FULL_MASK, start), mine = sm & le_mask;
+      const int s = mine ? p0 + 31 - __clz(mine) : level_start;
+      if (p0 + lane < n) {
+        const int j = nlv[side] - below - __popc(mine);
+        ord[(j ? lvend[j - 1] : 0) + p0 + lane - s] = make_uint2(e.y, e.z);
+      }
+      level_start = __shfl_sync(FULL_MASK, s, 31);
+      below += __popc(sm);
+    }
+    if (nag[side]) {                         // agent table: rank by counting over the chunks that hold agent entries
+      int32_t* ap = reinterpret_cast<int32_t*>(blob + L.agent_off + side * L.NA * 12);
+      int32_t* av = ap + L.NA;
+      uint32_t* ai = reinterpret_cast<uint32_t*>(ap + 2 * L.NA);
+      for (int c1 = afirst[side]; c1 <= alast[side]; c1 += 32) {
+        const int i1 = c1 + lane;
+        const uint4 e1 = i1 < n ? row[i1] : make_uint4(0u, 0u, 0u, 0u);
+        const bool mine = i1 < n && (e1.z & LOBSIM_REF_AGENT);
+        if (!__any_sync(FULL_MASK, mine)) continue;
+        const unsigned id1 = e1.z & 0x7fffffffu;
+        int rank = 0;
+        for (int c2 = afirst[side]; c2 <= alast[side]; c2 += 32) {
+          const int i2 = c2 + lane;
+          const unsigned r2 = i2 < n ? row[i2].z : 0u;
+          unsigned am = __ballot_sync(FULL_MASK, (r2 & LOBSIM_REF_AGENT) != 0);
+          while (am) {
+            const int l = __ffs(am) - 1;
+            am &= am - 1;
+            const unsigned id2 = __shfl_sync(FULL_MASK, r2, l) & 0x7fffffffu;
+            rank += id2 < id1 || (id2 == id1 && c2 + l < i1);
+          }
+        }
+        if (mine) { ap[rank] = (int32_t)e1.x; av[rank] = (int32_t)e1.y; ai[rank] = id1; }
+      }
+    }
+  }
+  max_id = __reduce_max_sync(FULL_MASK, max_id);
+  __syncwarp();
+  if (lane == 0) {
+    BookHdr* h = reinterpret_cast<BookHdr*>(blob);
+    for (int side = 0; side < 2; side++) { h->cnt[side][0] = nlv[side]; h->cnt[side][1] = cnt[side]; h->nag[side] = nag[side]; }
+    if (h->next_agent_id <= max_id) h->next_agent_id = max_id + 1;
+    h->dead = 0; h->err = 0;
+    status[env] = LOBSIM_SETBOOK_OK;
+  }
+}
+
 __global__ void k_init_blobs(unsigned char* blobs, Layout L, int n, long long inventory, double cash) {
   int i = blockIdx.x * blockDim.x + threadIdx.x;
   if (i >= n) return;
@@ -1045,6 +1287,37 @@ int lobsim_get_agent_orders_dev(lobsim_t* h, int32_t max_orders, int32_t* count_
   // reads flat and sorted blobs as they are (no ensure_sorted): one launch, no synchronisation, no allocation
   const AgentOrdersOut out = {count_dev, price_dev, volume_dev, id_dev, level_dev, ahead_orders_dev, ahead_volume_dev};
   k_agent_orders<<<(h->cfg.n_envs + 3) / 4, 128, 0, (cudaStream_t)stream>>>(h->blobs, h->L, h->cfg.n_envs, max_orders, out);
+  CUDA_TRY(cudaGetLastError());
+  h->launches++;
+  return LOBSIM_OK;
+}
+
+int lobsim_get_book_dev(lobsim_t* h, int32_t max_entries, int32_t* count_dev, lobsim_book_entry_t* entries_dev, void* stream) {
+  if (!h || !count_dev || !entries_dev) return fail(LOBSIM_E_INVALID, "null argument");
+  if (max_entries < 1 || max_entries > h->cfg.max_orders_per_side) return fail(LOBSIM_E_INVALID, "max_entries must be in [1, max_orders_per_side]");
+  if (((uintptr_t)entries_dev & 15) || ((uintptr_t)count_dev & 3)) return fail(LOBSIM_E_INVALID, "entries_dev must be 16-byte aligned, count_dev 4-byte aligned");
+  CUDA_TRY(cudaSetDevice(h->device));
+  // reads flat and sorted blobs as they are (no ensure_sorted): one launch, no synchronisation, no allocation
+  k_get_book<<<(h->cfg.n_envs + 3) / 4, 128, 0, (cudaStream_t)stream>>>(h->blobs, h->L, h->cfg.n_envs, max_entries, count_dev,
+                                                                         reinterpret_cast<uint4*>(entries_dev));
+  CUDA_TRY(cudaGetLastError());
+  h->launches++;
+  return LOBSIM_OK;
+}
+
+int lobsim_set_book_dev(lobsim_t* h, int32_t max_entries, const lobsim_book_entry_t* entries_dev, const int32_t* count_dev,
+                        int32_t* status_dev, void* stream) {
+  if (!h || !entries_dev || !count_dev || !status_dev) return fail(LOBSIM_E_INVALID, "null argument");
+  if (max_entries < 1) return fail(LOBSIM_E_INVALID, "max_entries must be at least 1");
+  if (((uintptr_t)entries_dev & 15) || ((uintptr_t)count_dev & 3) || ((uintptr_t)status_dev & 3))
+    return fail(LOBSIM_E_INVALID, "entries_dev must be 16-byte aligned, count_dev and status_dev 4-byte aligned");
+  CUDA_TRY(cudaSetDevice(h->device));
+  // no ensure_sorted: a set env's blob is written in the sorted form whatever form it was in, and the others keep theirs
+  // (maybe_flat stays as it is).  Whether an agent entry arrived is only known on the device: later replays take the tracked
+  // kernel, as after lobsim_set_book.
+  h->agent_orders_possible = true;
+  k_set_book<<<(h->cfg.n_envs + 3) / 4, 128, 0, (cudaStream_t)stream>>>(h->blobs, h->L, h->cfg.n_envs, max_entries,
+                                                                         reinterpret_cast<const uint4*>(entries_dev), count_dev, status_dev);
   CUDA_TRY(cudaGetLastError());
   h->launches++;
   return LOBSIM_OK;

@@ -314,6 +314,67 @@ class LobSim:
                                                 self._stream_arg(stream)))
         return out
 
+    def book_l3(self, max_entries: Optional[int] = None, out=None, stream=None):
+        """L3 of every env's central book, read on the device in one launch (lobsim_get_book_dev): ``dump_book`` for all
+        envs and both sides at once, bit for bit.
+
+        Returns torch CUDA tensors ``count`` int32 [N, 2] (resting orders per side, also beyond ``max_entries``, which
+        defaults to ``cfg.max_orders_per_side``) and ``entries`` int32 [N, 2, max_entries, 4] in ``abi.BOOK_ENTRY_DTYPE``
+        field order (price, volume, ref, level; ``ref`` holds the uint32 bits): side 0 = buy, best level first, FIFO inside
+        a level; unused slots (``abi.NO_PRICE``, 0, 0, -1).  ``out``: a tuple (count, entries) of preallocated tensors,
+        filled and returned instead (for CUDA graph capture).  No host synchronisation; the books are read in whatever form
+        they are in and left unchanged."""
+        E = self.cfg.max_orders_per_side if max_entries is None else int(max_entries)
+        if not 1 <= E <= self.cfg.max_orders_per_side:
+            raise LobsimError(f"max_entries must be in [1, max_orders_per_side = {self.cfg.max_orders_per_side}], got {E}")
+        N = self.n_envs
+        want = [(N, 2), (N, 2, E, 4)]
+        if out is None:
+            out = tuple(torch.empty(shape, dtype=torch.int32, device=self.device) for shape in want)
+        else:
+            out = tuple(out)
+            if len(out) != 2:
+                raise ValueError("out: expected a tuple (count, entries)")
+            for t, shape in zip(out, want):
+                if not isinstance(t, torch.Tensor) or t.dtype != torch.int32 or tuple(t.shape) != shape or t.device != self.device \
+                        or not t.is_contiguous():
+                    raise ValueError(f"out: expected a contiguous int32 tensor of shape {shape} on {self.device}")
+        check(lib().lobsim_get_book_dev(self._h, E, _dptr(out[0]), _dptr(out[1]), self._stream_arg(stream)))
+        return out
+
+    def set_books(self, entries: torch.Tensor, count=None, out=None, stream=None) -> torch.Tensor:
+        """``set_book`` for every env at once, on the device, in one launch (lobsim_set_book_dev): row i of ``entries``
+        replaces env i's books exactly as ``set_book(i, buy, sell)`` would with the same entries.
+
+        ``entries``: a contiguous int32 CUDA tensor [N, 2, E, 4] on this handle's device in ``abi.BOOK_ENTRY_DTYPE`` field
+        order (the layout ``book_l3`` returns; ``level`` is ignored), per side best level first and FIFO inside a level.
+        ``count``: the entries of each side to apply, an int32 tensor [N, 2] on the device (default E everywhere); an env with
+        a negative count on either side is skipped.  Returns ``status`` int32 [N]: ``abi.SETBOOK_OK``,
+        ``abi.SETBOOK_SKIPPED`` or an ``abi.SETBOOK_E_*`` code (that env is left exactly as it was).  ``out``: a preallocated
+        status tensor, filled and returned instead (for CUDA graph capture).  No host synchronisation.
+
+        The clock and the portfolio are not touched.  It has no pass-through on ``OrderbookSimulator`` or
+        ``HistoricalOrderbookEnvironment``: their order-id maps are host state per env and would not see the new refs."""
+        N = self.n_envs
+        if not (isinstance(entries, torch.Tensor) and entries.dtype == torch.int32 and entries.dim() == 4 and entries.shape[0] == N
+                and entries.shape[1] == 2 and entries.shape[3] == 4 and entries.device == self.device and entries.is_contiguous()):
+            raise ValueError(f"entries: expected a contiguous int32 tensor of shape [{N}, 2, E, 4] on {self.device}")
+        E = int(entries.shape[2])
+        if E < 1:
+            raise ValueError("entries: E must be at least 1")
+        if count is None:
+            count = torch.full((N, 2), E, dtype=torch.int32, device=self.device)
+        elif not (isinstance(count, torch.Tensor) and count.dtype == torch.int32 and tuple(count.shape) == (N, 2)
+                  and count.device == self.device and count.is_contiguous()):
+            raise ValueError(f"count: expected a contiguous int32 tensor of shape ({N}, 2) on {self.device}")
+        if out is None:
+            out = torch.empty(N, dtype=torch.int32, device=self.device)
+        elif not (isinstance(out, torch.Tensor) and out.dtype == torch.int32 and tuple(out.shape) == (N,) and out.device == self.device
+                  and out.is_contiguous()):
+            raise ValueError(f"out: expected a contiguous int32 tensor of shape ({N},) on {self.device}")
+        check(lib().lobsim_set_book_dev(self._h, E, _dptr(entries), _dptr(count), _dptr(out), self._stream_arg(stream)))
+        return out
+
     def state(self, first: int = 0, n: Optional[int] = None) -> np.ndarray:
         n = self.n_envs - first if n is None else n
         out = np.zeros(n, abi.ENV_STATE_DTYPE)

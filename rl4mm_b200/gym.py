@@ -357,6 +357,13 @@ class HistoricalOrderbookEnvironment:
         it may sit next to ``step_torch`` in a CUDA graph."""
         return self.sim.agent_orders(max_orders=max_orders, queue=queue, out=out, stream=stream)
 
+    def book_l3(self, max_entries=None, out=None, stream=None):
+        """Full-depth L3 observations: the central book of every env read on the device in one launch (``LobSim.book_l3``),
+        torch CUDA tensors count int32 [n_envs, 2] and entries int32 [n_envs, 2, max_entries, 4] (price, volume, ref, level).
+        Batched and not squeezed, also when n_envs == 1; no host round trip, so it may sit next to ``step_torch`` in a CUDA
+        graph."""
+        return self.sim.book_l3(max_entries=max_entries, out=out, stream=stream)
+
     def rollout(self, agent, T: int):
         """``generate_trajectory`` (rl4mm/gym/utils.py:100-117) for T steps of every env, fused on the device when the
         agent has a device implementation (FixedActionAgent, Teradactyl); returns torch tensors obs, act, rew, done."""

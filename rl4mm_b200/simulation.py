@@ -197,6 +197,12 @@ class OrderbookSimulator:
         and not squeezed, also when n_envs == 1 or this simulator is a view of one env (index with ``self.env``)."""
         return self.sim.agent_orders(max_orders=max_orders, queue=queue, out=out, stream=stream)
 
+    def book_l3(self, max_entries=None, out=None, stream=None):
+        """The L3 book of EVERY env of the underlying LobSim (``LobSim.book_l3``): count [n_envs, 2], entries
+        [n_envs, 2, max_entries, 4], batched and not squeezed, also when n_envs == 1 or this simulator is a view of one env
+        (index with ``self.env``)."""
+        return self.sim.book_l3(max_entries=max_entries, out=out, stream=stream)
+
     @property
     def min_buy_price(self) -> int:
         return int(self.sim.state(self.env, 1)[0]["min_buy_price"])
